@@ -8,11 +8,13 @@ A "step" is one pass of the hot path (psb_scan: packed 16-bit DPX kernel + 32-bi
 results D2H) over the rank's shard of the database.  The database is sharded by residue count
 across ranks with no data-path collective (SURVEY 8e); the total work is fixed as N grows.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Rank 0 prints ONE JSON line.  `--impl reference` times the CPU baseline instead (the
 parasail-equivalent striped AVX2 restatement under oracle/, all host threads, bounded sample).
+`--dump-outputs DIR` writes the per-subject results of the last timed step as DIR/<field>.npy, so
+that two builds can be compared output for output on the same seeded inputs.
 """
 import argparse
 import json
@@ -24,6 +26,8 @@ import time
 
 import numpy as np
 
+if __name__ == "__main__":
+    sys.dont_write_bytecode = True   # the tree may be read-only, and a benchmark run leaves nothing in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests")):
     if p not in sys.path:
@@ -48,6 +52,27 @@ def make_inputs(n_db):
     query = psb_data.random_seq(QUERY_SEED, 0, QUERY_LEN)
     cat, off = psb_data.protein_db(LEN_SEED, RES_SEED, n_db, query=query, planted_frac=0.01)
     return query, cat, off
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SAMPLE_SEED = 2004
+BATCH_FIELDS = ("score", "end_query", "end_ref", "matches", "similar", "length", "beg_query", "beg_ref", "saturated")
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """Write each per-subject array as out_dir/<name>.npy in float64 (exact for the int32 results).  If they
+    would take more than `limit` bytes, every array keeps the same seeded sample of subjects, in order,
+    and the sampled subject numbers go to out_dir/sample_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    per_subject = 8 * len(arrays)
+    if n * per_subject > limit:
+        keep = (limit - 4096 * (len(arrays) + 1)) // (per_subject + 8)   # 4 KB per file for the .npy header
+        rows = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(n, keep, replace=False))
+        arrays = {k: np.asarray(v)[rows] for k, v in arrays.items()}
+        arrays["sample_index"] = rows
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 class ClockSampler:
@@ -121,6 +146,8 @@ def run_reference(args, rank):
         res, secs, c = cpu_baseline(query, cat, off, n_sample)
         cells += c
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: res[k] for k in ("score", "end_query", "end_ref")})
     value = cells / dt / 1e9
     threads = int(res["threads"])
     sample = f"{n_sample} subjects of the C2 database per step ({cells / args.steps:.3g} cells), striped AVX2 8->16->32 bit"
@@ -167,7 +194,10 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=12)
     ap.add_argument("--cpu-sample", type=int, default=200000, help="subjects of the CPU-baseline sample (rank 0, N=1)")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -262,6 +292,12 @@ def main():
     value = total_cells * args.steps / (total_ms * 1e-3) / 1e9
     scan_scores = res.score.copy()
     scan_eq, scan_er = res.end_query.copy(), res.end_ref.copy()
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives, for this rank's shard (global subject numbers beside it)
+        outputs = {k: getattr(res, k) for k in BATCH_FIELDS if getattr(res, k) is not None}
+        if world > 1:
+            outputs["subject"] = mine
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- end to end: host buffers in, host results out, every step ---------------------------------
     # N = 1: one C call with HOST buffers, psb_scan_host (piecewise upload from pinned memory on a copy

@@ -2,6 +2,7 @@
 host-side logic (matrices, name grammar, error behaviour) works without a GPU; and the product
 fails loudly -- never falls back -- when no CUDA device exists."""
 import ctypes as C
+import json
 import os
 import re
 
@@ -47,18 +48,15 @@ def test_every_declared_symbol_is_exported(ps):
 
 
 def test_reference_binds_105_functions(ps):
-    # the four `use libparasail_sys::{..}` blocks: aligner 4 + profile 52 + matrix 8 + alignment 41
+    # the four `use libparasail_sys::{..}` blocks of parasail-rs, stored in tests/golden/reference_bindings.json:
+    # aligner 4 + profile 52 + matrix 8 + alignment 41
     from parasail_rs_b200 import _lib
     L = _lib.lib()
-    src = ""
-    for f in ("aligner", "profile", "matrix", "alignment"):
-        path = f"/root/reference/src/{f}/mod.rs"
-        if not os.path.exists(path):
-            pytest.skip("reference tree not mounted")
-        text = open(path).read()
-        src += text[text.index("use libparasail_sys::{"): text.index("};", text.index("use libparasail_sys::{"))]
-    fns = {n for n in re.findall(r"\bparasail_[a-z0-9_]+", src) if not n.endswith("_t") and n not in ("parasail_matrix", "parasail_profile")}
+    mods = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_bindings.json")))["modules"]
+    assert {m: len(set(v)) for m, v in mods.items()} == {"aligner": 4, "profile": 52, "matrix": 8, "alignment": 41}
+    fns = set().union(*mods.values())
     assert len(fns) == 105
+    assert fns <= header_symbols()
     assert not [n for n in sorted(fns) if not hasattr(L, n)]
 
 

@@ -3,6 +3,7 @@
 mkdir -p gpurun_out/r2a
 nvidia-smi --query-gpu=name,clocks.max.sm,clocks.sm --format=csv > gpurun_out/r2a/gpu.txt
 tools/dpx_bench gpurun_out/r2a/dpx_peak.json > gpurun_out/r2a/dpx_bench.txt 2>&1
+nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -o tools/cell_bench tools/cell_bench.cu
 tools/cell_bench gpurun_out/r2a/cell_bench.json > gpurun_out/r2a/cell_bench.txt 2>&1
 timeout 900 python -m pytest tests -m gpu -x -q > gpurun_out/r2a/pytest_gpu.txt 2>&1
 echo "pytest exit $?" >> gpurun_out/r2a/pytest_gpu.txt
