@@ -306,6 +306,17 @@ psb_db_t *psb_db_load(const char *path, const parasail_matrix_t *matrix);
  * best k of them on the host. */
 int psb_scan(const char *fn_name, const parasail_profile_t *profile, int open, int gap, const psb_db_t *db,
              psb_batch_t **out);
+/* the profile's query against selected subjects of a resident database: the alignments behind the hits of a
+ * psb_scan (psb_batch_topk gives the ids).  ids: n caller-order subject ids, repeats allowed, any order; or NULL
+ * with n == psb_db_count(db) for every subject.  fn_name: the profile grammar ("_profile"), with or without
+ * _trace / _stats; _table / _rowcol -> PSB_EUNSUPPORTED.  Result i belongs to ids[i]; the batch's arrays are
+ * those psb_align_pairs returns for the same name without "_profile" (cigar_off / cigar_ops / beg_* for _trace).
+ * The subjects are read out of the packed store on the device; nothing is uploaded but their ids. */
+int psb_db_align(const char *fn_name, const parasail_profile_t *profile, int open, int gap, const psb_db_t *db,
+                 const int64_t *ids, int64_t n, psb_batch_t **out);
+/* subject `id` of a resident database as matrix column indices (what the kernels align): writes min(len, cap)
+ * codes to `codes`, returns the subject's length, or a negative PSB_E* code */
+int64_t psb_db_subject(const psb_db_t *db, int64_t id, uint8_t *codes, int64_t cap);
 /* the same scan for a database that lives in HOST memory (pinned or pageable): the residues are cut
  * into pieces whose upload, device-side packing and scan are pipelined on two streams, so the
  * host-to-device copy hides under the kernels.  Nothing stays resident afterwards. */

@@ -5,7 +5,8 @@ Rust cannot be compiled in this environment, so the reference's safe wrapper
 `Alignment` getters) is mirrored here in Python with the same names, argument meaning and error
 behaviour, calling exactly the C symbols the Rust crate binds (include/parasail_b200.h).  The
 parity tests therefore read like [REF tests/test_parasail.rs].  Two entry points are new (north
-star): `Aligner.align_batch` (many pairs) and `Aligner.scan` (one profile vs a resident Database).
+star): `Aligner.align_batch` (many pairs) and `Aligner.scan` (one profile vs a resident Database), with
+`Aligner.search` / `Aligner.align_subjects` for the alignments of a scan's hits.
 
 All alignment work runs in hand-written CUDA (csrc/); nothing here computes a score on the CPU.
 """
@@ -465,6 +466,20 @@ class Database:
         if rc != 0:
             raise Error(f"psb_db_save failed ({rc}): {last_error()}")
 
+    def subject(self, i):
+        """subject `i` (caller order) read back out of the packed store (psb_db_subject), as the letters of the
+        matrix's alphabet: code c comes back as alphabet[c].  Lowercase input therefore comes back as the
+        alphabet's letter, and a residue the alphabet does not know as its wildcard (`*` for Matrix.create)."""
+        n = int(lib().psb_db_subject(self.inner, int(i), None, 0))
+        if n < 0:
+            raise DeviceError(f"psb_db_subject failed ({n}): {last_error()}")
+        codes = np.zeros(n, dtype=np.uint8)
+        rc = int(lib().psb_db_subject(self.inner, int(i), codes.ctypes.data_as(C.c_void_p), n))
+        if rc < 0:
+            raise DeviceError(f"psb_db_subject failed ({rc}): {last_error()}")
+        alphabet = np.frombuffer(self._keep.inner.contents.alphabet, dtype=np.uint8)
+        return alphabet[codes].tobytes()
+
     def __del__(self):
         try:
             if self.inner:
@@ -657,6 +672,38 @@ class Aligner:
         if rc_ != 0:
             raise DeviceError(f"psb_scan failed ({rc_}): {last_error()}")
         return BatchResult(out)
+
+    def align_subjects(self, database, ids=None):
+        """the aligner's profile against selected subjects of a resident Database (psb_db_align): row i belongs to
+        ids[i] (caller-order ids, any order, repeats allowed); ids=None aligns every subject.  With use_trace()
+        the rows carry CIGARs and begin coordinates, with a stats profile matches/similar/length."""
+        if self._profile.is_null():
+            raise Panic("align_subjects() needs an aligner built with .profile(...)")
+        if ids is None:
+            ptr, n = None, database.n
+        else:
+            ids = np.ascontiguousarray(ids, dtype=np.int64)
+            ptr, n = ids.ctypes.data_as(C.c_void_p), len(ids)
+        out = C.POINTER(CBatch)()
+        rc_ = lib().psb_db_align(self.fn_name.encode(), self._profile.inner, self.gap_open, self.gap_extend, database.inner,
+                                 ptr, n, C.byref(out))
+        if rc_ != 0:
+            raise DeviceError(f"psb_db_align failed ({rc_}): {last_error()}")
+        return BatchResult(out)
+
+    def search(self, database, k):
+        """scan the whole Database score-only, keep the k best subjects (ties by smaller id) and align those with this
+        aligner's own function: returns (ids, BatchResult) with row i belonging to ids[i]"""
+        if self._profile.is_null():
+            raise Panic("search() needs an aligner built with .profile(...)")
+        score_only = self.fn_name.replace("_trace", "").replace("_stats", "")
+        out = C.POINTER(CBatch)()
+        rc_ = lib().psb_scan(score_only.encode(), self._profile.inner, self.gap_open, self.gap_extend, database.inner,
+                             C.byref(out))
+        if rc_ != 0:
+            raise DeviceError(f"psb_scan failed ({rc_}): {last_error()}")
+        ids, _ = BatchResult(out).topk(k)
+        return ids, self.align_subjects(database, ids)
 
 
 def _scan_host(self, subjects):

@@ -721,7 +721,13 @@ static int run_pairs_range(const PairsRequest &req, int64_t lo, int64_t hi, psb_
         PSB_CUDA(cudaMemsetAsync(d_q.p, 0xff, qbytes, c.stream));  // no query residues: nothing "matches"
     else
         PSB_CUDA(upload_h2d(d_q.p, req.q_cat + q_lo, qbytes, c.stream));
-    PSB_CUDA(upload_h2d(d_r.p, req.r_cat + r_lo, (size_t)(r_hi - r_lo), c.stream));
+    DevMem d_rids;
+    if (req.r_db) {
+        PSB_TRY(d_rids.alloc((size_t)n * sizeof(int), c.stream));
+        PSB_CUDA(upload_h2d(d_rids.p, req.r_ids + lo, (size_t)n * sizeof(int), c.stream));
+    } else {
+        PSB_CUDA(upload_h2d(d_r.p, req.r_cat + r_lo, (size_t)(r_hi - r_lo), c.stream));
+    }
     if (q_two) PSB_CUDA(cudaMemcpyAsync(d_qoff.p, qoff2, sizeof(qoff2), cudaMemcpyHostToDevice, c.stream));
     else PSB_CUDA(upload_h2d(d_qoff.p, req.q_off + lo, ((size_t)n + 1) * sizeof(long long), c.stream));
     PSB_CUDA(upload_h2d(d_roff.p, req.r_off + lo, ((size_t)n + 1) * sizeof(long long), c.stream));
@@ -872,8 +878,17 @@ static int run_pairs_range(const PairsRequest &req, int64_t lo, int64_t hi, psb_
             map_residues_kernel<<<blocks, 256, 0, c.stream>>>(mp);
             c.launches++;
         }
-        mp.data = d_r.as<uint8_t>(); mp.n = (long long)(r_hi - r_lo);
-        map_residues_kernel<<<blocks, 256, 0, c.stream>>>(mp);
+        if (req.r_db) {
+            // the references straight out of the packed store: already matrix codes, written at the same biased
+            // offsets an upload would have put them
+            UnpackParams u;
+            u.words = req.r_db->d_words; u.word_off = req.r_db->d_word_off; u.ids = d_rids.as<int>(); u.inv_perm = req.r_db->d_inv_perm;
+            u.out_off = d_roff.as<long long>(); u.out = d_r.as<uint8_t>() - r_lo; u.n = n; u.bits = req.r_db->bits;
+            unpack_db_kernel<<<(unsigned)std::min<int64_t>((n + 7) / 8, blocks), 256, 0, c.stream>>>(u);
+        } else {
+            mp.data = d_r.as<uint8_t>(); mp.n = (long long)(r_hi - r_lo);
+            map_residues_kernel<<<blocks, 256, 0, c.stream>>>(mp);
+        }
         c.launches++;
     }
 
@@ -1112,7 +1127,7 @@ void free_batch(psb_batch_t *b) {
 
 int run_pairs(const PairsRequest &req, psb_batch_t **out) {
     if (out) *out = nullptr;
-    if (!out || !req.matrix || !req.r_cat || !req.r_off || req.n <= 0 || (!req.q_cat && req.matrix->type != PARASAIL_MATRIX_TYPE_PSSM)) {
+    if (!out || !req.matrix || !(req.r_cat || (req.r_db && req.r_ids)) || !req.r_off || req.n <= 0 || (!req.q_cat && req.matrix->type != PARASAIL_MATRIX_TYPE_PSSM)) {
         set_error("psb: NULL argument or empty batch");
         return PSB_EINVAL;
     }
@@ -1494,7 +1509,7 @@ static int scan_sw16(const FnConfig &cfg, const parasail_profile *prof, DevProfi
         PSB_CUDA(cudaMemsetAsync(d_ctl.p, 0, ((size_t)nroute * nstrips + 2) * sizeof(int), c.stream));
         PSB_CUDA(cudaStreamSynchronize(c.stream));  // `loff` is a host temporary
         UnpackParams u;
-        u.words = db->d_words; u.word_off = db->d_word_off; u.ids = nullptr; u.out_off = d_loff.as<long long>();
+        u.words = db->d_words; u.word_off = db->d_word_off; u.ids = nullptr; u.inv_perm = nullptr; u.out_off = d_loff.as<long long>();
         u.out = d_lbytes.as<uint8_t>(); u.n = nroute; u.bits = db->bits;
         unpack_db_kernel<<<(unsigned)std::min<int64_t>(nroute, 1024), 256, 0, c.stream>>>(u);
         Wave32Params w;
@@ -2020,7 +2035,7 @@ void psb_db_free(psb_db_t *db) {
     int cur = 0;
     cudaGetDevice(&cur);
     cudaSetDevice(db->device);
-    void *ptrs[] = {db->d_words, db->d_word_off, db->d_perm, db->d_len, db->d_res_off};
+    void *ptrs[] = {db->d_words, db->d_word_off, db->d_perm, db->d_len, db->d_res_off, db->d_inv_perm};
     for (void *p : ptrs) if (p) cudaFreeAsync(p, db->stream);
     cudaSetDevice(cur);
     delete db;
@@ -2098,6 +2113,35 @@ static int scan_check(const char *who, const char *fn_name, const parasail_profi
     if (cfg->trace || cfg->table || cfg->rowcol) { set_error(std::string(who) + ": trace/table/rowcol outputs are not available for database scans"); return PSB_EUNSUPPORTED; }
     return PSB_OK;
 }
+// what every call that reads a resident database's subjects by caller id checks: the calling thread's device holds it
+static int db_check(const char *who, const psb_db *db) {
+    PSB_TRY(ensure_ctx());
+    if (db->device != g_ctx.device) { set_error(std::string(who) + ": database lives on another device"); return PSB_EINVAL; }
+    if (db->host_len.empty()) { set_error(std::string(who) + ": the database has no subject lengths on the host"); return PSB_EUNSUPPORTED; }
+    return PSB_OK;
+}
+// The database's inverse permutation, built on first use: the scatter runs on db->stream, behind the sort/pack chain
+// psb_db_create queued there (it returns before that chain has finished), and that stream is synchronised before the
+// pointer is published.  So whoever sees the pointer -- any host thread, any stream -- also sees finished packed words.
+static int db_inv_perm(psb_db *db, int *launched) {
+    *launched = 0;
+    if (db->d_inv_perm) return PSB_OK;
+    std::lock_guard<std::mutex> lk(db->mu);
+    if (db->d_inv_perm) return PSB_OK;
+    int *inv = nullptr;
+    PSB_CUDA(cudaMallocAsync(&inv, (size_t)db->n * sizeof(int), db->stream));
+    invert_perm_kernel<<<(unsigned)std::min<int64_t>((db->n + 255) / 256, (int64_t)g_ctx.sms * 8), 256, 0, db->stream>>>(db->d_perm, db->n, inv);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaStreamSynchronize(db->stream);
+    if (e != cudaSuccess) {
+        cudaFreeAsync(inv, db->stream);
+        set_error(std::string("psb_db: inverse permutation: ") + cudaGetErrorString(e));
+        return PSB_ECUDA;
+    }
+    db->d_inv_perm = inv;
+    *launched = 1;
+    return PSB_OK;
+}
 }  // namespace psb
 
 extern "C" {
@@ -2132,6 +2176,86 @@ int psb_scan(const char *fn_name, const parasail_profile_t *profile, int open, i
             }
     *out = b;
     return PSB_OK;
+}
+
+int psb_db_align(const char *fn_name, const parasail_profile_t *profile, int open, int gap, const psb_db_t *db_c,
+                 const int64_t *ids, int64_t n, psb_batch_t **out) {
+    if (out) *out = nullptr;
+    FnConfig cfg;
+    if (!parse_fn_name(fn_name, &cfg) || !cfg.profile) { set_error(std::string("psb_db_align: not a profile function name: ") + (fn_name ? fn_name : "(null)")); return PSB_EINVAL; }
+    if (!profile) { set_error("psb_db_align: NULL profile"); return PSB_EINVAL; }
+    if (cfg.table || cfg.rowcol) { set_error("psb_db_align: _table/_rowcol outputs exist only on the single-pair API"); return PSB_EUNSUPPORTED; }
+    if (!db_c || !out) { set_error("psb_db_align: NULL argument"); return PSB_EINVAL; }
+    psb_db *db = const_cast<psb_db *>(db_c);
+    PSB_TRY(db_check("psb_db_align", db));
+    if (profile->matrix.size != db->msize || std::memcmp(profile->matrix.mapper, db->mapper, 256) != 0) {
+        set_error("psb_db_align: profile and database were built with different alphabets");
+        return PSB_EINVAL;
+    }
+    if (n <= 0 || (!ids && n != db->n)) {
+        set_error("psb_db_align: " + std::to_string(n) + " ids for a database of " + std::to_string(db->n) + " subjects");
+        return PSB_EINVAL;
+    }
+    // the pairs pass classifies, sorts and cuts by the references' lengths: offsets from the caller-order lengths
+    std::vector<int> rid((size_t)n);
+    std::vector<int64_t> r_off((size_t)n + 1);
+    r_off[0] = 0;
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t id = ids ? ids[i] : i;
+        if (id < 0 || id >= db->n) {
+            set_error("psb_db_align: ids[" + std::to_string(i) + "] = " + std::to_string(id) + " is not a subject of a database of " + std::to_string(db->n));
+            return PSB_EINVAL;
+        }
+        rid[(size_t)i] = (int)id;
+        r_off[(size_t)i + 1] = r_off[(size_t)i] + db->host_len[(size_t)id];
+    }
+    int first_use = 0;
+    PSB_TRY(db_inv_perm(db, &first_use));
+    const int64_t lq = (int64_t)profile->query.size();
+    const int64_t q_off[2] = {0, lq};
+    PairsRequest req;
+    req.cfg = cfg;
+    req.matrix = &profile->matrix; req.open = open; req.gap = gap;
+    req.q_cat = profile->query.data(); req.q_off = q_off; req.shared_query = true;
+    req.r_off = r_off.data(); req.n = n; req.r_db = db; req.r_ids = rid.data();
+    const int rc = run_pairs(req, out);
+    g_ctx.launches += first_use;
+    if (rc == PSB_OK && (cfg.width == 8 || cfg.width == 16)) {
+        psb_batch_t *b = *out;
+        for (int64_t i = 0; i < n; ++i)
+            if (saturates(cfg, profile->matrix, b->score[i], (int)lq, (int)(r_off[(size_t)i + 1] - r_off[(size_t)i]), open, gap)) {
+                b->saturated[i] = 1; b->score[i] = 0; b->end_query[i] = 0; b->end_ref[i] = 0;
+            }
+    }
+    return rc;
+}
+
+int64_t psb_db_subject(const psb_db_t *db_c, int64_t id, uint8_t *codes, int64_t cap) {
+    if (!db_c || cap < 0 || (cap > 0 && !codes)) { set_error("psb_db_subject: NULL argument or negative capacity"); return PSB_EINVAL; }
+    psb_db *db = const_cast<psb_db *>(db_c);
+    PSB_TRY(db_check("psb_db_subject", db));
+    if (id < 0 || id >= db->n) { set_error("psb_db_subject: id " + std::to_string(id) + " is not a subject of a database of " + std::to_string(db->n)); return PSB_EINVAL; }
+    int first_use = 0;
+    PSB_TRY(db_inv_perm(db, &first_use));
+    const int64_t len = db->host_len[(size_t)id];
+    if (cap == 0) return len;
+    Ctx &c = g_ctx;
+    const int sid = (int)id;
+    const long long off[2] = {0, (long long)len};
+    DevMem d_id, d_off, d_out;
+    PSB_TRY(d_id.alloc(sizeof(int), c.stream));
+    PSB_TRY(d_off.alloc(sizeof(off), c.stream));
+    PSB_TRY(d_out.alloc((size_t)len, c.stream));
+    PSB_CUDA(cudaMemcpyAsync(d_id.p, &sid, sizeof(int), cudaMemcpyHostToDevice, c.stream));
+    PSB_CUDA(cudaMemcpyAsync(d_off.p, off, sizeof(off), cudaMemcpyHostToDevice, c.stream));
+    UnpackParams u;
+    u.words = db->d_words; u.word_off = db->d_word_off; u.ids = d_id.as<int>(); u.inv_perm = db->d_inv_perm;
+    u.out_off = d_off.as<long long>(); u.out = d_out.as<uint8_t>(); u.n = 1; u.bits = db->bits;
+    unpack_db_kernel<<<1, 32, 0, c.stream>>>(u);
+    PSB_CUDA(cudaGetLastError());
+    PSB_CUDA(cudaMemcpyAsync(codes, d_out.p, (size_t)std::min(len, cap), cudaMemcpyDeviceToHost, c.stream));
+    PSB_CUDA(cudaStreamSynchronize(c.stream));   // (`sid` / `off` are host temporaries)
+    return len;
 }
 
 }  // extern "C"

@@ -78,10 +78,18 @@ PSB_KERNEL void pack_db_kernel(PackParams p) {
     }
 }
 
+// sorted position -> caller id (a database's permutation) inverted: inv[perm[s]] = s
+PSB_KERNEL void invert_perm_kernel(const int *perm, long long n, int *inv) {
+    const long long stride = (long long)grid_blocks() * threads_per_block();
+    for (long long s = (long long)block_id() * threads_per_block() + thread_in_block(); s < n; s += stride) inv[perm[s]] = (int)s;
+}
+
+// packed subjects -> matrix codes, one warp per subject
 struct UnpackParams {
     const unsigned *words;
     const long long *word_off;   // sorted order
-    const int *ids;              // which sorted subjects to unpack (NULL: all, 0..n-1)
+    const int *ids;              // which subjects to unpack (NULL: all sorted subjects, 0..n-1)
+    const int *inv_perm;         // non-NULL: `ids` are caller-order ids, resolved to sorted positions through it
     const long long *out_off;    // n+1 byte offsets of the outputs
     uint8_t *out;
     long long n;
@@ -94,7 +102,7 @@ PSB_KERNEL void unpack_db_kernel(UnpackParams p) {
     const long long nwarps = ((long long)grid_blocks() * threads_per_block()) >> 5;
     const int lane = lane_id();
     for (long long s = warp; s < p.n; s += nwarps) {
-        const long long sid = p.ids ? p.ids[s] : s;
+        const long long sid = p.ids ? (p.inv_perm ? p.inv_perm[p.ids[s]] : p.ids[s]) : s;
         const long long w0 = p.word_off[sid];
         const long long o0 = p.out_off[s];
         const int len = (int)(p.out_off[s + 1] - o0);

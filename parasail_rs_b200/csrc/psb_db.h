@@ -23,6 +23,7 @@ struct psb_db {
     int *d_perm = nullptr;            // sorted position -> caller's subject id
     int *d_len = nullptr;             // sorted order
     long long *d_res_off = nullptr;   // n+1 prefix sum of d_len: boundary lines of the strip-wise scan (built on first use)
+    int *d_inv_perm = nullptr;        // caller's subject id -> sorted position (built on first use by psb_db_align / psb_db_subject)
     std::mutex mu;
 };
 

@@ -112,6 +112,11 @@ struct PairsRequest {
     const uint8_t *r_cat = nullptr;
     const int64_t *r_off = nullptr;
     int64_t n = 0;
+    // references out of a resident database instead of r_cat (psb_db_align): pair i's reference is subject r_ids[i]
+    // (caller order), gathered from the packed store on the device; r_off still holds their offsets (from host_len).
+    // The database's inverse permutation must exist before run_pairs is called.
+    const psb_db_t *r_db = nullptr;
+    const int *r_ids = nullptr;
     // single-pair API extras (n == 1): full tables / last row+col / row-major trace bytes
     psb_result_extra *extra = nullptr;
     // single-pair API, `_trace`: the flag-byte block itself is wanted (the lazy trace-table export), so even a long
