@@ -404,7 +404,9 @@ static bool wave_walk_ok(const HostMatrix &m, int open, int gap, bool is_sw, int
     if (!wave32v3_range_ok(kWaveTraceK, 4, is_sw, lq, lr, m.max, m.min, open, gap)) return false;
     return wave_trace_bytes(lq, lr) + ((size_t)1 << 30) <= avail;
 }
-// what a new allocation can get: the driver's free figure + what the stream-ordered pool holds idle
+// what a new allocation can get: the driver's free figure + what the stream-ordered pool holds idle (0 if the driver
+// cannot say).  Counting only the former would make a figure that shrinks as the pool warms up: every call would then
+// cut its passes differently, ask for buffers of new sizes, grow the pool again ... -- calls of 2 s instead of 0.3 s.
 static size_t device_mem_available() {
     size_t free_b = 0, total_b = 0;
     if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) { cudaGetLastError(); return 0; }
@@ -418,36 +420,98 @@ static size_t device_mem_available() {
     return free_b;
 }
 
-static int launch_wave32(const Gotoh32Params &g, const HostMatrix &m, long long q_byte_off, int lq, long long r_byte_off, int lr, int out_index,
-                         const WaveWalk *ww = nullptr) {
-    Ctx &c = g_ctx;
-    // strips of 32*K rows: enough strips to occupy the chip, as few as possible beyond that
-    int K = lq / 512 >= 2 * c.sms ? 16 : (lq / 256 >= 2 * c.sms ? 8 : 4);
-    int wpb = kWarpsPerBlock;
-    const bool v2 = wave32_v2_ok(m, g.open, g.gap);
+// PSB_DEBUG_TIMING on the pairs path (inert without it): where the host time of a pass goes, the device time of its
+// marked launches and its timed region, as "[psb]" lines on stderr (tools/pairs_host_probe.py and
+// tools/db_align_probe.py read them).  One per pass, on the calling thread's stream.
+struct PassTimeline {
+    const bool on = std::getenv("PSB_DEBUG_TIMING") != nullptr;
+    std::chrono::steady_clock::time_point h_last = std::chrono::steady_clock::now();
+    std::string h_line;
+    struct Mark { std::string what; cudaEvent_t begin, end; };
+    std::vector<Mark> marks;
+    PassTimeline() = default;
+    PassTimeline(const PassTimeline &) = delete;
+    PassTimeline &operator=(const PassTimeline &) = delete;
+    ~PassTimeline() {
+        for (Mark &k : marks) { cudaEventDestroy(k.begin); if (k.end) cudaEventDestroy(k.end); }
+    }
+    void phase(const char *what) {
+        if (!on) return;
+        const auto now = std::chrono::steady_clock::now();
+        char buf[64];
+        std::snprintf(buf, sizeof buf, " %s %.3f", what, std::chrono::duration<double, std::milli>(now - h_last).count());
+        h_line += buf; h_last = now;
+    }
+    static cudaEvent_t record() {
+        cudaEvent_t ev = nullptr;
+        cudaEventCreate(&ev);
+        cudaEventRecord(ev, g_ctx.stream);
+        return ev;
+    }
+    void begin(std::string what) { if (on) marks.push_back({std::move(what), record(), nullptr}); }
+    void end() { if (on) marks.back().end = record(); }
+    // the device time of the last mark, taken off the list (waits for it)
+    float take_last_ms() {
+        const Mark k = marks.back();
+        marks.pop_back();
+        float t = 0.f;
+        cudaEventSynchronize(k.end);
+        cudaEventElapsedTime(&t, k.begin, k.end);
+        cudaEventDestroy(k.begin); cudaEventDestroy(k.end);
+        return t;
+    }
+    void report(int64_t lo, int64_t hi, float ms) const {
+        if (!on) return;
+        std::fprintf(stderr, "[psb] pass %lld..%lld host ms:%s\n", (long long)lo, (long long)hi, h_line.c_str());
+        for (const Mark &k : marks) {
+            float t = 0.f;
+            if (k.end && cudaEventElapsedTime(&t, k.begin, k.end) == cudaSuccess)
+                std::fprintf(stderr, "[psb] %-48s %9.3f ms\n", k.what.c_str(), t);
+        }
+        std::fprintf(stderr, "[psb] pass of %lld pairs: timed region %.3f ms\n", (long long)(hi - lo), ms);
+    }
+};
+
+// launch shape of one long pair: generation (1 and 2: wave32_fn; 3: the column-blocked wave32v3_fn), rows per lane
+// and warps per CTA
+struct WaveShape {
+    const void *fn;
+    int K, wpb, gen;
+};
+static WaveShape wave_shape(const HostMatrix &m, int open, int gap, bool is_sw, int lq, int lr, bool traced) {
+    const int sms = g_ctx.sms;
+    auto strips = [lq](int K) { return (lq + 32 * K - 1) / (32 * K); };
     // the column-blocked generation (K x 4 tiles per lane and step) has the shortest critical path,
     // Lq/K + Lr/4 steps: every mode takes it when its preconditions hold (C5 local 46.5 -> 21.1 ms;
-    // 50 kb x 50 kb global 26.6 -> 19.3 ms)
-    const bool is_sw = g.mode == MODE_SW;
-    bool v3 = v2;
+    // 50 kb x 50 kb global 26.6 -> 19.3 ms).  Measured on C5 (tools/c5_probe.py): a step costs about the same for 4
+    // and 8 rows per lane (a warp alone on its scheduler is bound by per-step latencies) and twice as much for 16,
+    // while every strip adds ~34 steps to the path: 8 rows, 4 warps per CTA (one per scheduler)
+    WaveShape s{nullptr, 8, kWarpsPerBlock, wave32_v2_ok(m, open, gap) ? 3 : 1};
     // experiment knobs (tools/c5_probe.py): generation, rows per lane and warps per CTA of the launch
-    if (const char *ev = std::getenv("PSB_WAVE_GEN")) { if (std::atoi(ev) == 2) v3 = false; }
-    if (v3) {
-        // measured on C5 (tools/c5_probe.py): a step costs about the same for 4 and 8 rows per lane (a
-        // warp alone on its scheduler is bound by per-step latencies) and twice as much for 16, while
-        // every strip adds ~34 steps to the path: 8 rows, 4 warps per CTA (one per scheduler)
-        K = 8; wpb = 4;
-        if ((lq + 32 * K - 1) / (32 * K) > c.sms * 16) K = 16;
-        if ((lq + 32 * K - 1) / (32 * K) > c.sms * 16 || !wave32v3_range_ok(K, 4, is_sw, lq, lr, m.max, m.min, g.open, g.gap)) v3 = false;
-        if (!v3) { K = lq / 512 >= 2 * c.sms ? 16 : (lq / 256 >= 2 * c.sms ? 8 : 4); wpb = kWarpsPerBlock; }
+    if (const char *ev = std::getenv("PSB_WAVE_GEN")) { if (std::atoi(ev) == 2 && s.gen == 3) s.gen = 2; }
+    if (s.gen == 3) {
+        if (strips(s.K) > sms * 16) s.K = 16;
+        if (strips(s.K) > sms * 16 || !wave32v3_range_ok(s.K, 4, is_sw, lq, lr, m.max, m.min, open, gap)) s.gen = 2;
     }
+    // the older generations: strips of 32*K rows, enough strips to occupy the chip, as few as possible beyond that
+    if (s.gen < 3) s.K = lq / 512 >= 2 * sms ? 16 : (lq / 256 >= 2 * sms ? 8 : 4);
     if (const char *ev = std::getenv("PSB_WAVE_K")) {
         const int k = std::atoi(ev);
-        if ((k == 1 || k == 2 || k == 4 || k == 8 || k == 16) && (!v3 || k >= 4)) K = k;
+        if ((k == 1 || k == 2 || k == 4 || k == 8 || k == 16) && (s.gen < 3 || k >= 4)) s.K = k;
     }
-    if (const char *ev = std::getenv("PSB_WAVE_WARPS")) { const int w = std::atoi(ev); if (w >= 1 && w <= 32) wpb = w; }
-    if (ww) { v3 = true; K = kWaveTraceK; }   // (wave_walk_ok held when the pair was routed here)
-    const void *fn = v3 ? wave32v3_fn(K, is_sw, ww != nullptr) : wave32_fn(K, v2);
+    if (const char *ev = std::getenv("PSB_WAVE_WARPS")) { const int w = std::atoi(ev); if (w >= 1 && w <= 32) s.wpb = w; }
+    if (traced) { s.gen = 3; s.K = kWaveTraceK; }   // (wave_walk_ok held when the pair was routed here)
+    s.fn = s.gen == 3 ? wave32v3_fn(s.K, is_sw, traced) : wave32_fn(s.K, s.gen == 2);
+    return s;
+}
+
+static int launch_wave32(const Gotoh32Params &g, const HostMatrix &m, long long q_byte_off, int lq, long long r_byte_off, int lr, int out_index,
+                         const WaveWalk *ww, PassTimeline &tl) {
+    Ctx &c = g_ctx;
+    const bool is_sw = g.mode == MODE_SW;
+    const WaveShape s = wave_shape(m, g.open, g.gap, is_sw, lq, lr, ww != nullptr);
+    const int K = s.K, wpb = s.wpb;
+    const bool v3 = s.gen == 3;
     const int nstrips = (lq + 32 * K - 1) / (32 * K);
     DevMem d_bnd, d_ctl, d_cand, d_th, d_tb;
     if (ww) {
@@ -468,16 +532,16 @@ static int launch_wave32(const Gotoh32Params &g, const HostMatrix &m, long long 
     p.bnd = d_bnd.as<int>(); p.progress = d_ctl.as<int>() + 1; p.next_strip = d_ctl.as<int>(); p.cand = d_cand.as<int>();
     p.multi_n = 0; p.r_off = nullptr;
     p.trace_h = d_th.as<uint4>(); p.trace_bits = d_tb.as<uint2>();
-    const size_t smem = v3 ? wave32v3_smem_bytes(g.size, wpb, K) : (v2 ? wave32v2_smem_bytes(g.size, wpb) : wave32_smem_bytes(g.size, wpb));
-    if (smem > 48 * 1024) PSB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const size_t smem = v3 ? wave32v3_smem_bytes(g.size, wpb, K) : (s.gen == 2 ? wave32v2_smem_bytes(g.size, wpb) : wave32_smem_bytes(g.size, wpb));
+    if (smem > 48 * 1024) PSB_CUDA(cudaFuncSetAttribute(s.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
-    PSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, wpb * 32, smem));
+    PSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, s.fn, wpb * 32, smem));
     if (per_sm < 1) per_sm = 1;
     // every launched warp must be resident at once: the strips wait on one another
     long long blocks = std::min<long long>((nstrips + wpb - 1) / wpb, (long long)c.sms * per_sm);
     if (blocks < 1) blocks = 1;
     void *args[] = {&p};
-    PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(wpb * 32), args, smem, c.stream));
+    PSB_CUDA(cudaLaunchKernel(s.fn, dim3((unsigned)blocks), dim3(wpb * 32), args, smem, c.stream));
     WaveReduceParams r;
     r.cand = d_cand.as<int>(); r.nstrips = nstrips; r.mode = g.mode; r.s1_end = g.s1_end; r.s2_end = g.s2_end; r.Lr = lr;
     r.score = g.score + out_index; r.end_query = g.end_query + out_index; r.end_ref = g.end_ref + out_index;
@@ -495,23 +559,17 @@ static int launch_wave32(const Gotoh32Params &g, const HostMatrix &m, long long 
         w.rev_ops = ww->rev_ops; w.rev_off = ww->rev_off; w.nops = ww->nops; w.beg_query = ww->beg_query; w.beg_ref = ww->beg_ref;
         w.matches = g.matches; w.similar = g.similar; w.length = g.length;
         const size_t wsm = walk32_smem_bytes(g.size);
-        const bool dbg = std::getenv("PSB_DEBUG_TIMING") != nullptr;
-        cudaEvent_t e0 = nullptr, e1 = nullptr;
-        if (dbg) { cudaEventCreate(&e0); cudaEventCreate(&e1); cudaEventRecord(e0, c.stream); }
+        tl.begin("walk32");
         if (ww->stats) walk32_kernel<true><<<1, 32, wsm, c.stream>>>(w);
         else walk32_kernel<false><<<1, 32, wsm, c.stream>>>(w);
         PSB_CUDA(cudaGetLastError());
         c.launches++;
-        if (dbg) {
-            cudaEventRecord(e1, c.stream);
-            cudaEventSynchronize(e1);
-            float t = 0.f;
-            cudaEventElapsedTime(&t, e0, e1);
-            std::fprintf(stderr, "[psb] walk32 of a %d x %d pair: %.3f ms (trace %.2f GB)\n", lq, lr, t, (double)wave_trace_bytes(lq, lr) / 1e9);
-            cudaEventDestroy(e0); cudaEventDestroy(e1);
-        }
+        tl.end();
+        if (tl.on)
+            std::fprintf(stderr, "[psb] walk32 of a %d x %d pair: %.3f ms (trace %.2f GB)\n", lq, lr, tl.take_last_ms(),
+                         (double)wave_trace_bytes(lq, lr) / 1e9);
     }
-    if (v3 && std::getenv("PSB_DEBUG_TIMING")) {
+    if (v3 && tl.on) {
         // per-strip timeline of the column-blocked kernel: claimed / first columns available / done (us)
         std::vector<int> h((size_t)nstrips * 8);
         PSB_CUDA(cudaMemcpyAsync(h.data(), d_cand.p, h.size() * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
@@ -573,10 +631,8 @@ struct PassCutter {
                 const int64_t lr = req.r_off[hi + 1] - req.r_off[hi];
                 int64_t need;
                 if (p16_scheme && lq <= 512) need = (lr + 32) * (lq + 96) * 5 / 4 + 8 * (lq + lr);   // one byte of H per cell of the padded frame
-                else if (req.cfg.trace) {
-                    const int K = 16;  // upper bound on rows per lane of any class
-                    need = ((lq + 32 * K - 1) / (32 * K)) * (lr + 31) * 32 * K + 8 * (lq + lr);
-                } else need = 0;
+                else if (req.cfg.trace) need = trace_block_cells(16, lq, lr) + 8 * (lq + lr);   // (16: the most rows per lane of any class)
+                else need = 0;
                 if (hi > lo && (bytes + need > budget || res_upto(hi + 1) - res_lo > pass_res)) break;
                 bytes += need; ++hi;
             }
@@ -606,81 +662,100 @@ __global__ void rev_off_kernel(const long long *q_off, const long long *r_off, i
         out[i] = (q_shared ? i * qlen : q_off[i] - q_base) + (r_off[i] - r_base) + 2 * i;
 }
 
-static int run_pairs_range(const PairsRequest &req, int64_t lo, int64_t hi, psb_batch_t *b, PassOut *po) {
-    Ctx &c = g_ctx;
-    const int launches_at_entry = c.launches;
-    // PSB_DEBUG_TIMING: where the HOST time of a pass goes
-    const bool host_dbg = std::getenv("PSB_DEBUG_TIMING") != nullptr;
-    auto h_last = std::chrono::steady_clock::now();
-    std::string h_line;
-    auto hphase = [&](const char *what) {
-        if (!host_dbg) return;
-        const auto now = std::chrono::steady_clock::now();
-        char buf[64];
-        std::snprintf(buf, sizeof buf, " %s %.3f", what, std::chrono::duration<double, std::milli>(now - h_last).count());
-        h_line += buf; h_last = now;
-    };
+// the packed 16-bit path (kern_pairs16.cuh) may take this request's scoring scheme: not switched off (PSB_NO_P16),
+// within the static 16-bit bound, and no explicit 32/64-bit width asked for.  Each caller adds its own conditions.
+static bool p16_allowed(const PairsRequest &req) {
+    const HostMatrix &m = *req.matrix;
+    return !std::getenv("PSB_NO_P16") && pairs16_scheme_ok(m.size, m.min, m.max, req.open, req.gap, m.type == PARASAIL_MATRIX_TYPE_PSSM) &&
+           req.cfg.width != 32 && req.cfg.width != 64;
+}
+
+// which kernel each pair of a pass goes to (pair ids count from the pass's first pair)
+struct PassPlan {
+    const PairsRequest *req = nullptr;
+    int64_t lo = 0, hi = 0, n = 0;
+    int64_t q_lo = 0, q_hi = 0, r_lo = 0, r_hi = 0;   // the pass's residues in the caller's arrays
+    bool pssm = false, q_two = false;                 // q_two: one query for every pair (offsets {0, qbytes})
+    size_t qbytes = 0;
+    bool want_table = false, banded = false, fine = false;
+    ClassTable ct{};
+    bool p16_on = false, p16_walk = false;
+    std::vector<int> c16_of;                  // query length -> packed class (-1: none)
+    std::vector<std::vector<int>> p16_ids;    // pairs of each packed 16-bit class
+    long long n_p16 = 0;
+    std::vector<std::vector<int>> cls;        // pairs of each 32-bit class
+    std::vector<int> wave_ids;                // long pairs: spread over the whole GPU one at a time
+    bool uniform = true;                      // every pair of the same lengths and class: no ordering needed
+    int first_cls = -1;
+    int max_lr_multistrip = 0;
+    bool wide_stats = false;                  // the strip-boundary scratch carries the wide statistics word
+    double cells = 0;
+    int lq(int64_t i) const {
+        return pssm ? req->matrix->length : (int)(req->shared_query ? q_hi - q_lo : req->q_off[lo + i + 1] - req->q_off[lo + i]);
+    }
+    int lr(int64_t i) const { return (int)(req->r_off[lo + i + 1] - req->r_off[lo + i]); }
+    // longest reference first: a dynamic queue then ends on short pairs, and the pairs of a packed word (and the words
+    // of a warp) are of similar size
+    void longest_first(std::vector<int> &ids) const {
+        std::stable_sort(ids.begin(), ids.end(), [this](int a, int b) { return lr(a) > lr(b); });
+    }
+};
+
+static int plan_pass(const PairsRequest &req, int64_t lo, int64_t hi, PassPlan *plan) {
+    PassPlan &P = *plan;
     const FnConfig &cfg = req.cfg;
     const HostMatrix &m = *req.matrix;
-    const int64_t n = hi - lo;
-    const bool pssm = m.type == PARASAIL_MATRIX_TYPE_PSSM;
-    const bool want_table = req.extra && (cfg.table || cfg.rowcol);
-    const bool want_trace = cfg.trace;
-
-    // lengths, classes, byte ranges
-    const int64_t q_lo = req.shared_query ? req.q_off[0] : req.q_off[lo];
-    const int64_t q_hi = req.shared_query ? req.q_off[1] : req.q_off[hi];
-    const int64_t r_lo = req.r_off[lo], r_hi = req.r_off[hi];
-    const bool banded = cfg.band > 0 && cfg.mode == MODE_NW && n == 1 && !cfg.stats && !cfg.trace && !want_table;
-    const bool fine = gotoh32_profile_ok(m.size, m.min, m.max, req.open, pssm) && !want_table && !banded;
-    const ClassTable ct = class_table(fine);
-    std::vector<std::vector<int>> cls(kNumClass);
-    // packed 16-bit path (kern_pairs16.cuh): pairs whose scoring scheme and lengths pass the static 16-bit
-    // bound; `_stats` results come from the trace walk there.  Explicit 32/64-bit requests, table outputs and
-    // the single-pair trace-table export stay on the 32-bit kernels.
-    const bool p16_walk = cfg.trace || cfg.stats;
-    const bool p16_on = !std::getenv("PSB_NO_P16") && pairs16_scheme_ok(m.size, m.min, m.max, req.open, req.gap, pssm) && !want_table &&
-                        !banded && cfg.width != 32 && cfg.width != 64 && !(req.extra && cfg.trace) &&
-                        (!p16_walk || pairs16_trace_ok(m.min, m.max, req.open));
-    std::vector<std::vector<int>> p16_ids(p16_on ? p16_num_classes() : 0);
-    long long n_p16 = 0;
-    std::vector<int> wave_ids;   // long pairs: spread over the whole GPU one at a time
-    size_t wave_avail = ~(size_t)0;   // device memory a traced wavefront launch may use (queried on the first long pair)
-    int max_lr_multistrip = 0;
-    int max_sum = 0, max_min = 0;
-    bool uniform = true;
-    int first_cls = -1;
-    long long first_cells = -1;
-    int first_lq = -1, first_lr = -1;
-    // query length -> packed class.  Wide (32-lane) groups halve the profile bytes per warp: taken when the
-    // narrow class would leave fewer than 8 warps per SM (protein alphabets, queries beyond ~200 residues)
-    std::vector<int> c16_of(513, -1);
-    if (p16_on) {
+    P.req = &req; P.lo = lo; P.hi = hi; P.n = hi - lo;
+    P.pssm = m.type == PARASAIL_MATRIX_TYPE_PSSM;
+    P.q_lo = req.shared_query ? req.q_off[0] : req.q_off[lo];
+    P.q_hi = req.shared_query ? req.q_off[1] : req.q_off[hi];
+    P.r_lo = req.r_off[lo]; P.r_hi = req.r_off[hi];
+    P.q_two = req.shared_query || P.pssm;
+    P.qbytes = P.pssm ? (size_t)m.length : (size_t)(P.q_hi - P.q_lo);
+    P.want_table = req.extra && (cfg.table || cfg.rowcol);
+    P.banded = cfg.band > 0 && cfg.mode == MODE_NW && P.n == 1 && !cfg.stats && !cfg.trace && !P.want_table;
+    P.fine = gotoh32_profile_ok(m.size, m.min, m.max, req.open, P.pssm) && !P.want_table && !P.banded;
+    P.ct = class_table(P.fine);
+    P.cls.resize(kNumClass);
+    // packed 16-bit path: pairs whose scoring scheme and lengths pass the static 16-bit bound; `_stats` results come
+    // from the trace walk there.  Explicit 32/64-bit requests, table outputs and the single-pair trace-table export
+    // stay on the 32-bit kernels.
+    P.p16_walk = cfg.trace || cfg.stats;
+    P.p16_on = p16_allowed(req) && !P.want_table && !P.banded && !(req.extra && cfg.trace) &&
+               (!P.p16_walk || pairs16_trace_ok(m.min, m.max, req.open));
+    P.p16_ids.resize(P.p16_on ? p16_num_classes() : 0);
+    // Wide (32-lane) groups halve the profile bytes per warp: taken when the narrow class would leave fewer than 8
+    // warps per SM (protein alphabets, queries beyond ~200 residues)
+    P.c16_of.assign(513, -1);
+    if (P.p16_on) {
         const char *ev = std::getenv("PSB_P16_WIDE");
         for (int lq = 1; lq <= 512; ++lq) {
             const int narrow = p16_pick_class(lq, false);
             bool wide = narrow >= 0 && 227 * 1024 / pairs16_warp_smem(p16_class(narrow).K, m.size + 1, cfg.mode == MODE_SW) < 8;
             if (ev) wide = std::atoi(ev) != 0;
-            c16_of[lq] = p16_pick_class(lq, wide);
+            P.c16_of[lq] = p16_pick_class(lq, wide);
         }
     }
-    for (int64_t i = 0; i < n; ++i) {
-        const int lq = pssm ? m.length : (int)(req.shared_query ? q_hi - q_lo : req.q_off[lo + i + 1] - req.q_off[lo + i]);
-        const int lr = (int)(req.r_off[lo + i + 1] - req.r_off[lo + i]);
+    size_t wave_avail = ~(size_t)0;   // device memory a traced wavefront launch may use (queried on the first long pair)
+    int max_sum = 0, max_min = 0;
+    long long first_cells = -1;
+    int first_lq = -1, first_lr = -1;
+    for (int64_t i = 0; i < P.n; ++i) {
+        const int lq = P.lq(i), lr = P.lr(i);
         if (lq <= 0 || lr <= 0) { set_error("empty sequence in batch (pair " + std::to_string(lo + i) + ")"); return PSB_EINVAL; }
         if (first_lq < 0) { first_lq = lq; first_lr = lr; }
-        else if (lq != first_lq || lr != first_lr) uniform = false;
-        if (p16_on && lq <= 512) {
-            const int c16 = c16_of[lq];
+        else if (lq != first_lq || lr != first_lr) P.uniform = false;
+        if (P.p16_on && lq <= 512) {
+            const int c16 = P.c16_of[lq];
             if (c16 >= 0 && pairs16_fits(p16_class(c16).G * p16_class(c16).K, lq, lr, m.max, m.min, req.open, req.gap, cfg.mode == MODE_SW)) {
-                p16_ids[c16].push_back((int)i);
-                ++n_p16;
-                po->cells += (double)lq * lr;
+                P.p16_ids[c16].push_back((int)i);
+                ++P.n_p16;
+                P.cells += (double)lq * lr;
                 continue;
             }
         }
-        const int cl = class_of_len(ct, lq);
-        bool wave = lq >= kWaveMinLq && lr >= 64 && !pssm && !(req.extra && (cfg.table || cfg.rowcol || (cfg.trace && req.want_flag_bytes))) && !banded;
+        const int cl = class_of_len(P.ct, lq);
+        bool wave = lq >= kWaveMinLq && lr >= 64 && !P.pssm && !(req.extra && (cfg.table || cfg.rowcol || (cfg.trace && req.want_flag_bytes))) && !P.banded;
         if (wave && (cfg.stats || cfg.trace)) {
             // with traceback / statistics: the traced wavefront launch + walk32_kernel when its preconditions hold
             // and its 1.25 bytes per cell fit (the single-pair API's trace-table export needs the flag bytes of the
@@ -688,402 +763,447 @@ static int run_pairs_range(const PairsRequest &req, int64_t lo, int64_t hi, psb_
             if (wave_avail == ~(size_t)0) wave_avail = device_mem_available();
             wave = wave_walk_ok(m, req.open, req.gap, cfg.mode == MODE_SW, lq, lr, wave_avail);
         }
-        if (wave) { wave_ids.push_back((int)i); uniform = false; }
-        else cls[cl].push_back((int)i);
-        if (!wave && lq > 32 * ct.k[cl]) max_lr_multistrip = std::max(max_lr_multistrip, lr);
+        if (wave) { P.wave_ids.push_back((int)i); P.uniform = false; }
+        else P.cls[cl].push_back((int)i);
+        if (!wave && lq > 32 * P.ct.k[cl]) P.max_lr_multistrip = std::max(P.max_lr_multistrip, lr);
         max_sum = std::max(max_sum, lq + lr);
         max_min = std::max(max_min, std::min(lq, lr));
         const long long cells = (long long)lq * lr;
-        if (first_cls < 0) { first_cls = cl; first_cells = cells; }
-        else if (cl != first_cls || cells != first_cells) uniform = false;
-        po->cells += (double)cells;
+        if (P.first_cls < 0) { P.first_cls = cl; first_cells = cells; }
+        else if (cl != P.first_cls || cells != first_cells) P.uniform = false;
+        P.cells += (double)cells;
     }
     // the coarse family carries only the wide statistics word: the strip-boundary scratch is sized for it
-    const bool wide_stats = !(max_min < 1024 && max_sum < 4096) || !fine;
-    hphase("classify");
+    P.wide_stats = !(max_min < 1024 && max_sum < 4096) || !P.fine;
+    return PSB_OK;
+}
 
-    // upload residues + offsets (relative to this range) and map them to matrix columns
-    DevMem d_q, d_r, d_qoff, d_roff, d_matrix;
-    const size_t qbytes = pssm ? (size_t)m.length : (size_t)(q_hi - q_lo);
-    PSB_TRY(d_q.alloc(qbytes, c.stream));
-    PSB_TRY(d_r.alloc((size_t)(r_hi - r_lo), c.stream));
+// the buffers of a pass that outlive a stage.  The driver owns them: device buffers go back to the pool on the stream
+// when the pass returns (after its last synchronise), and the host vectors are the sources of queued copies.
+struct PassBufs {
+    DevMem d_q, d_r, d_qoff, d_roff, d_matrix, d_rids;
+    DevMem d_out[6], d_counter, d_bnd;
+    DevMem d_traceoff, d_tab[4], d_revoff, d_nops, d_beg[2];
+    KeptMem d_trace{0}, d_rev{1};
+    std::vector<long long> trace_off;   // pairs on the 32-bit kernels: offset of the pair's trace / table block
+    long long trace_total = 0;
+    Gotoh32Params p;                    // the pass's device pointers, shared by every launch
+    DevMem d_items, d_toff16, d_slot16, d_ids16, d_mat8, d_cnt16;
+    KeptMem d_trace16{2};
+    std::vector<int> h_items, h_slot16, h_ids16;
+    std::vector<long long> h_toff16;
+    std::vector<int8_t> h_mat8 = std::vector<int8_t>(33 * 32);
+    std::vector<int> cls_item0, cls_id0;   // first item / pair of each packed class in d_items / d_ids16
+    std::vector<DevMem> d_orders = std::vector<DevMem>(kNumClass);
+    DevMem d_csroff, d_scan_tmp;
+};
+
+// upload residues + offsets (relative to this range) and the matrix; references out of a resident database: their ids
+static int upload_pass(const PairsRequest &req, const PassPlan &P, PassBufs &B) {
+    Ctx &c = g_ctx;
+    const HostMatrix &m = *req.matrix;
+    const int64_t n = P.n, lo = P.lo;
+    PSB_TRY(B.d_q.alloc(P.qbytes, c.stream));
+    PSB_TRY(B.d_r.alloc((size_t)(P.r_hi - P.r_lo), c.stream));
     // the offsets go up as the caller gave them (absolute): the device pointers are biased by the range's first
     // byte instead, so that base + off[pair] lands inside this pass's upload (no per-pair pass to make them relative)
     static_assert(sizeof(int64_t) == sizeof(long long), "offset arrays are uploaded as they are");
-    const bool q_two = req.shared_query || pssm;
-    const long long qoff2[2] = {0, (long long)qbytes};
-    PSB_TRY(d_qoff.alloc((q_two ? 2 : (size_t)n + 1) * sizeof(long long), c.stream));
-    PSB_TRY(d_roff.alloc(((size_t)n + 1) * sizeof(long long), c.stream));
-    PSB_TRY(d_matrix.alloc(m.table.size() * sizeof(int), c.stream));
-    if (pssm && m.query.size() == (size_t)m.length)
-        PSB_CUDA(cudaMemcpyAsync(d_q.p, m.query.data(), qbytes, cudaMemcpyHostToDevice, c.stream));
-    else if (pssm)
-        PSB_CUDA(cudaMemsetAsync(d_q.p, 0xff, qbytes, c.stream));  // no query residues: nothing "matches"
+    const long long qoff2[2] = {0, (long long)P.qbytes};
+    PSB_TRY(B.d_qoff.alloc((P.q_two ? 2 : (size_t)n + 1) * sizeof(long long), c.stream));
+    PSB_TRY(B.d_roff.alloc(((size_t)n + 1) * sizeof(long long), c.stream));
+    PSB_TRY(B.d_matrix.alloc(m.table.size() * sizeof(int), c.stream));
+    if (P.pssm && m.query.size() == (size_t)m.length)
+        PSB_CUDA(cudaMemcpyAsync(B.d_q.p, m.query.data(), P.qbytes, cudaMemcpyHostToDevice, c.stream));
+    else if (P.pssm)
+        PSB_CUDA(cudaMemsetAsync(B.d_q.p, 0xff, P.qbytes, c.stream));  // no query residues: nothing "matches"
     else
-        PSB_CUDA(upload_h2d(d_q.p, req.q_cat + q_lo, qbytes, c.stream));
-    DevMem d_rids;
+        PSB_CUDA(upload_h2d(B.d_q.p, req.q_cat + P.q_lo, P.qbytes, c.stream));
     if (req.r_db) {
-        PSB_TRY(d_rids.alloc((size_t)n * sizeof(int), c.stream));
-        PSB_CUDA(upload_h2d(d_rids.p, req.r_ids + lo, (size_t)n * sizeof(int), c.stream));
+        PSB_TRY(B.d_rids.alloc((size_t)n * sizeof(int), c.stream));
+        PSB_CUDA(upload_h2d(B.d_rids.p, req.r_ids + lo, (size_t)n * sizeof(int), c.stream));
     } else {
-        PSB_CUDA(upload_h2d(d_r.p, req.r_cat + r_lo, (size_t)(r_hi - r_lo), c.stream));
+        PSB_CUDA(upload_h2d(B.d_r.p, req.r_cat + P.r_lo, (size_t)(P.r_hi - P.r_lo), c.stream));
     }
-    if (q_two) PSB_CUDA(cudaMemcpyAsync(d_qoff.p, qoff2, sizeof(qoff2), cudaMemcpyHostToDevice, c.stream));
-    else PSB_CUDA(upload_h2d(d_qoff.p, req.q_off + lo, ((size_t)n + 1) * sizeof(long long), c.stream));
-    PSB_CUDA(upload_h2d(d_roff.p, req.r_off + lo, ((size_t)n + 1) * sizeof(long long), c.stream));
-    PSB_CUDA(cudaMemcpyAsync(d_matrix.p, m.table.data(), m.table.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
-    hphase("uploads");
-    // outputs
-    DevMem d_out[6], d_counter, d_bnd;
-    const int nout = cfg.stats || want_table ? 6 : 3;
-    for (int k = 0; k < nout; ++k) PSB_TRY(d_out[k].alloc((size_t)n * sizeof(int), c.stream));
-    PSB_TRY(d_counter.alloc(sizeof(int) * (kNumClass + 1), c.stream));
-    PSB_CUDA(cudaMemsetAsync(d_counter.p, 0, sizeof(int) * (kNumClass + 1), c.stream));
-    const bool stats_kernel = cfg.stats || want_table;
-    const int bnd_words_per_col = 2 + (stats_kernel ? 2 * ((wide_stats || want_table) ? 2 : 1) : 0);
-    const long long bnd_stride = (long long)max_lr_multistrip * bnd_words_per_col;
-    if (bnd_stride > 0) PSB_TRY(d_bnd.alloc((size_t)(bnd_stride * max_grid_warps(n)) * sizeof(int), c.stream));
+    if (P.q_two) PSB_CUDA(cudaMemcpyAsync(B.d_qoff.p, qoff2, sizeof(qoff2), cudaMemcpyHostToDevice, c.stream));
+    else PSB_CUDA(upload_h2d(B.d_qoff.p, req.q_off + lo, ((size_t)n + 1) * sizeof(long long), c.stream));
+    PSB_CUDA(upload_h2d(B.d_roff.p, req.r_off + lo, ((size_t)n + 1) * sizeof(long long), c.stream));
+    PSB_CUDA(cudaMemcpyAsync(B.d_matrix.p, m.table.data(), m.table.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
+    return PSB_OK;
+}
 
-    // trace / table blocks: [strip][step][lane][K] per pair
-    DevMem d_traceoff, d_tab[4], d_revoff, d_nops, d_beg[2];
-    KeptMem d_trace(0), d_rev(1);
-    std::vector<long long> trace_off;
-    long long trace_total = 0;
+// outputs, strip-boundary scratch, the trace / table blocks of the pairs on the 32-bit kernels and the CIGAR scratch
+// of the device-side walks; fills the pass's Gotoh32Params
+static int alloc_pass(const PairsRequest &req, const PassPlan &P, PassBufs &B) {
+    Ctx &c = g_ctx;
+    const FnConfig &cfg = req.cfg;
+    const HostMatrix &m = *req.matrix;
+    const int64_t n = P.n;
+    const int nout = cfg.stats || P.want_table ? 6 : 3;
+    for (int k = 0; k < nout; ++k) PSB_TRY(B.d_out[k].alloc((size_t)n * sizeof(int), c.stream));
+    PSB_TRY(B.d_counter.alloc(sizeof(int) * (kNumClass + 1), c.stream));
+    PSB_CUDA(cudaMemsetAsync(B.d_counter.p, 0, sizeof(int) * (kNumClass + 1), c.stream));
+    const bool stats_kernel = cfg.stats || P.want_table;
+    const int bnd_words_per_col = 2 + (stats_kernel ? 2 * ((P.wide_stats || P.want_table) ? 2 : 1) : 0);
+    const long long bnd_stride = (long long)P.max_lr_multistrip * bnd_words_per_col;
+    if (bnd_stride > 0) PSB_TRY(B.d_bnd.alloc((size_t)(bnd_stride * max_grid_warps(n)) * sizeof(int), c.stream));
+
     // CIGAR scratch: pair i owns lq + lr + 2 words, in pair order, so its offset has a closed form that the device
-    // computes from the offset arrays it already holds (rev_off_kernel); only the decision blocks of pairs on the
+    // computes from the offset arrays it already holds (rev_off_kernel); only the trace blocks of pairs on the
     // 32-bit kernels (none in a typical batch) need a host pass
-    const long long rev_total = (q_two ? (long long)n * (long long)qbytes : (long long)(q_hi - q_lo)) + (long long)(r_hi - r_lo) + 2 * (long long)n;
+    const long long rev_total = (P.q_two ? (long long)n * (long long)P.qbytes : (long long)(P.q_hi - P.q_lo)) + (long long)(P.r_hi - P.r_lo) + 2 * (long long)n;
     bool any32 = false;
-    for (int cl = 0; cl < kNumClass; ++cl) any32 = any32 || !cls[cl].empty();
-    if ((want_trace || want_table) && any32) {
-        trace_off.assign(n, 0);
+    for (int cl = 0; cl < kNumClass; ++cl) any32 = any32 || !P.cls[cl].empty();
+    if ((cfg.trace || P.want_table) && any32) {
+        B.trace_off.assign(n, 0);
         for (int cl = 0; cl < kNumClass; ++cl)
-            for (int id : cls[cl]) {
-                const int K = ct.k[cl];
-                const int lq = pssm ? m.length : (int)(req.shared_query ? q_hi - q_lo : req.q_off[lo + id + 1] - req.q_off[lo + id]);
-                const int lr = (int)(req.r_off[lo + id + 1] - req.r_off[lo + id]);
-                const long long strips = (lq + 32 * K - 1) / (32 * K);
-                trace_off[id] = trace_total;
-                trace_total += ((strips * (lr + 31) * 32 * K + 15) / 16) * 16;
+            for (int id : P.cls[cl]) {
+                B.trace_off[id] = B.trace_total;
+                B.trace_total += ((trace_block_cells(P.ct.k[cl], P.lq(id), P.lr(id)) + 15) / 16) * 16;
             }
-        PSB_TRY(d_traceoff.alloc((size_t)n * sizeof(long long), c.stream));
-        PSB_CUDA(cudaMemcpyAsync(d_traceoff.p, trace_off.data(), (size_t)n * sizeof(long long), cudaMemcpyHostToDevice, c.stream));
-        if (want_trace) PSB_TRY(d_trace.alloc((size_t)trace_total, c.stream));
-        if (want_table) for (int k = 0; k < 4; ++k) PSB_TRY(d_tab[k].alloc((size_t)trace_total * sizeof(int), c.stream));
+        PSB_TRY(B.d_traceoff.alloc((size_t)n * sizeof(long long), c.stream));
+        PSB_CUDA(cudaMemcpyAsync(B.d_traceoff.p, B.trace_off.data(), (size_t)n * sizeof(long long), cudaMemcpyHostToDevice, c.stream));
+        if (cfg.trace) PSB_TRY(B.d_trace.alloc((size_t)B.trace_total, c.stream));
+        if (P.want_table) for (int k = 0; k < 4; ++k) PSB_TRY(B.d_tab[k].alloc((size_t)B.trace_total * sizeof(int), c.stream));
     }
 
-    hphase("trace-offsets");
-    Gotoh32Params p;
+    Gotoh32Params &p = B.p;
     std::memset(&p, 0, sizeof(p));
-    p.q = d_q.as<uint8_t>() - (q_two ? 0 : q_lo); p.q_off = d_qoff.as<long long>();
-    p.r = d_r.as<uint8_t>() - r_lo; p.r_off = d_roff.as<long long>();
-    p.shared_query = (req.shared_query || pssm) ? 1 : 0;
-    p.matrix = d_matrix.as<int>(); p.size = m.size; p.is_pssm = pssm ? 1 : 0;
+    p.q = B.d_q.as<uint8_t>() - (P.q_two ? 0 : P.q_lo); p.q_off = B.d_qoff.as<long long>();
+    p.r = B.d_r.as<uint8_t>() - P.r_lo; p.r_off = B.d_roff.as<long long>();
+    p.shared_query = P.q_two ? 1 : 0;
+    p.matrix = B.d_matrix.as<int>(); p.size = m.size; p.is_pssm = P.pssm ? 1 : 0;
     p.open = req.open; p.gap = req.gap;
     p.mode = cfg.mode; p.s1_beg = cfg.s1_beg; p.s1_end = cfg.s1_end; p.s2_beg = cfg.s2_beg; p.s2_end = cfg.s2_end;
-    p.score = d_out[0].as<int>(); p.end_query = d_out[1].as<int>(); p.end_ref = d_out[2].as<int>();
-    p.matches = d_out[3].as<int>(); p.similar = d_out[4].as<int>(); p.length = d_out[5].as<int>();
-    p.bnd = d_bnd.as<int>(); p.bnd_stride = bnd_stride;
-    p.trace = d_trace.as<uint8_t>(); p.trace_off = d_traceoff.as<long long>();
-    p.tabH = d_tab[0].as<int>(); p.tabM = d_tab[1].as<int>(); p.tabS = d_tab[2].as<int>(); p.tabL = d_tab[3].as<int>();
-    p.tab_off = d_traceoff.as<long long>();
-    if (banded) {
+    p.score = B.d_out[0].as<int>(); p.end_query = B.d_out[1].as<int>(); p.end_ref = B.d_out[2].as<int>();
+    p.matches = B.d_out[3].as<int>(); p.similar = B.d_out[4].as<int>(); p.length = B.d_out[5].as<int>();
+    p.bnd = B.d_bnd.as<int>(); p.bnd_stride = bnd_stride;
+    p.trace = B.d_trace.as<uint8_t>(); p.trace_off = B.d_traceoff.as<long long>();
+    p.tabH = B.d_tab[0].as<int>(); p.tabM = B.d_tab[1].as<int>(); p.tabS = B.d_tab[2].as<int>(); p.tabL = B.d_tab[3].as<int>();
+    p.tab_off = B.d_traceoff.as<long long>();
+    if (P.banded) {
         // [REF src/aligner/mod.rs:457-489] band of half-width k around the main diagonal, widened by the
         // length difference so that the corner (Lq-1, Lr-1) stays inside
-        const int lq1 = pssm ? m.length : (int)(q_hi - q_lo), lr1 = (int)(r_hi - r_lo), d = lr1 - lq1;
+        const int d = P.lr(0) - P.lq(0);
         p.banded = 1; p.band_lo = -cfg.band + (d < 0 ? d : 0); p.band_hi = cfg.band + (d > 0 ? d : 0);
     }
 
-    // CIGAR scratch of the device-side walks (both kernel families write the same reversed run lists)
-    if (want_trace) {
-        PSB_TRY(d_rev.alloc((size_t)rev_total * sizeof(unsigned), c.stream));
-        PSB_TRY(d_revoff.alloc((size_t)n * sizeof(long long), c.stream));
+    // CIGAR scratch of the device-side walks (every kernel family writes the same reversed run lists)
+    if (cfg.trace) {
+        PSB_TRY(B.d_rev.alloc((size_t)rev_total * sizeof(unsigned), c.stream));
+        PSB_TRY(B.d_revoff.alloc((size_t)n * sizeof(long long), c.stream));
         rev_off_kernel<<<(unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)c.sms * 8), 256, 0, c.stream>>>(
-            d_qoff.as<long long>(), d_roff.as<long long>(), q_two ? 1 : 0, (long long)qbytes, (long long)q_lo, (long long)r_lo, (long long)n,
-            d_revoff.as<long long>());
+            B.d_qoff.as<long long>(), B.d_roff.as<long long>(), P.q_two ? 1 : 0, (long long)P.qbytes, (long long)P.q_lo, (long long)P.r_lo,
+            (long long)n, B.d_revoff.as<long long>());
         c.launches++;
-        PSB_TRY(d_nops.alloc(((size_t)n + 1) * sizeof(int), c.stream));
-        PSB_CUDA(cudaMemsetAsync(d_nops.p, 0, ((size_t)n + 1) * sizeof(int), c.stream));
-        PSB_TRY(d_beg[0].alloc((size_t)n * sizeof(int), c.stream));
-        PSB_TRY(d_beg[1].alloc((size_t)n * sizeof(int), c.stream));
+        PSB_TRY(B.d_nops.alloc(((size_t)n + 1) * sizeof(int), c.stream));
+        PSB_CUDA(cudaMemsetAsync(B.d_nops.p, 0, ((size_t)n + 1) * sizeof(int), c.stream));
+        PSB_TRY(B.d_beg[0].alloc((size_t)n * sizeof(int), c.stream));
+        PSB_TRY(B.d_beg[1].alloc((size_t)n * sizeof(int), c.stream));
     }
+    return PSB_OK;
+}
 
-    // ---- packed 16-bit classes: two pairs per register, sorted by reference length so that the pairs of
-    // a word (and the words of a warp) are of similar size -----------------------------------------------
-    DevMem d_items, d_toff16, d_slot16, d_ids16, d_mat8, d_cnt16;
-    KeptMem d_trace16(2);
-    std::vector<int> h_items, h_slot16, h_ids16;   // kept alive until the stream has consumed them
-    std::vector<long long> h_toff16;
-    std::vector<int8_t> h_mat8(33 * 32);
+// packed 16-bit classes: two pairs per register, sorted by reference length so that the pairs of a word (and the
+// words of a warp) are of similar size.  Builds and queues the items, their trace offsets and the byte matrix.
+static int queue_items16(const PairsRequest &req, PassPlan &P, PassBufs &B) {
+    Ctx &c = g_ctx;
+    const HostMatrix &m = *req.matrix;
+    const size_t nc16 = P.p16_ids.size();
+    const bool top_free = req.cfg.mode == MODE_SW || (req.cfg.mode == MODE_SG && req.cfg.s1_beg);
+    B.cls_item0.assign(nc16 + 1, 0);
+    B.cls_id0.assign(nc16 + 1, 0);
+    if (P.n_p16 == 0) return PSB_OK;
+    B.h_items.reserve((size_t)P.n_p16 + 2 * nc16);
+    B.h_ids16.reserve((size_t)P.n_p16);
+    if (P.p16_walk) B.h_slot16.assign((size_t)P.n, 0);
+    B.h_toff16.push_back(0);
+    for (size_t c16 = 0; c16 < nc16; ++c16) {
+        std::vector<int> &ids = P.p16_ids[c16];
+        B.cls_item0[c16] = (int)(B.h_items.size() / 2);
+        B.cls_id0[c16] = (int)B.h_ids16.size();
+        if (ids.empty()) continue;
+        const P16Class pc = p16_class((int)c16);
+        if (!P.uniform) P.longest_first(ids);
+        for (size_t t = 0; t < ids.size(); t += 2) {
+            const int a = ids[t], bb = t + 1 < ids.size() ? ids[t + 1] : -1;
+            const int item = (int)(B.h_items.size() / 2);
+            B.h_items.push_back(a); B.h_items.push_back(bb);
+            if (P.p16_walk) {
+                const int lrb = bb >= 0 ? P.lr(bb) : 0;
+                B.h_toff16.push_back(B.h_toff16.back() + pairs16_item_trace_words(pc.G, pc.K, std::max(P.lr(a), lrb)));
+                B.h_slot16[a] = 2 * item;
+                if (bb >= 0) B.h_slot16[bb] = 2 * item + 1;
+            }
+        }
+        B.h_ids16.insert(B.h_ids16.end(), ids.begin(), ids.end());
+    }
+    B.cls_item0[nc16] = (int)(B.h_items.size() / 2);
+    B.cls_id0[nc16] = (int)B.h_ids16.size();
+    pairs16_build_mat8(m.table.data(), m.size, req.open, top_free, B.h_mat8.data());
+    PSB_TRY(B.d_items.alloc(B.h_items.size() * sizeof(int), c.stream));
+    PSB_TRY(B.d_mat8.alloc(B.h_mat8.size(), c.stream));
+    PSB_TRY(B.d_cnt16.alloc(sizeof(int) * (nc16 + 1), c.stream));
+    PSB_CUDA(cudaMemcpyAsync(B.d_items.p, B.h_items.data(), B.h_items.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
+    PSB_CUDA(cudaMemcpyAsync(B.d_mat8.p, B.h_mat8.data(), B.h_mat8.size(), cudaMemcpyHostToDevice, c.stream));
+    PSB_CUDA(cudaMemsetAsync(B.d_cnt16.p, 0, sizeof(int) * (nc16 + 1), c.stream));
+    if (P.p16_walk) {
+        PSB_TRY(B.d_toff16.alloc(B.h_toff16.size() * sizeof(long long), c.stream));
+        PSB_TRY(B.d_slot16.alloc(B.h_slot16.size() * sizeof(int), c.stream));
+        PSB_TRY(B.d_ids16.alloc(B.h_ids16.size() * sizeof(int), c.stream));
+        PSB_TRY(B.d_trace16.alloc((size_t)B.h_toff16.back() * sizeof(unsigned) + 64, c.stream));
+        PSB_CUDA(cudaMemcpyAsync(B.d_toff16.p, B.h_toff16.data(), B.h_toff16.size() * sizeof(long long), cudaMemcpyHostToDevice, c.stream));
+        PSB_CUDA(cudaMemcpyAsync(B.d_slot16.p, B.h_slot16.data(), B.h_slot16.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
+        PSB_CUDA(cudaMemcpyAsync(B.d_ids16.p, B.h_ids16.data(), B.h_ids16.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
+    }
+    return PSB_OK;
+}
+
+// residues to matrix columns on the device; references out of a resident database are gathered from its packed
+// store instead (already matrix codes, written at the same biased offsets an upload would have put them)
+static void launch_map(const PairsRequest &req, const PassPlan &P, PassBufs &B) {
+    Ctx &c = g_ctx;
+    const HostMatrix &m = *req.matrix;
+    MapParams mp;
+    fill_lut(mp.lut, m.mapper);
+    const int blocks = c.sms * 8;
+    if (!(P.pssm && m.query.size() != (size_t)m.length)) {
+        mp.data = B.d_q.as<uint8_t>(); mp.n = (long long)P.qbytes;
+        map_residues_kernel<<<blocks, 256, 0, c.stream>>>(mp);
+        c.launches++;
+    }
+    if (req.r_db) {
+        UnpackParams u;
+        u.words = req.r_db->d_words; u.word_off = req.r_db->d_word_off; u.ids = B.d_rids.as<int>(); u.inv_perm = req.r_db->d_inv_perm;
+        u.out_off = B.d_roff.as<long long>(); u.out = B.d_r.as<uint8_t>() - P.r_lo; u.n = P.n; u.bits = req.r_db->bits;
+        unpack_db_kernel<<<(unsigned)std::min<int64_t>((P.n + 7) / 8, blocks), 256, 0, c.stream>>>(u);
+    } else {
+        mp.data = B.d_r.as<uint8_t>(); mp.n = (long long)(P.r_hi - P.r_lo);
+        map_residues_kernel<<<blocks, 256, 0, c.stream>>>(mp);
+    }
+    c.launches++;
+}
+
+// the packed classes' fill kernels, each followed by its walk when the request wants traceback or statistics
+static int launch_pairs16(const PairsRequest &req, const PassPlan &P, PassBufs &B, PassTimeline &tl) {
+    Ctx &c = g_ctx;
+    const FnConfig &cfg = req.cfg;
+    const HostMatrix &m = *req.matrix;
+    const Gotoh32Params &p = B.p;
     const bool sw = cfg.mode == MODE_SW;
-    const bool top_free = sw || (cfg.mode == MODE_SG && cfg.s1_beg);
-    std::vector<int> cls_item0(p16_ids.size() + 1, 0), cls_id0(p16_ids.size() + 1, 0);
-    if (n_p16 > 0) {
-        h_items.reserve((size_t)n_p16 + 2 * p16_ids.size());
-        h_ids16.reserve((size_t)n_p16);
-        if (p16_walk) h_slot16.assign((size_t)n, 0);
-        h_toff16.push_back(0);
-        for (int c16 = 0; c16 < (int)p16_ids.size(); ++c16) {
-            std::vector<int> &ids = p16_ids[c16];
-            cls_item0[c16] = (int)(h_items.size() / 2);
-            cls_id0[c16] = (int)h_ids16.size();
-            if (ids.empty()) continue;
-            const P16Class pc = p16_class(c16);
-            if (!uniform)
-                std::stable_sort(ids.begin(), ids.end(), [&](int a, int bb) {
-                    return req.r_off[lo + a + 1] - req.r_off[lo + a] > req.r_off[lo + bb + 1] - req.r_off[lo + bb];
-                });
-            for (size_t t = 0; t < ids.size(); t += 2) {
-                const int a = ids[t], bb = t + 1 < ids.size() ? ids[t + 1] : -1;
-                const int item = (int)(h_items.size() / 2);
-                h_items.push_back(a); h_items.push_back(bb);
-                if (p16_walk) {
-                    const long long lra = req.r_off[lo + a + 1] - req.r_off[lo + a];
-                    const long long lrb = bb >= 0 ? req.r_off[lo + bb + 1] - req.r_off[lo + bb] : 0;
-                    h_toff16.push_back(h_toff16.back() + pairs16_item_trace_words(pc.G, pc.K, (int)std::max(lra, lrb)));
-                    h_slot16[a] = 2 * item;
-                    if (bb >= 0) h_slot16[bb] = 2 * item + 1;
-                }
-            }
-            h_ids16.insert(h_ids16.end(), ids.begin(), ids.end());
-        }
-        cls_item0[p16_ids.size()] = (int)(h_items.size() / 2);
-        cls_id0[p16_ids.size()] = (int)h_ids16.size();
-        pairs16_build_mat8(m.table.data(), m.size, req.open, top_free, h_mat8.data());
-        PSB_TRY(d_items.alloc(h_items.size() * sizeof(int), c.stream));
-        PSB_TRY(d_mat8.alloc(h_mat8.size(), c.stream));
-        PSB_TRY(d_cnt16.alloc(sizeof(int) * (p16_ids.size() + 1), c.stream));
-        PSB_CUDA(cudaMemcpyAsync(d_items.p, h_items.data(), h_items.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
-        PSB_CUDA(cudaMemcpyAsync(d_mat8.p, h_mat8.data(), h_mat8.size(), cudaMemcpyHostToDevice, c.stream));
-        PSB_CUDA(cudaMemsetAsync(d_cnt16.p, 0, sizeof(int) * (p16_ids.size() + 1), c.stream));
-        if (p16_walk) {
-            PSB_TRY(d_toff16.alloc(h_toff16.size() * sizeof(long long), c.stream));
-            PSB_TRY(d_slot16.alloc(h_slot16.size() * sizeof(int), c.stream));
-            PSB_TRY(d_ids16.alloc(h_ids16.size() * sizeof(int), c.stream));
-            PSB_TRY(d_trace16.alloc((size_t)h_toff16.back() * sizeof(unsigned) + 64, c.stream));
-            PSB_CUDA(cudaMemcpyAsync(d_toff16.p, h_toff16.data(), h_toff16.size() * sizeof(long long), cudaMemcpyHostToDevice, c.stream));
-            PSB_CUDA(cudaMemcpyAsync(d_slot16.p, h_slot16.data(), h_slot16.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
-            PSB_CUDA(cudaMemcpyAsync(d_ids16.p, h_ids16.data(), h_ids16.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
-        }
-    }
-    hphase("items");
-    // every host->device copy of this pass is queued: the timed region (psb_last_kernel_ms) starts here
-    PSB_CUDA(cudaEventRecord(c.ev0, c.stream));
-    {
-        MapParams mp;
-        fill_lut(mp.lut, m.mapper);
-        const int blocks = c.sms * 8;
-        if (!(pssm && m.query.size() != (size_t)m.length)) {
-            mp.data = d_q.as<uint8_t>(); mp.n = (long long)qbytes;
-            map_residues_kernel<<<blocks, 256, 0, c.stream>>>(mp);
-            c.launches++;
-        }
-        if (req.r_db) {
-            // the references straight out of the packed store: already matrix codes, written at the same biased
-            // offsets an upload would have put them
-            UnpackParams u;
-            u.words = req.r_db->d_words; u.word_off = req.r_db->d_word_off; u.ids = d_rids.as<int>(); u.inv_perm = req.r_db->d_inv_perm;
-            u.out_off = d_roff.as<long long>(); u.out = d_r.as<uint8_t>() - r_lo; u.n = n; u.bits = req.r_db->bits;
-            unpack_db_kernel<<<(unsigned)std::min<int64_t>((n + 7) / 8, blocks), 256, 0, c.stream>>>(u);
-        } else {
-            mp.data = d_r.as<uint8_t>(); mp.n = (long long)(r_hi - r_lo);
-            map_residues_kernel<<<blocks, 256, 0, c.stream>>>(mp);
-        }
+    if (P.n_p16 == 0) return PSB_OK;
+    std::string err;
+    for (int c16 = 0; c16 < (int)P.p16_ids.size(); ++c16) {
+        const int nitems = B.cls_item0[c16 + 1] - B.cls_item0[c16];
+        if (nitems == 0) continue;
+        Pairs16Params pp;
+        std::memset(&pp, 0, sizeof(pp));
+        pp.q = p.q; pp.q_off = p.q_off; pp.r = p.r; pp.r_off = p.r_off; pp.shared_query = p.shared_query;
+        pp.items = B.d_items.as<int>() + 2 * (size_t)B.cls_item0[c16]; pp.nitems = nitems;
+        pp.mat8 = B.d_mat8.as<int8_t>(); pp.size = m.size; pp.open = req.open; pp.gap = req.gap;
+        pp.mode = cfg.mode; pp.s1_beg = cfg.s1_beg; pp.s1_end = cfg.s1_end; pp.s2_beg = cfg.s2_beg; pp.s2_end = cfg.s2_end;
+        pp.score = p.score; pp.end_query = p.end_query; pp.end_ref = p.end_ref;
+        pp.trace = B.d_trace16.as<unsigned>(); pp.trace_off = P.p16_walk ? B.d_toff16.as<long long>() + B.cls_item0[c16] : nullptr;
+        pp.counter = B.d_cnt16.as<int>() + c16;
+        int wps = 0;
+        tl.begin("pairs16 fill G" + std::to_string(p16_class(c16).G) + " K" + std::to_string(p16_class(c16).K) + " items " + std::to_string(nitems));
+        const int rc16 = p16_launch(c16, sw, P.p16_walk, pp, c.sms, c.stream, &err, &wps);
+        tl.end();
+        if (tl.on) tl.marks.back().what += " warps/SM " + std::to_string(wps);
+        if (rc16 != PSB_OK) { set_error(err); return rc16; }
         c.launches++;
-    }
-
-    const bool dbg_time = std::getenv("PSB_DEBUG_TIMING") != nullptr;
-    std::vector<std::pair<std::string, std::pair<cudaEvent_t, cudaEvent_t>>> dbg_ev;
-    auto dbg_mark = [&](const std::string &what, bool begin) {
-        if (!dbg_time) return;
-        cudaEvent_t ev = nullptr;
-        cudaEventCreate(&ev);
-        cudaEventRecord(ev, c.stream);
-        if (begin) dbg_ev.push_back({what, {ev, nullptr}}); else dbg_ev.back().second.second = ev;
-    };
-    if (n_p16 > 0) {
-        std::string err;
-        for (int c16 = 0; c16 < (int)p16_ids.size(); ++c16) {
-            const int nitems = cls_item0[c16 + 1] - cls_item0[c16];
-            if (nitems == 0) continue;
-            Pairs16Params pp;
-            std::memset(&pp, 0, sizeof(pp));
-            pp.q = p.q; pp.q_off = p.q_off; pp.r = p.r; pp.r_off = p.r_off; pp.shared_query = p.shared_query;
-            pp.items = d_items.as<int>() + 2 * (size_t)cls_item0[c16]; pp.nitems = nitems;
-            pp.mat8 = d_mat8.as<int8_t>(); pp.size = m.size; pp.open = req.open; pp.gap = req.gap;
-            pp.mode = cfg.mode; pp.s1_beg = cfg.s1_beg; pp.s1_end = cfg.s1_end; pp.s2_beg = cfg.s2_beg; pp.s2_end = cfg.s2_end;
-            pp.score = p.score; pp.end_query = p.end_query; pp.end_ref = p.end_ref;
-            pp.trace = d_trace16.as<unsigned>(); pp.trace_off = p16_walk ? d_toff16.as<long long>() + cls_item0[c16] : nullptr;
-            pp.counter = d_cnt16.as<int>() + c16;
-            int wps = 0;
-            dbg_mark("pairs16 fill G" + std::to_string(p16_class(c16).G) + " K" + std::to_string(p16_class(c16).K) + " items " + std::to_string(nitems), true);
-            const int rc16 = p16_launch(c16, sw, p16_walk, pp, c.sms, c.stream, &err, &wps);
-            dbg_mark("", false);
-            if (dbg_time) dbg_ev.back().first += " warps/SM " + std::to_string(wps);
-            if (rc16 != PSB_OK) { set_error(err); return rc16; }
+        if (P.p16_walk) {
+            Walk16Params w;
+            std::memset(&w, 0, sizeof(w));
+            w.q = p.q; w.q_off = p.q_off; w.r = p.r; w.r_off = p.r_off; w.shared_query = p.shared_query;
+            w.pair_ids = B.d_ids16.as<int>() + B.cls_id0[c16]; w.pair_slot = B.d_slot16.as<int>(); w.n = B.cls_id0[c16 + 1] - B.cls_id0[c16];
+            w.G = p16_class(c16).G; w.K = p16_class(c16).K;
+            w.trace = B.d_trace16.as<unsigned>(); w.trace_off = B.d_toff16.as<long long>();
+            w.matrix = p.matrix; w.size = m.size; w.open = req.open; w.gap = req.gap; w.is_sw = sw ? 1 : 0;
+            w.top_free = (sw || (cfg.mode == MODE_SG && cfg.s1_beg)) ? 1 : 0; w.left_free = (sw || (cfg.mode == MODE_SG && cfg.s2_beg)) ? 1 : 0;
+            w.score = p.score; w.end_query = p.end_query; w.end_ref = p.end_ref;
+            w.rev_ops = B.d_rev.as<unsigned>(); w.rev_off = B.d_revoff.as<long long>();
+            w.nops = B.d_nops.as<int>(); w.beg_query = B.d_beg[0].as<int>(); w.beg_ref = B.d_beg[1].as<int>();
+            w.matches = p.matches; w.similar = p.similar; w.length = p.length;
+            tl.begin("walk16");
+            const int rcw = p16_launch_walk(w, !cfg.trace, c.stream, &err);
+            tl.end();
+            if (rcw != PSB_OK) { set_error(err); return rcw; }
             c.launches++;
-            if (p16_walk) {
-                Walk16Params w;
-                std::memset(&w, 0, sizeof(w));
-                w.q = p.q; w.q_off = p.q_off; w.r = p.r; w.r_off = p.r_off; w.shared_query = p.shared_query;
-                w.pair_ids = d_ids16.as<int>() + cls_id0[c16]; w.pair_slot = d_slot16.as<int>(); w.n = cls_id0[c16 + 1] - cls_id0[c16];
-                w.G = p16_class(c16).G; w.K = p16_class(c16).K;
-                w.trace = d_trace16.as<unsigned>(); w.trace_off = d_toff16.as<long long>();
-                w.matrix = p.matrix; w.size = m.size; w.open = req.open; w.gap = req.gap; w.is_sw = sw ? 1 : 0;
-                w.top_free = top_free ? 1 : 0; w.left_free = (sw || (cfg.mode == MODE_SG && cfg.s2_beg)) ? 1 : 0;
-                w.score = p.score; w.end_query = p.end_query; w.end_ref = p.end_ref;
-                w.rev_ops = d_rev.as<unsigned>(); w.rev_off = d_revoff.as<long long>();
-                w.nops = d_nops.as<int>(); w.beg_query = d_beg[0].as<int>(); w.beg_ref = d_beg[1].as<int>();
-                w.matches = p.matches; w.similar = p.similar; w.length = p.length;
-                dbg_mark("walk16", true);
-                const int rcw = p16_launch_walk(w, !cfg.trace, c.stream, &err);
-                dbg_mark("", false);
-                if (rcw != PSB_OK) { set_error(err); return rcw; }
-                c.launches++;
-            }
         }
     }
+    return PSB_OK;
+}
 
-    std::vector<DevMem> d_orders(kNumClass);
+// one launch of the one-warp-per-pair kernel per 32-bit class, longest pairs first unless every pair is alike
+static int launch_classes(const PairsRequest &req, PassPlan &P, PassBufs &B) {
+    Ctx &c = g_ctx;
+    const FnConfig &cfg = req.cfg;
+    Gotoh32Params &p = B.p;
     for (int cl = 0; cl < kNumClass; ++cl) {
-        if (cls[cl].empty()) continue;
-        std::vector<int> &ids = cls[cl];
+        std::vector<int> &ids = P.cls[cl];
+        if (ids.empty()) continue;
         p.order = nullptr;
-        if (!uniform) {
-            // longest first so the dynamic queue ends on short pairs
-            std::stable_sort(ids.begin(), ids.end(), [&](int a, int bb) {
-                const long long la = req.r_off[lo + a + 1] - req.r_off[lo + a], lb = req.r_off[lo + bb + 1] - req.r_off[lo + bb];
-                return la > lb;
-            });
-            PSB_TRY(d_orders[cl].alloc(ids.size() * sizeof(int), c.stream));
-            PSB_CUDA(cudaMemcpyAsync(d_orders[cl].p, ids.data(), ids.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
-            p.order = d_orders[cl].as<int>();
+        if (!P.uniform) {
+            P.longest_first(ids);
+            PSB_TRY(B.d_orders[cl].alloc(ids.size() * sizeof(int), c.stream));
+            PSB_CUDA(cudaMemcpyAsync(B.d_orders[cl].p, ids.data(), ids.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
+            p.order = B.d_orders[cl].as<int>();
         }
         p.n = (int)ids.size();
-        p.counter = d_counter.as<int>() + cl;
-        const Variant v = want_table ? V_TABLE : (want_trace ? V_TRACE : (cfg.stats ? (wide_stats ? V_STATS64 : V_STATS32) : V_SCORE));
-        PSB_TRY(launch_gotoh32(ct.k[cl], v, p, p.n, fine));
+        p.counter = B.d_counter.as<int>() + cl;
+        const Variant v = P.want_table ? V_TABLE : (cfg.trace ? V_TRACE : (cfg.stats ? (P.wide_stats ? V_STATS64 : V_STATS32) : V_SCORE));
+        PSB_TRY(launch_gotoh32(P.ct.k[cl], v, p, p.n, P.fine));
     }
+    return PSB_OK;
+}
 
-    for (int id : wave_ids) {
+// the long pairs, one at a time over the whole GPU
+static int launch_waves(const PairsRequest &req, const PassPlan &P, PassBufs &B, PassTimeline &tl) {
+    const FnConfig &cfg = req.cfg;
+    for (int id : P.wave_ids) {
         // (byte offsets relative to the biased p.q / p.r)
-        const long long qb = req.shared_query ? 0 : req.q_off[lo + id], rb = req.r_off[lo + id];
-        const int lq = (int)(req.shared_query ? q_hi - q_lo : req.q_off[lo + id + 1] - req.q_off[lo + id]);
-        const int lr = (int)(req.r_off[lo + id + 1] - req.r_off[lo + id]);
+        const long long qb = req.shared_query ? 0 : req.q_off[P.lo + id], rb = req.r_off[P.lo + id];
         WaveWalk ww;
         ww.stats = !cfg.trace;
-        ww.rev_ops = d_rev.as<unsigned>(); ww.rev_off = d_revoff.as<long long>();
-        ww.nops = d_nops.as<int>(); ww.beg_query = d_beg[0].as<int>(); ww.beg_ref = d_beg[1].as<int>();
-        PSB_TRY(launch_wave32(p, m, qb, lq, rb, lr, id, (cfg.stats || cfg.trace) ? &ww : nullptr));
+        ww.rev_ops = B.d_rev.as<unsigned>(); ww.rev_off = B.d_revoff.as<long long>();
+        ww.nops = B.d_nops.as<int>(); ww.beg_query = B.d_beg[0].as<int>(); ww.beg_ref = B.d_beg[1].as<int>();
+        PSB_TRY(launch_wave32(B.p, *req.matrix, qb, P.lq(id), rb, P.lr(id), id, (cfg.stats || cfg.trace) ? &ww : nullptr, tl));
     }
+    return PSB_OK;
+}
 
-    // device-side trace walk -> CIGAR CSR
-    DevMem d_csroff, d_scan_tmp;
-    if (want_trace) {
-        for (int cl = 0; cl < kNumClass; ++cl) {
-            if (cls[cl].empty()) continue;
-            if (!d_orders[cl].p) {
-                PSB_TRY(d_orders[cl].alloc(cls[cl].size() * sizeof(int), c.stream));
-                PSB_CUDA(cudaMemcpyAsync(d_orders[cl].p, cls[cl].data(), cls[cl].size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
-            }
-            WalkParams w;
-            w.q = p.q; w.q_off = p.q_off; w.r = p.r; w.r_off = p.r_off; w.shared_query = p.shared_query;
-            w.ids = d_orders[cl].as<int>(); w.n = (int)cls[cl].size(); w.K = ct.k[cl];
-            w.trace = p.trace; w.trace_off = p.trace_off; w.end_query = p.end_query; w.end_ref = p.end_ref;
-            w.rev_ops = d_rev.as<unsigned>(); w.rev_off = d_revoff.as<long long>();
-            w.nops = d_nops.as<int>(); w.beg_query = d_beg[0].as<int>(); w.beg_ref = d_beg[1].as<int>();
-            walk_trace_kernel<<<(w.n + 127) / 128, 128, 0, c.stream>>>(w);
-            c.launches++;
+// traceback: the walks of the pairs on the 32-bit kernels, then the CIGAR CSR offsets (exclusive scan of the run counts)
+static int launch_walks(const PairsRequest &req, const PassPlan &P, PassBufs &B) {
+    Ctx &c = g_ctx;
+    const Gotoh32Params &p = B.p;
+    const int64_t n = P.n;
+    if (!req.cfg.trace) return PSB_OK;
+    for (int cl = 0; cl < kNumClass; ++cl) {
+        if (P.cls[cl].empty()) continue;
+        if (!B.d_orders[cl].p) {
+            PSB_TRY(B.d_orders[cl].alloc(P.cls[cl].size() * sizeof(int), c.stream));
+            PSB_CUDA(cudaMemcpyAsync(B.d_orders[cl].p, P.cls[cl].data(), P.cls[cl].size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
         }
-        // exclusive scan of nops[0..n] -> csr offsets (n+1)
-        PSB_TRY(d_csroff.alloc(((size_t)n + 1) * sizeof(long long), c.stream));
-        size_t tmp_bytes = 0;
-        auto in_it = d_nops.as<int>();
-        PSB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, in_it, d_csroff.as<long long>(), (int)(n + 1), c.stream));
-        PSB_TRY(d_scan_tmp.alloc(tmp_bytes, c.stream));
-        PSB_CUDA(cub::DeviceScan::ExclusiveSum(d_scan_tmp.p, tmp_bytes, in_it, d_csroff.as<long long>(), (int)(n + 1), c.stream));
+        WalkParams w;
+        w.q = p.q; w.q_off = p.q_off; w.r = p.r; w.r_off = p.r_off; w.shared_query = p.shared_query;
+        w.ids = B.d_orders[cl].as<int>(); w.n = (int)P.cls[cl].size(); w.K = P.ct.k[cl];
+        w.trace = p.trace; w.trace_off = p.trace_off; w.end_query = p.end_query; w.end_ref = p.end_ref;
+        w.rev_ops = B.d_rev.as<unsigned>(); w.rev_off = B.d_revoff.as<long long>();
+        w.nops = B.d_nops.as<int>(); w.beg_query = B.d_beg[0].as<int>(); w.beg_ref = B.d_beg[1].as<int>();
+        walk_trace_kernel<<<(w.n + 127) / 128, 128, 0, c.stream>>>(w);
         c.launches++;
     }
-    PSB_CUDA(cudaEventRecord(c.ev1, c.stream));
-    hphase("launches");
+    // exclusive scan of nops[0..n] -> csr offsets (n+1)
+    PSB_TRY(B.d_csroff.alloc(((size_t)n + 1) * sizeof(long long), c.stream));
+    size_t tmp_bytes = 0;
+    auto in_it = B.d_nops.as<int>();
+    PSB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, in_it, B.d_csroff.as<long long>(), (int)(n + 1), c.stream));
+    PSB_TRY(B.d_scan_tmp.alloc(tmp_bytes, c.stream));
+    PSB_CUDA(cub::DeviceScan::ExclusiveSum(B.d_scan_tmp.p, tmp_bytes, in_it, B.d_csroff.as<long long>(), (int)(n + 1), c.stream));
+    c.launches++;
+    return PSB_OK;
+}
 
-    // results back to the batch's pinned arrays
+// results back to the batch's pinned arrays; with traceback, the walks' run lists compacted into the pass's CIGAR words
+static int copy_results(const PairsRequest &req, const PassPlan &P, PassBufs &B, psb_batch_t *b, PassOut *po, PassTimeline &tl) {
+    Ctx &c = g_ctx;
+    const int64_t n = P.n, lo = P.lo;
     int *outs[6] = {b->score, b->end_query, b->end_ref, b->matches, b->similar, b->length};
-    const int ncopy = cfg.stats ? 6 : 3;
+    const int ncopy = req.cfg.stats ? 6 : 3;
     for (int k = 0; k < ncopy; ++k)
-        PSB_CUDA(cudaMemcpyAsync(outs[k] + lo, d_out[k].p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
-    if (want_trace) {
-        std::vector<long long> csr_off(n + 1);
-        PSB_CUDA(cudaMemcpyAsync(csr_off.data(), d_csroff.p, ((size_t)n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, c.stream));
-        PSB_CUDA(cudaStreamSynchronize(c.stream));
-        hphase("wait-kernels");
-        const long long total = csr_off[n];
-        PSB_TRY(po->d_csr.alloc((size_t)total * sizeof(unsigned), c.stream));
-        CompactParams cp;
-        cp.rev_ops = d_rev.as<unsigned>(); cp.rev_off = d_revoff.as<long long>();
-        cp.csr_off = d_csroff.as<long long>(); cp.csr_ops = po->d_csr.as<unsigned>(); cp.n = (int)n;
-        compact_cigar_kernel<<<c.sms * 8, 256, 0, c.stream>>>(cp);
-        c.launches++;
-        PSB_CUDA(cudaMemcpyAsync(b->beg_query + lo, d_beg[0].p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
-        PSB_CUDA(cudaMemcpyAsync(b->beg_ref + lo, d_beg[1].p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
-        po->csr_off.swap(csr_off);
-    }
-
-    // single-pair extras: row-major trace bytes, tables, last row / column
-    if (req.extra && n == 1 && (want_trace || want_table)) {
-        psb_result_extra *x = req.extra;
-        const int cl = first_cls, K = cl >= 0 ? ct.k[cl] : 1;
-        const int lq = x->qlen, lr = x->rlen, nsteps = lr + 31;
-        auto cell_index = [&](int i, int j) {
-            const int strip = i / (32 * K), rem = i % (32 * K), lane = rem / K, k = rem % K;
-            return (((size_t)strip * nsteps + (j + lane)) * 32 + lane) * K + k;
-        };
-        if (want_trace && first_cls >= 0 && trace_total > 0) {   // (a pair on the wavefront kernel has no flag bytes)
-            // the block comes back as it is; psb_result_extra::trace_table() makes it row-major for the caller that
-            // asks (cell (i, j) sits at cell_index(i, j); the copy is synchronised with the results below)
-            x->trace_blob.resize((size_t)trace_total);
-            x->trace_K = K;
-            PSB_CUDA(cudaMemcpyAsync(x->trace_blob.data(), d_trace.p, x->trace_blob.size(), cudaMemcpyDeviceToHost, c.stream));
-        }
-        if (want_table) {
-            std::vector<int> planes[4];
-            const int np = cfg.stats ? 4 : 1;
-            for (int k = 0; k < np; ++k) {
-                planes[k].resize((size_t)trace_total);
-                PSB_CUDA(cudaMemcpyAsync(planes[k].data(), d_tab[k].p, planes[k].size() * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
-            }
-            PSB_CUDA(cudaStreamSynchronize(c.stream));
-            std::vector<int> *tabs[4] = {&x->score_table, &x->matches_table, &x->similar_table, &x->length_table};
-            std::vector<int> *rows[4] = {&x->score_row, &x->matches_row, &x->similar_row, &x->length_row};
-            std::vector<int> *cols[4] = {&x->score_col, &x->matches_col, &x->similar_col, &x->length_col};
-            for (int k = 0; k < np; ++k) {
-                if (cfg.table) {
-                    tabs[k]->resize((size_t)lq * lr);
-                    for (int i = 0; i < lq; ++i)
-                        for (int j = 0; j < lr; ++j) (*tabs[k])[(size_t)i * lr + j] = planes[k][cell_index(i, j)];
-                } else {
-                    rows[k]->resize(lr); cols[k]->resize(lq);
-                    for (int j = 0; j < lr; ++j) (*rows[k])[j] = planes[k][cell_index(lq - 1, j)];
-                    for (int i = 0; i < lq; ++i) (*cols[k])[i] = planes[k][cell_index(i, lr - 1)];
-                }
-            }
-        }
-    }
-    hphase("results-queued");
+        PSB_CUDA(cudaMemcpyAsync(outs[k] + lo, B.d_out[k].p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+    if (!req.cfg.trace) return PSB_OK;
+    std::vector<long long> csr_off(n + 1);
+    PSB_CUDA(cudaMemcpyAsync(csr_off.data(), B.d_csroff.p, ((size_t)n + 1) * sizeof(long long), cudaMemcpyDeviceToHost, c.stream));
     PSB_CUDA(cudaStreamSynchronize(c.stream));
-    hphase("wait");
+    tl.phase("wait-kernels");
+    const long long total = csr_off[n];
+    PSB_TRY(po->d_csr.alloc((size_t)total * sizeof(unsigned), c.stream));
+    CompactParams cp;
+    cp.rev_ops = B.d_rev.as<unsigned>(); cp.rev_off = B.d_revoff.as<long long>();
+    cp.csr_off = B.d_csroff.as<long long>(); cp.csr_ops = po->d_csr.as<unsigned>(); cp.n = (int)n;
+    compact_cigar_kernel<<<c.sms * 8, 256, 0, c.stream>>>(cp);
+    c.launches++;
+    PSB_CUDA(cudaMemcpyAsync(b->beg_query + lo, B.d_beg[0].p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+    PSB_CUDA(cudaMemcpyAsync(b->beg_ref + lo, B.d_beg[1].p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+    po->csr_off.swap(csr_off);
+    return PSB_OK;
+}
+
+// single-pair extras: the trace block as it is (psb_result_extra::trace_table() makes it row-major for the caller that
+// asks), tables, last row / column
+static int copy_extras(const PairsRequest &req, const PassPlan &P, PassBufs &B) {
+    Ctx &c = g_ctx;
+    const FnConfig &cfg = req.cfg;
+    if (!(req.extra && P.n == 1 && (cfg.trace || P.want_table))) return PSB_OK;
+    psb_result_extra *x = req.extra;
+    const int K = P.first_cls >= 0 ? P.ct.k[P.first_cls] : 1;
+    const int lq = x->qlen, lr = x->rlen;
+    if (cfg.trace && P.first_cls >= 0 && B.trace_total > 0) {   // (a pair on the wavefront kernel has no flag bytes)
+        // (the copy is synchronised with the results)
+        x->trace_blob.resize((size_t)B.trace_total);
+        x->trace_K = K;
+        PSB_CUDA(cudaMemcpyAsync(x->trace_blob.data(), B.d_trace.p, x->trace_blob.size(), cudaMemcpyDeviceToHost, c.stream));
+    }
+    if (!P.want_table) return PSB_OK;
+    std::vector<int> planes[4];
+    const int np = cfg.stats ? 4 : 1;
+    for (int k = 0; k < np; ++k) {
+        planes[k].resize((size_t)B.trace_total);
+        PSB_CUDA(cudaMemcpyAsync(planes[k].data(), B.d_tab[k].p, planes[k].size() * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
+    }
+    PSB_CUDA(cudaStreamSynchronize(c.stream));
+    std::vector<int> *tabs[4] = {&x->score_table, &x->matches_table, &x->similar_table, &x->length_table};
+    std::vector<int> *rows[4] = {&x->score_row, &x->matches_row, &x->similar_row, &x->length_row};
+    std::vector<int> *cols[4] = {&x->score_col, &x->matches_col, &x->similar_col, &x->length_col};
+    for (int k = 0; k < np; ++k) {
+        if (cfg.table) {
+            tabs[k]->resize((size_t)lq * lr);
+            for (int i = 0; i < lq; ++i)
+                for (int j = 0; j < lr; ++j) (*tabs[k])[(size_t)i * lr + j] = planes[k][trace_cell_index(K, lr, i, j)];
+        } else {
+            rows[k]->resize(lr); cols[k]->resize(lq);
+            for (int j = 0; j < lr; ++j) (*rows[k])[j] = planes[k][trace_cell_index(K, lr, lq - 1, j)];
+            for (int i = 0; i < lq; ++i) (*cols[k])[i] = planes[k][trace_cell_index(K, lr, i, lr - 1)];
+        }
+    }
+    return PSB_OK;
+}
+
+// One pass: pairs lo..hi-1 of the batch.  Their results land in the batch's slices lo..hi-1 and in *po.
+static int run_pairs_range(const PairsRequest &req, int64_t lo, int64_t hi, psb_batch_t *b, PassOut *po) {
+    Ctx &c = g_ctx;
+    const int launches_at_entry = c.launches;
+    PassTimeline tl;
+    PassPlan plan;
+    PSB_TRY(plan_pass(req, lo, hi, &plan));
+    po->cells = plan.cells;
+    tl.phase("classify");
+    PassBufs bufs;
+    PSB_TRY(upload_pass(req, plan, bufs));
+    tl.phase("uploads");
+    PSB_TRY(alloc_pass(req, plan, bufs));
+    tl.phase("trace-offsets");
+    PSB_TRY(queue_items16(req, plan, bufs));
+    tl.phase("items");
+    // every host->device copy of this pass is queued: the timed region (psb_last_kernel_ms) starts here
+    PSB_CUDA(cudaEventRecord(c.ev0, c.stream));
+    launch_map(req, plan, bufs);
+    PSB_TRY(launch_pairs16(req, plan, bufs, tl));
+    PSB_TRY(launch_classes(req, plan, bufs));
+    PSB_TRY(launch_waves(req, plan, bufs, tl));
+    PSB_TRY(launch_walks(req, plan, bufs));
+    PSB_CUDA(cudaEventRecord(c.ev1, c.stream));
+    tl.phase("launches");
+    PSB_TRY(copy_results(req, plan, bufs, b, po, tl));
+    PSB_TRY(copy_extras(req, plan, bufs));
+    tl.phase("results-queued");
+    PSB_CUDA(cudaStreamSynchronize(c.stream));
+    tl.phase("wait");
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, c.ev0, c.ev1) == cudaSuccess) { c.last_ms += ms; po->ms = ms; }
-    if (host_dbg) std::fprintf(stderr, "[psb] pass %lld..%lld host ms:%s\n", (long long)lo, (long long)hi, h_line.c_str());
     po->launches = c.launches - launches_at_entry;
-    for (auto &d : dbg_ev) {
-        float t = 0.f;
-        if (d.second.second && cudaEventElapsedTime(&t, d.second.first, d.second.second) == cudaSuccess)
-            std::fprintf(stderr, "[psb] %-48s %9.3f ms\n", d.first.c_str(), t);
-        cudaEventDestroy(d.second.first);
-        if (d.second.second) cudaEventDestroy(d.second.second);
-    }
-    if (dbg_time) std::fprintf(stderr, "[psb] pass of %lld pairs: timed region %.3f ms\n", (long long)n, ms);
+    tl.report(lo, hi, ms);
     return PSB_OK;
 }
 
@@ -1146,26 +1266,12 @@ int run_pairs(const PairsRequest &req, psb_batch_t **out) {
     // the walk) are cut so that a pass's decision bits + scratch stay within a budget of device memory
     int64_t budget = (int64_t)64 << 30;
     if (req.n > 4096 && (req.cfg.trace || req.cfg.stats)) {   // (a driver query: kept off the single-pair path)
-        // what is available = what the driver reports free + what this device's memory pool holds without using it.
-        // (Counting only the former makes the budget shrink as the pool warms up: every call would then cut its
-        // passes differently, ask for buffers of new sizes, grow the pool again ... -- calls of 2 s instead of 0.3 s.)
-        size_t free_b = 0, total_b = 0;
-        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess) {
-            cudaMemPool_t pool;
-            unsigned long long reserved = 0, used = 0;
-            if (cudaDeviceGetDefaultMemPool(&pool, c.device) == cudaSuccess &&
-                cudaMemPoolGetAttribute(pool, cudaMemPoolAttrReservedMemCurrent, &reserved) == cudaSuccess &&
-                cudaMemPoolGetAttribute(pool, cudaMemPoolAttrUsedMemCurrent, &used) == cudaSuccess && reserved > used)
-                free_b += (size_t)(reserved - used);
-            else cudaGetLastError();
-            budget = std::min<int64_t>(budget, (int64_t)(free_b / 2));
-        } else cudaGetLastError();
+        if (const size_t avail = device_mem_available()) budget = std::min<int64_t>(budget, (int64_t)(avail / 2));   // (0: unknown)
         budget = std::max<int64_t>(budget, (int64_t)1 << 30);
         budget = budget >> 30 << 30;   // whole gigabytes: small changes of the free figure do not move the cuts
     }
     const HostMatrix &hm0 = *req.matrix;
-    const bool p16_scheme = !std::getenv("PSB_NO_P16") && pairs16_scheme_ok(hm0.size, hm0.min, hm0.max, req.open, req.gap, hm0.type == PARASAIL_MATRIX_TYPE_PSSM) &&
-                            pairs16_trace_ok(hm0.min, hm0.max, req.open) && req.cfg.width != 32 && req.cfg.width != 64 && !req.extra;
+    const bool p16_scheme = p16_allowed(req) && pairs16_trace_ok(hm0.min, hm0.max, req.open) && !req.extra;
     // ---- passes.  A large batch is cut into passes twice over: by device memory (above) and by residues, so that
     // two host threads ("lanes", each with its own streams) can work on alternate passes: the uploads and the host
     // preparation of one pass run under the kernels of the other.  Small batches stay one pass on the calling thread.

@@ -42,6 +42,17 @@ struct HostMatrix {
 };
 
 // ---- results -------------------------------------------------------------------------------
+// The flag-byte / table block of one pair traced with K rows per lane (gotoh32_kernel) is [strip][step][lane][K]:
+// strips of 32 * K rows, rlen + 31 steps of a strip (lane l reaches column j at step j + l), one byte (or int) per
+// row of a lane.  The byte index of cell (i, j):
+inline size_t trace_cell_index(int K, int rlen, int i, int j) {
+    const int strip = i / (32 * K), rem = i % (32 * K), lane = rem / K, k = rem % K;
+    return (((size_t)strip * (rlen + 31) + (j + lane)) * 32 + lane) * K + k;
+}
+// and its size in cells (not rounded)
+inline long long trace_block_cells(int K, long long qlen, long long rlen) {
+    return ((qlen + 32 * K - 1) / (32 * K)) * (rlen + 31) * 32 * K;
+}
 }  // namespace psb
 
 struct psb_result_extra {
@@ -64,18 +75,17 @@ struct psb_result_extra {
         std::call_once(trace_once, [this]() {
             if (trace_blob.empty() && trace_lazy) { trace_lazy(this); trace_lazy = nullptr; }
             if (trace_blob.empty() || trace_K <= 0) return;
-            const int K = trace_K, nsteps = rlen + 31, rows = 32 * K;
+            const int K = trace_K, rows = 32 * K;
             trace.resize((size_t)qlen * rlen);
-            // cell (i, j) of strip i / rows sits at ((strip * nsteps + j + lane) * 32 + lane) * K + k: a row reads the
-            // block with a stride of one step record (32 * K bytes).  Column blocks of kBlock keep the ~kBlock + 31
-            // records a strip's rows share in cache (a 20 kb x 20 kb table: 400 MB through this loop)
+            // a row reads the block with a stride of one step record (32 * K bytes, psb::trace_cell_index).  Column
+            // blocks of kBlock keep the ~kBlock + 31 records a strip's rows share in cache (a 20 kb x 20 kb table:
+            // 400 MB through this loop)
             constexpr int kBlock = 64;
             for (int i0 = 0; i0 < qlen; i0 += rows)
                 for (int j0 = 0; j0 < rlen; j0 += kBlock) {
                     const int j1 = j0 + kBlock < rlen ? j0 + kBlock : rlen, i1 = i0 + rows < qlen ? i0 + rows : qlen;
                     for (int i = i0; i < i1; ++i) {
-                        const int strip = i0 / rows, rem = i - i0, lane = rem / K, k = rem % K;
-                        const uint8_t *src = trace_blob.data() + (((size_t)strip * nsteps + lane) * 32 + lane) * K + k;   // cell (i, 0)
+                        const uint8_t *src = trace_blob.data() + psb::trace_cell_index(K, rlen, i, 0);
                         int8_t *dst = trace.data() + (size_t)i * rlen;
                         for (int j = j0; j < j1; ++j) dst[j] = (int8_t)src[(size_t)j * rows];
                     }
