@@ -37,24 +37,32 @@ class Gotoh32Params(C.Structure):
                 ("banded", C.c_int), ("band_lo", C.c_int), ("band_hi", C.c_int)]
 
 
-def trace_to_rowmajor(blob, off, K, lq, lr):
-    """kernel trace layout [strip][step][lane][K] -> row-major lq x lr bytes"""
+def trace_to_rowmajor(blob, off, K, lq, lr, dtype=np.int8):
+    """kernel trace / table layout [strip][step][lane][K] -> row-major lq x lr cells"""
     nsteps = lr + 31
-    out = np.zeros((lq, lr), dtype=np.int8)
+    out = np.zeros((lq, lr), dtype=dtype)
     i = np.arange(lq)
     strip, rem = i // (32 * K), i % (32 * K)
     t, k = rem // K, rem % K
     for j in range(lr):
         s = j + t
         idx = off + ((strip * nsteps + s) * 32 + t) * K + k
-        out[:, j] = blob[idx].astype(np.int8)
+        out[:, j] = blob[idx].astype(dtype)
     return out
 
 
+TABLE_PLANES = ("score_table", "matches_table", "similar_table", "length_table")
+
+
 def gotoh32(qs, rs, mat, K, mode, open, gap, flags=(1, 1, 1, 1), stats=False, trace=False, wide=False,
-            shared_query=False, nblocks=1, profile=False, packed_bits=0):
-    """Run the emulated general kernel on pairs (lists of uint8 arrays of raw residues)."""
+            shared_query=False, nblocks=1, profile=False, packed_bits=0, table=False):
+    """Run the emulated general kernel on pairs (lists of uint8 arrays of raw residues).
+    table: the TABLE instantiation (statistics with the wide word, as the device runs it); the four int32 planes
+    come back row-major as outs[plane name][pair]."""
     assert lib().emu_sizeof_params() == C.sizeof(Gotoh32Params)
+    if table:
+        assert not trace and not profile and not packed_bits
+        stats = wide = True
     mapper = mat.mapper.astype(np.uint8)
     qm = [mapper[np.asarray(q, dtype=np.uint8)] for q in qs]
     rm = [mapper[np.asarray(r, dtype=np.uint8)] for r in rs]
@@ -63,7 +71,7 @@ def gotoh32(qs, rs, mat, K, mode, open, gap, flags=(1, 1, 1, 1), stats=False, tr
     qoff = np.zeros(len(qm) + 1, dtype=np.int64); qoff[1:] = np.cumsum([len(x) for x in qm])
     rcat = np.concatenate(rm).astype(np.uint8)
     roff = np.zeros(n + 1, dtype=np.int64); roff[1:] = np.cumsum([len(x) for x in rm])
-    table = np.ascontiguousarray(mat.table, dtype=np.int32)
+    matrix = np.ascontiguousarray(mat.table, dtype=np.int32)
     outs = {k: np.full(n, -777, dtype=np.int32) for k in ("score", "end_query", "end_ref", "matches", "similar", "length")}
     maxlr = int(max(len(x) for x in rm))
     per_col = 2 + (2 * (2 if wide else 1) if stats else 0)
@@ -77,12 +85,17 @@ def gotoh32(qs, rs, mat, K, mode, open, gap, flags=(1, 1, 1, 1), stats=False, tr
         trace_off[p] = tot
         tot += ((nstrips * (len(rm[p]) + 31) * 32 * K + 15) // 16) * 16
     blob = np.zeros(tot if trace else 16, dtype=np.uint8)
+    # (cells the kernel never writes keep a sentinel that no table value takes)
+    planes = [np.full(tot, -0x7fff0000, dtype=np.int32) for _ in TABLE_PLANES] if table else []
     ptr = lambda a: a.ctypes.data_as(C.c_void_p)
-    p = Gotoh32Params(ptr(qcat), ptr(qoff), ptr(rcat), ptr(roff), None, n, int(shared_query), ptr(table),
+    p = Gotoh32Params(ptr(qcat), ptr(qoff), ptr(rcat), ptr(roff), None, n, int(shared_query), ptr(matrix),
                       mat.size, int(mat.is_pssm), open, gap, mode, flags[0], flags[1], flags[2], flags[3],
                       ptr(outs["score"]), ptr(outs["end_query"]), ptr(outs["end_ref"]), ptr(outs["matches"]),
                       ptr(outs["similar"]), ptr(outs["length"]), ptr(bnd), per_col * maxlr, ptr(blob),
                       ptr(trace_off), ptr(counter), None, None, None, None, None, None, None, None, None, 0, None, 0, 0, 0)
+    if table:
+        p.tabH, p.tabM, p.tabS, p.tabL = (ptr(x).value for x in planes)
+        p.tab_off = ptr(trace_off).value
     if packed_bits:
         # subjects from the bit-packed store, in the store's (length-sorted) order; work count from memory
         words, word_off, lens, perm = pack_db(rm, packed_bits)
@@ -95,9 +108,11 @@ def gotoh32(qs, rs, mat, K, mode, open, gap, flags=(1, 1, 1, 1), stats=False, tr
     rc = lib().emu_gotoh32(K, int(stats), int(trace), int(wide), C.byref(p), nblocks)
     lib().emu_gotoh32_use_profile(0)
     assert rc == 0
+    lq_of = lambda i: len(qm[0]) if shared_query else len(qm[i])
     if trace:
-        outs["trace"] = [trace_to_rowmajor(blob, int(trace_off[i]), K, len(qm[0]) if shared_query else len(qm[i]), len(rm[i]))
-                         for i in range(n)]
+        outs["trace"] = [trace_to_rowmajor(blob, int(trace_off[i]), K, lq_of(i), len(rm[i])) for i in range(n)]
+    for name, plane in zip(TABLE_PLANES, planes):
+        outs[name] = [trace_to_rowmajor(plane, int(trace_off[i]), K, lq_of(i), len(rm[i]), np.int32) for i in range(n)]
     return outs
 
 

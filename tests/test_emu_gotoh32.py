@@ -87,6 +87,30 @@ def test_per_warp_profile_variant(oracle, blosum62, mode, variant):
     compare(oracle, mat, qs, rs, 2, mode, 0, 0, stats=variant == "stats", trace=variant == "trace", profile=True)
 
 
+@pytest.mark.parametrize("protein", [False, True])
+@pytest.mark.parametrize("K", [1, 2])
+def test_table_planes(oracle, blosum62, K, protein):
+    # the TABLE instantiation (single-pair _table / _rowcol exports): every cell of the score, matches, similar and
+    # length planes, with strips of 32 or 64 rows so that the pairs cross several strip boundaries (and end mid-strip)
+    mat = blosum62 if protein else oracle.Matrix.create(b"ACGT", 2, -3)
+    o, e = (10, 1) if protein else (5, 2)
+    qs, rs = pairs(81 + K, 3, (70, 150), (1, 90), protein)
+    qs[1] = qs[1][:32 * K + 1]   # one row into the second strip
+    cases = [(mode, (1, 1, 1, 1)) for mode in (0, 1, 2)] + [(1, f) for f in ((1, 0, 0, 0), (0, 1, 1, 0), (0, 0, 0, 1), (0, 1, 0, 1))]
+    for mode, flags in cases:
+        got = emu_harness.gotoh32(qs, rs, mat, K, mode, o, e, flags, table=True)
+        for i, (q, r) in enumerate(zip(qs, rs)):
+            exp = oracle.align(q, r, mat, mode=mode, open=o, gap=e, s1_beg=flags[0], s1_end=flags[1],
+                               s2_beg=flags[2], s2_end=flags[3], tables=True)
+            tag = (i, K, mode, flags, len(q), len(r))
+            assert (got["score"][i], got["end_query"][i], got["end_ref"][i]) == (exp["score"], exp["end_query"], exp["end_ref"]), tag
+            assert (got["matches"][i], got["similar"][i], got["length"][i]) == (exp["matches"], exp["similar"], exp["length"]), tag
+            for name in emu_harness.TABLE_PLANES:
+                bad = np.argwhere(got[name][i] != exp[name])
+                assert len(bad) == 0, f"{tag} {name}: {len(bad)} cells differ, first at (i, j) = {tuple(bad[0])}: " \
+                                      f"got {got[name][i][tuple(bad[0])]} expected {exp[name][tuple(bad[0])]}"
+
+
 @pytest.mark.parametrize("bits,protein", [(5, True), (2, False)])
 def test_packed_subjects_and_device_count(oracle, blosum62, bits, protein):
     # database-scan form: one query, subjects read from the 5-bit / 2-bit packed store, results
