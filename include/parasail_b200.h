@@ -220,9 +220,10 @@ void parasail_traceback_generic(const char *seqA, int lena, const char *seqB, in
                                 char match, char pos, char neg, int width, int name_width, int use_stats);
 
 /* ------------------------------------------------------------------------------------------
- * Part 1f: side APIs bound by parasail-rs but outside the accelerated path (SURVEY 8f item 4).
- * Exported so that the crate links; parasail_nw_banded runs the full (unbanded) NW fill on
- * the GPU and sets the BANDED flag, the SSW emulation returns NULL.
+ * Part 1f: side APIs bound by parasail-rs (SURVEY 8f item 4).  parasail_nw_banded fills only the
+ * band (half-width k, widened by the length difference) on the GPU's band kernel and sets the BANDED
+ * flag; a band that covers the whole table is an ordinary nw fill, a band wider than the band kernel's
+ * limit falls back to the masked full-table fill.  parasail_ssw is a local alignment with traceback.
  * ---------------------------------------------------------------------------------------- */
 parasail_result_t *parasail_nw_banded(const char *s1, int s1Len, const char *s2, int s2Len, int open, int gap,
                                       int k, const parasail_matrix_t *matrix); /* REF src/aligner/mod.rs:471 */
@@ -272,6 +273,16 @@ void psb_batch_free(psb_batch_t *batch);
 int psb_align_pairs(const char *fn_name, const parasail_matrix_t *matrix, int open, int gap,
                     const uint8_t *q_cat, const int64_t *q_off, const uint8_t *r_cat, const int64_t *r_off,
                     int64_t n, psb_batch_t **out);
+
+/* banded global alignment of many pairs: cell (i, j) is reachable iff lo <= j - i <= hi with d = rlen - qlen,
+ * lo = -k + min(d, 0), hi = k + max(d, 0) (the band of parasail_nw_banded).  Only the band is filled: work per pair
+ * is W * (qlen + rlen) cells with W = hi - lo + 1.  fn_name: the psb_align_pairs grammar restricted to nw (with or
+ * without _trace / _stats); the batch is the one psb_align_pairs returns for that name, with PARASAIL_FLAG_BANDED in
+ * batch->flag.  PSB_EINVAL: sg / sw names, k <= 0, NULL arguments, empty sequences; PSB_EUNSUPPORTED: _table /
+ * _rowcol, or a pair whose band neither covers its table nor fits the band kernel (W > 4096). */
+int psb_align_pairs_banded(const char *fn_name, const parasail_matrix_t *matrix, int open, int gap, int k,
+                           const uint8_t *q_cat, const int64_t *q_off, const uint8_t *r_cat, const int64_t *r_off,
+                           int64_t n, psb_batch_t **out);
 
 /* a database resident on the current device: residues mapped through `matrix`'s mapper and
  * bit-packed on the GPU -- 5 bit/residue for protein alphabets, 3 bit for alphabets of up to 8 letters,

@@ -662,6 +662,28 @@ class Aligner:
             raise DeviceError(f"psb_align_pairs failed ({rc_}): {last_error()}")
         return BatchResult(out)
 
+    def banded_nw_batch(self, queries, references):
+        """banded global alignment of many pairs (psb_align_pairs_banded) with the aligner's bandwidth(k): only the
+        band of each pair is filled.  Inputs as align_batch; use_trace() / use_stats() select the outputs."""
+        if not self._profile.is_null():
+            raise Panic("banded_nw_batch takes explicit queries, not a profile")
+        if not self.fn_name.startswith("nw"):
+            raise Panic(f"banded_nw_batch is global alignment only, not {self.fn_name}")
+        if self._bandwidth is None:
+            raise NoBandwidth()
+        qc, qo = _concat(queries)
+        rc, ro = _concat(references)
+        if len(qo) != len(ro):
+            raise Panic("banded_nw_batch: queries and references differ in count")
+        out = C.POINTER(CBatch)()
+        rc_ = lib().psb_align_pairs_banded(self.fn_name.encode(), self.matrix.inner, self.gap_open, self.gap_extend,
+                                           self._bandwidth, qc.ctypes.data_as(C.c_void_p), qo.ctypes.data_as(C.c_void_p),
+                                           rc.ctypes.data_as(C.c_void_p), ro.ctypes.data_as(C.c_void_p), len(ro) - 1,
+                                           C.byref(out))
+        if rc_ != 0:
+            raise DeviceError(f"psb_align_pairs_banded failed ({rc_}): {last_error()}")
+        return BatchResult(out)
+
     def scan(self, database):
         """the aligner's resident profile against a resident Database (psb_scan)"""
         if self._profile.is_null():

@@ -28,6 +28,7 @@
 #include <future>
 #include <vector>
 
+#include "kern_band32.cuh"
 #include "kern_gotoh32.cuh"
 #include "kern_sw16.cuh"
 #include "kern_util.cuh"
@@ -607,6 +608,45 @@ struct PassOut {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // (multi-lane only) begin / end of the pass on the device
 };
 
+// ---- banded nw (kern_band32.cuh) ----------------------------------------------------------------------
+// A pair of a banded request goes to the band kernel unless its band covers the whole table, boundary row and column
+// included: then nothing is masked and the pair is an ordinary nw pair (packed 16-bit, general or wavefront kernels).
+static bool band_covers(const BandGeom &b, int lq, int lr) { return b.lo <= -lq && b.hi >= lr; }
+static bool band_kernel_pair(const FnConfig &cfg, int lq, int lr) {
+    return cfg.band > 0 && cfg.mode == MODE_NW && !band_covers(band_geom(lq, lr, cfg.band), lq, lr);
+}
+// band-kernel variants: R = 2, 4, 8, 16 offsets per lane in registers, then the shared-memory form
+static constexpr int kBandGroups = 5;
+static int band_group(int W) {
+    for (int g = 0; g < 4; ++g) if (W <= 64 << g) return g;
+    return 4;
+}
+template <int R, bool SMEM> static const void *band32_fn_r(bool stats, bool trace) {
+    if (trace) return (const void *)band32_kernel<R, SMEM, false, true>;
+    if (stats) return (const void *)band32_kernel<R, SMEM, true, false>;
+    return (const void *)band32_kernel<R, SMEM, false, false>;
+}
+static const void *band32_fn(int group, bool stats, bool trace) {
+    switch (group) {
+        case 0: return band32_fn_r<2, false>(stats, trace);
+        case 1: return band32_fn_r<4, false>(stats, trace);
+        case 2: return band32_fn_r<8, false>(stats, trace);
+        case 3: return band32_fn_r<16, false>(stats, trace);
+        case 4: return band32_fn_r<2, true>(stats, trace);
+    }
+    return nullptr;
+}
+// cells of the table inside the band: the whole table less the two triangles beyond the band's edges
+static double band_cells(int lq, int lr, const BandGeom &b) {
+    // sum over x = 0 .. n-1 of max(0, m - x)
+    auto tri = [](long long m, long long n) -> double {
+        if (m <= 0) return 0;
+        if (m <= n) return (double)m * (m + 1) / 2;
+        return (double)n * m - (double)n * (n - 1) / 2;
+    };
+    return (double)lq * lr - tri((long long)lr - b.hi - 1, lq) - tri((long long)lq + b.lo - 1, lr);
+}
+
 // hands out the passes of a batch in order, cutting each one when it is asked for (thread-safe: the lanes ask)
 struct PassCutter {
     const PairsRequest &req;
@@ -630,7 +670,9 @@ struct PassCutter {
                 const int64_t lq = req.shared_query ? req.q_off[1] - req.q_off[0] : req.q_off[hi + 1] - req.q_off[hi];
                 const int64_t lr = req.r_off[hi + 1] - req.r_off[hi];
                 int64_t need;
-                if (p16_scheme && lq <= 512) need = (lr + 32) * (lq + 96) * 5 / 4 + 8 * (lq + lr);   // one byte of H per cell of the padded frame
+                if (band_kernel_pair(req.cfg, (int)lq, (int)lr))   // one flag byte per offset and row
+                    need = req.cfg.trace ? band_block_cells(lq, band_geom((int)lq, (int)lr, req.cfg.band).W) + 8 * (lq + lr) : 0;
+                else if (p16_scheme && lq <= 512) need = (lr + 32) * (lq + 96) * 5 / 4 + 8 * (lq + lr);   // one byte of H per cell of the padded frame
                 else if (req.cfg.trace) need = trace_block_cells(16, lq, lr) + 8 * (lq + lr);   // (16: the most rows per lane of any class)
                 else need = 0;
                 if (hi > lo && (bytes + need > budget || res_upto(hi + 1) - res_lo > pass_res)) break;
@@ -685,6 +727,9 @@ struct PassPlan {
     long long n_p16 = 0;
     std::vector<std::vector<int>> cls;        // pairs of each 32-bit class
     std::vector<int> wave_ids;                // long pairs: spread over the whole GPU one at a time
+    int band_k = 0;                           // banded nw: the band's half-width (0: no band kernel in this pass)
+    std::vector<int> band_ids[kBandGroups];   // pairs of each band-kernel variant (band_group)
+    int band_maxW[kBandGroups] = {};
     bool uniform = true;                      // every pair of the same lengths and class: no ordering needed
     int first_cls = -1;
     int max_lr_multistrip = 0;
@@ -713,7 +758,17 @@ static int plan_pass(const PairsRequest &req, int64_t lo, int64_t hi, PassPlan *
     P.q_two = req.shared_query || P.pssm;
     P.qbytes = P.pssm ? (size_t)m.length : (size_t)(P.q_hi - P.q_lo);
     P.want_table = req.extra && (cfg.table || cfg.rowcol);
-    P.banded = cfg.band > 0 && cfg.mode == MODE_NW && P.n == 1 && !cfg.stats && !cfg.trace && !P.want_table;
+    // banded nw: every pair whose band does not cover the table goes to the band kernel.  The single-pair API
+    // (parasail_nw_banded) keeps the masked general kernel for a band wider than kBandMaxW, and for every band under
+    // PSB_NO_BAND_KERNEL (A/B tests)
+    P.band_k = cfg.band > 0 && cfg.mode == MODE_NW ? cfg.band : 0;
+    if (P.band_k && req.extra && P.n == 1) {
+        const int lq0 = P.lq(0), lr0 = P.lr(0);
+        const BandGeom b = band_geom(lq0, lr0, P.band_k);
+        P.banded = (std::getenv("PSB_NO_BAND_KERNEL") || (!band_covers(b, lq0, lr0) && b.W > kBandMaxW)) && !cfg.stats && !cfg.trace &&
+                   !P.want_table;
+        if (P.banded) P.band_k = 0;
+    }
     P.fine = gotoh32_profile_ok(m.size, m.min, m.max, req.open, P.pssm) && !P.want_table && !P.banded;
     P.ct = class_table(P.fine);
     P.cls.resize(kNumClass);
@@ -745,6 +800,25 @@ static int plan_pass(const PairsRequest &req, int64_t lo, int64_t hi, PassPlan *
         if (lq <= 0 || lr <= 0) { set_error("empty sequence in batch (pair " + std::to_string(lo + i) + ")"); return PSB_EINVAL; }
         if (first_lq < 0) { first_lq = lq; first_lr = lr; }
         else if (lq != first_lq || lr != first_lr) P.uniform = false;
+        if (P.band_k) {
+            const BandGeom b = band_geom(lq, lr, P.band_k);
+            if (!band_covers(b, lq, lr)) {
+                if (b.W > kBandMaxW) {
+                    set_error("band of " + std::to_string(b.W) + " diagonals (pair " + std::to_string(lo + i) + ") is wider than the band kernel's " +
+                              std::to_string(kBandMaxW));
+                    return PSB_EUNSUPPORTED;
+                }
+                if (cfg.stats && (std::min(lq, lr) >= (1 << 21) || lq + lr >= (1 << 22))) {
+                    set_error("pair " + std::to_string(lo + i) + " too long for the band kernel's statistics word");
+                    return PSB_EUNSUPPORTED;
+                }
+                const int g = band_group(b.W);
+                P.band_ids[g].push_back((int)i);
+                P.band_maxW[g] = std::max(P.band_maxW[g], b.W);
+                P.cells += band_cells(lq, lr, b);
+                continue;
+            }
+        }
         if (P.p16_on && lq <= 512) {
             const int c16 = P.c16_of[lq];
             if (c16 >= 0 && pairs16_fits(p16_class(c16).G * p16_class(c16).K, lq, lr, m.max, m.min, req.open, req.gap, cfg.mode == MODE_SW)) {
@@ -796,6 +870,8 @@ struct PassBufs {
     std::vector<int> cls_item0, cls_id0;   // first item / pair of each packed class in d_items / d_ids16
     std::vector<DevMem> d_orders = std::vector<DevMem>(kNumClass);
     DevMem d_csroff, d_scan_tmp;
+    std::vector<DevMem> d_band_orders = std::vector<DevMem>(kBandGroups);
+    DevMem d_band_cnt;
 };
 
 // upload residues + offsets (relative to this range) and the matrix; references out of a resident database: their ids
@@ -853,12 +929,18 @@ static int alloc_pass(const PairsRequest &req, const PassPlan &P, PassBufs &B) {
     const long long rev_total = (P.q_two ? (long long)n * (long long)P.qbytes : (long long)(P.q_hi - P.q_lo)) + (long long)(P.r_hi - P.r_lo) + 2 * (long long)n;
     bool any32 = false;
     for (int cl = 0; cl < kNumClass; ++cl) any32 = any32 || !P.cls[cl].empty();
+    for (int g = 0; g < kBandGroups; ++g) any32 = any32 || !P.band_ids[g].empty();
     if ((cfg.trace || P.want_table) && any32) {
         B.trace_off.assign(n, 0);
         for (int cl = 0; cl < kNumClass; ++cl)
             for (int id : P.cls[cl]) {
                 B.trace_off[id] = B.trace_total;
                 B.trace_total += ((trace_block_cells(P.ct.k[cl], P.lq(id), P.lr(id)) + 15) / 16) * 16;
+            }
+        for (int g = 0; g < kBandGroups; ++g)
+            for (int id : P.band_ids[g]) {
+                B.trace_off[id] = B.trace_total;
+                B.trace_total += ((band_block_cells(P.lq(id), band_geom(P.lq(id), P.lr(id), P.band_k).W) + 15) / 16) * 16;
             }
         PSB_TRY(B.d_traceoff.alloc((size_t)n * sizeof(long long), c.stream));
         PSB_CUDA(cudaMemcpyAsync(B.d_traceoff.p, B.trace_off.data(), (size_t)n * sizeof(long long), cudaMemcpyHostToDevice, c.stream));
@@ -1072,6 +1154,54 @@ static int launch_waves(const PairsRequest &req, const PassPlan &P, PassBufs &B,
     return PSB_OK;
 }
 
+// the pairs of a banded request on the band kernel: one launch per variant, longest reference first
+static int launch_band(const PairsRequest &req, PassPlan &P, PassBufs &B) {
+    Ctx &c = g_ctx;
+    const FnConfig &cfg = req.cfg;
+    const Gotoh32Params &g = B.p;
+    bool any = false;
+    for (int gi = 0; gi < kBandGroups; ++gi) any = any || !P.band_ids[gi].empty();
+    if (!any) return PSB_OK;
+    PSB_TRY(B.d_band_cnt.alloc(sizeof(int) * kBandGroups, c.stream));
+    PSB_CUDA(cudaMemsetAsync(B.d_band_cnt.p, 0, sizeof(int) * kBandGroups, c.stream));
+    for (int gi = 0; gi < kBandGroups; ++gi) {
+        std::vector<int> &ids = P.band_ids[gi];
+        if (ids.empty()) continue;
+        P.longest_first(ids);
+        PSB_TRY(B.d_band_orders[gi].alloc(ids.size() * sizeof(int), c.stream));
+        PSB_CUDA(cudaMemcpyAsync(B.d_band_orders[gi].p, ids.data(), ids.size() * sizeof(int), cudaMemcpyHostToDevice, c.stream));
+        Band32Params p;
+        std::memset(&p, 0, sizeof(p));
+        p.q = g.q; p.q_off = g.q_off; p.r = g.r; p.r_off = g.r_off; p.shared_query = g.shared_query;
+        p.order = B.d_band_orders[gi].as<int>(); p.n = (int)ids.size();
+        p.matrix = g.matrix; p.size = g.size; p.is_pssm = g.is_pssm; p.open = g.open; p.gap = g.gap; p.k = P.band_k;
+        p.score = g.score; p.end_query = g.end_query; p.end_ref = g.end_ref;
+        p.matches = g.matches; p.similar = g.similar; p.length = g.length;
+        p.trace = g.trace; p.trace_off = g.trace_off;
+        p.counter = B.d_band_cnt.as<int>() + gi;
+        const bool smem_form = gi == kBandGroups - 1;
+        p.rr = smem_form ? 2 * ((P.band_maxW[gi] + 63) / 64) : 0;
+        const void *fn = band32_fn(gi, cfg.stats, cfg.trace);
+        // the shared-memory form: as many warps per CTA (up to kWarpsPerBlock) as the band state of each leaves room for
+        const size_t mat = band32_smem_bytes(g.is_pssm ? 0 : g.size, 1, false, 0, false);
+        int wpb = kWarpsPerBlock;
+        if (smem_form)
+            while (wpb > 1 && mat + (size_t)wpb * band32_warp_smem(p.rr, cfg.stats) > (size_t)200 * 1024) --wpb;
+        const size_t smem = band32_smem_bytes(g.is_pssm ? 0 : g.size, wpb, smem_form, p.rr, cfg.stats);
+        if (smem > (size_t)227 * 1024) { set_error("band state and substitution matrix too large for shared memory"); return PSB_EUNSUPPORTED; }
+        if (smem > 48 * 1024) PSB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        int per_sm = 0;
+        PSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, wpb * 32, smem));
+        if (per_sm < 1) per_sm = 1;
+        long long blocks = std::min<long long>((p.n + wpb - 1) / wpb, (long long)c.sms * per_sm);
+        if (blocks < 1) blocks = 1;
+        void *args[] = {&p};
+        PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(wpb * 32), args, smem, c.stream));
+        c.launches++;
+    }
+    return PSB_OK;
+}
+
 // traceback: the walks of the pairs on the 32-bit kernels, then the CIGAR CSR offsets (exclusive scan of the run counts)
 static int launch_walks(const PairsRequest &req, const PassPlan &P, PassBufs &B) {
     Ctx &c = g_ctx;
@@ -1091,6 +1221,18 @@ static int launch_walks(const PairsRequest &req, const PassPlan &P, PassBufs &B)
         w.rev_ops = B.d_rev.as<unsigned>(); w.rev_off = B.d_revoff.as<long long>();
         w.nops = B.d_nops.as<int>(); w.beg_query = B.d_beg[0].as<int>(); w.beg_ref = B.d_beg[1].as<int>();
         walk_trace_kernel<<<(w.n + 127) / 128, 128, 0, c.stream>>>(w);
+        c.launches++;
+    }
+    for (int gi = 0; gi < kBandGroups; ++gi) {
+        if (P.band_ids[gi].empty()) continue;
+        WalkParams w;
+        std::memset(&w, 0, sizeof(w));
+        w.q = p.q; w.q_off = p.q_off; w.r = p.r; w.r_off = p.r_off; w.shared_query = p.shared_query;
+        w.ids = B.d_band_orders[gi].as<int>(); w.n = (int)P.band_ids[gi].size();
+        w.trace = p.trace; w.trace_off = p.trace_off; w.end_query = p.end_query; w.end_ref = p.end_ref;
+        w.rev_ops = B.d_rev.as<unsigned>(); w.rev_off = B.d_revoff.as<long long>();
+        w.nops = B.d_nops.as<int>(); w.beg_query = B.d_beg[0].as<int>(); w.beg_ref = B.d_beg[1].as<int>();
+        walk_band_kernel<<<(w.n + 127) / 128, 128, 0, c.stream>>>(w, P.band_k);
         c.launches++;
     }
     // exclusive scan of nops[0..n] -> csr offsets (n+1)
@@ -1192,6 +1334,7 @@ static int run_pairs_range(const PairsRequest &req, int64_t lo, int64_t hi, psb_
     PSB_TRY(launch_pairs16(req, plan, bufs, tl));
     PSB_TRY(launch_classes(req, plan, bufs));
     PSB_TRY(launch_waves(req, plan, bufs, tl));
+    PSB_TRY(launch_band(req, plan, bufs));
     PSB_TRY(launch_walks(req, plan, bufs));
     PSB_CUDA(cudaEventRecord(c.ev1, c.stream));
     tl.phase("launches");
@@ -1822,18 +1965,18 @@ int psb_last_launches(void) { return g_ctx.launches; }
 
 void psb_batch_free(psb_batch_t *batch) { free_batch(batch); }
 
-int psb_align_pairs(const char *fn_name, const parasail_matrix_t *matrix, int open, int gap, const uint8_t *q_cat,
-                    const int64_t *q_off, const uint8_t *r_cat, const int64_t *r_off, int64_t n, psb_batch_t **out) {
-    FnConfig cfg;
-    if (!parse_fn_name(fn_name, &cfg) || cfg.profile) { set_error(std::string("psb_align_pairs: unknown function name: ") + (fn_name ? fn_name : "(null)")); return PSB_EINVAL; }
-    if (!matrix) { set_error("psb_align_pairs: NULL matrix"); return PSB_EINVAL; }
-    HostMatrix hm(matrix);
+}  // extern "C"
+
+namespace psb {
+// psb_align_pairs / psb_align_pairs_banded once the name is parsed: the pairs pass, then, for explicit narrow widths,
+// the pairs whose values do not fit flagged (SURVEY A.8), the same rule as align_one
+static int align_pairs(const FnConfig &cfg, const HostMatrix &hm, int open, int gap, const uint8_t *q_cat, const int64_t *q_off,
+                       const uint8_t *r_cat, const int64_t *r_off, int64_t n, psb_batch_t **out) {
     PairsRequest req;
     req.cfg = cfg; req.matrix = &hm; req.open = open; req.gap = gap;
     req.q_cat = q_cat; req.q_off = q_off; req.r_cat = r_cat; req.r_off = r_off; req.n = n;
     const int rc = run_pairs(req, out);
     if (rc == PSB_OK && (cfg.width == 8 || cfg.width == 16)) {
-        // explicit narrow widths: flag pairs whose values do not fit (SURVEY A.8), the same rule as align_one
         psb_batch_t *b = *out;
         const bool pssm = hm.type == PARASAIL_MATRIX_TYPE_PSSM;
         for (int64_t i = 0; i < n; ++i) {
@@ -1843,6 +1986,48 @@ int psb_align_pairs(const char *fn_name, const parasail_matrix_t *matrix, int op
             }
         }
     }
+    return rc;
+}
+}  // namespace psb
+
+extern "C" {
+
+int psb_align_pairs(const char *fn_name, const parasail_matrix_t *matrix, int open, int gap, const uint8_t *q_cat,
+                    const int64_t *q_off, const uint8_t *r_cat, const int64_t *r_off, int64_t n, psb_batch_t **out) {
+    FnConfig cfg;
+    if (!parse_fn_name(fn_name, &cfg) || cfg.profile) { set_error(std::string("psb_align_pairs: unknown function name: ") + (fn_name ? fn_name : "(null)")); return PSB_EINVAL; }
+    if (!matrix) { set_error("psb_align_pairs: NULL matrix"); return PSB_EINVAL; }
+    HostMatrix hm(matrix);
+    return align_pairs(cfg, hm, open, gap, q_cat, q_off, r_cat, r_off, n, out);
+}
+
+int psb_align_pairs_banded(const char *fn_name, const parasail_matrix_t *matrix, int open, int gap, int k, const uint8_t *q_cat,
+                           const int64_t *q_off, const uint8_t *r_cat, const int64_t *r_off, int64_t n, psb_batch_t **out) {
+    if (out) *out = nullptr;
+    FnConfig cfg;
+    if (!parse_fn_name(fn_name, &cfg) || cfg.profile) { set_error(std::string("psb_align_pairs_banded: unknown function name: ") + (fn_name ? fn_name : "(null)")); return PSB_EINVAL; }
+    if (cfg.mode != MODE_NW) { set_error(std::string("psb_align_pairs_banded: banded alignment is global only (nw): ") + fn_name); return PSB_EINVAL; }
+    if (cfg.table || cfg.rowcol) { set_error("psb_align_pairs_banded: _table/_rowcol outputs exist only on the single-pair API"); return PSB_EUNSUPPORTED; }
+    if (k <= 0) { set_error("psb_align_pairs_banded: band half-width " + std::to_string(k) + " is not positive"); return PSB_EINVAL; }
+    if (!matrix || !q_off || !r_cat || !r_off || !out || n <= 0 || (!q_cat && matrix->type != PARASAIL_MATRIX_TYPE_PSSM)) {
+        set_error("psb_align_pairs_banded: NULL argument or empty batch");
+        return PSB_EINVAL;
+    }
+    HostMatrix hm(matrix);
+    const bool pssm = hm.type == PARASAIL_MATRIX_TYPE_PSSM;
+    for (int64_t i = 0; i < n; ++i) {
+        const int lq = pssm ? hm.length : (int)(q_off[i + 1] - q_off[i]), lr = (int)(r_off[i + 1] - r_off[i]);
+        if (lq <= 0 || lr <= 0) { set_error("psb_align_pairs_banded: empty sequence in batch (pair " + std::to_string(i) + ")"); return PSB_EINVAL; }
+        const BandGeom b = band_geom(lq, lr, k);
+        if (!band_covers(b, lq, lr) && b.W > kBandMaxW) {
+            set_error("psb_align_pairs_banded: pair " + std::to_string(i) + " (" + std::to_string(lq) + " x " + std::to_string(lr) + ") has a band of W = " +
+                      std::to_string(b.W) + " diagonals; the band kernel takes at most " + std::to_string(kBandMaxW));
+            return PSB_EUNSUPPORTED;
+        }
+    }
+    cfg.band = k;
+    const int rc = align_pairs(cfg, hm, open, gap, q_cat, q_off, r_cat, r_off, n, out);
+    if (rc == PSB_OK) (*out)->flag |= PARASAIL_FLAG_BANDED;
     return rc;
 }
 

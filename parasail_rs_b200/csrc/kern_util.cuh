@@ -175,6 +175,51 @@ PSB_KERNEL void walk_trace_kernel(WalkParams p) {
     p.beg_ref[pid] = j + 1;
 }
 
+// The same walk over the band-layout trace bytes of band32_kernel (row i, offset t = j - i - lo at byte i * W + t),
+// from the corner (Lq - 1, Lr - 1); `K` of the parameters is unused, `k` is the band's half-width.  Same run lists,
+// same scratch: compact_cigar_kernel and the CIGAR CSR build take them as they are.
+PSB_KERNEL void walk_band_kernel(WalkParams p, int k) {
+    const long long t = (long long)block_id() * threads_per_block() + thread_in_block();
+    if (t >= p.n) return;
+    const int pid = p.ids ? p.ids[t] : (int)t;
+    const long long qo = p.shared_query ? p.q_off[0] : p.q_off[pid];
+    const uint8_t *q = p.q + qo;
+    const int Lq = (int)((p.shared_query ? p.q_off[1] : p.q_off[pid + 1]) - qo);
+    const long long ro = p.r_off[pid];
+    const uint8_t *r = p.r + ro;
+    const int Lr = (int)(p.r_off[pid + 1] - ro);
+    const int d = Lr - Lq, lo = -k + (d < 0 ? d : 0), W = 2 * k + (d < 0 ? -d : d) + 1;
+    const uint8_t *tr = p.trace + p.trace_off[pid];
+    unsigned *out = p.rev_ops + p.rev_off[pid];
+    int i = Lq - 1, j = Lr - 1;
+    int where = TR_DIAG, cur = -1, n = 0;
+    unsigned len = 0;
+    while (i >= 0 || j >= 0) {
+        int op;
+        if (i < 0) { op = 2; --j; }
+        else if (j < 0) { op = 1; --i; }
+        else {
+            const int tf = tr[(size_t)i * W + (j - i - lo)];
+            if (where == TR_DIAG) {
+                if (tf & TR_DIAG) { op = (q[i] == r[j]) ? 7 : 8; --i; --j; }
+                else if (tf & TR_INS) { where = TR_INS; continue; }
+                else if (tf & TR_DEL) { where = TR_DEL; continue; }
+                else break;
+            } else if (where == TR_INS) { op = 2; where = (tf & TR_DIAG_E) ? TR_DIAG : TR_INS; --j; }
+            else { op = 1; where = (tf & TR_DIAG_F) ? TR_DIAG : TR_DEL; --i; }
+        }
+        if (op == cur) ++len;
+        else {
+            if (cur >= 0) out[n++] = (len << 4) | (unsigned)cur;
+            cur = op; len = 1;
+        }
+    }
+    if (cur >= 0) out[n++] = (len << 4) | (unsigned)cur;
+    p.nops[pid] = n;
+    p.beg_query[pid] = i + 1;
+    p.beg_ref[pid] = j + 1;
+}
+
 struct CompactParams {
     const unsigned *rev_ops;
     const long long *rev_off;   // by pair id

@@ -53,6 +53,11 @@ inline size_t trace_cell_index(int K, int rlen, int i, int j) {
 inline long long trace_block_cells(int K, long long qlen, long long rlen) {
     return ((qlen + 32 * K - 1) / (32 * K)) * (rlen + 31) * 32 * K;
 }
+// The flag-byte block of one pair on the band kernel (band32_kernel, band of W offsets starting at diagonal lo =
+// j - i of offset 0) is [row][offset]: the byte index of cell (i, j) of the band
+inline size_t band_cell_index(int W, int lo, int i, int j) { return (size_t)i * W + (size_t)(j - i - lo); }
+// and the block's size in cells
+inline long long band_block_cells(long long qlen, int W) { return qlen * W; }
 }  // namespace psb
 
 struct psb_result_extra {

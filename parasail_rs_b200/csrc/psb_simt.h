@@ -11,6 +11,7 @@
 // ------------------------------------------------------------------------------------------
 #include <cuda_runtime.h>
 #define PSB_DEV __device__ __forceinline__
+#define PSB_HD __host__ __device__ __forceinline__   // shared by a kernel and its host-side launcher
 #define PSB_KERNEL __global__
 #define PSB_SHARED_DECL(name) extern __shared__ __align__(16) unsigned char name[]
 
@@ -67,6 +68,7 @@ PSB_DEV unsigned prmt(unsigned a, unsigned b, unsigned sel) {
 #include <thread>
 #include <vector>
 #define PSB_DEV inline
+#define PSB_HD inline
 #define PSB_KERNEL
 #define PSB_SHARED_DECL(name) unsigned char *name = psb::emu::tls().smem
 
