@@ -8,6 +8,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <memory>
@@ -258,6 +259,23 @@ struct BatchImpl {
     }
 };
 
+// a batch's per-pair result arrays in the order the kernels' outputs use (score, end_query, end_ref, then the statistics)
+static std::array<int *, 6> batch_outputs(psb_batch_t *b) { return {b->score, b->end_query, b->end_ref, b->matches, b->similar, b->length}; }
+// the length of sequence i of a concatenation
+static int span(const int64_t *off, int64_t i) { return (int)(off[i + 1] - off[i]); }
+// explicit _8/_16 widths: the pairs whose values do not fit are flagged and their results zeroed (SURVEY A.8), by the
+// rule of saturates(); `lens(i)` is pair i's (query, reference) lengths
+template <typename Lens>
+static void flag_saturated(const FnConfig &cfg, const HostMatrix &hm, int open, int gap, psb_batch_t *b, Lens lens) {
+    if (cfg.width != 8 && cfg.width != 16) return;
+    for (int64_t i = 0; i < b->n; ++i) {
+        const std::pair<int, int> l = lens(i);
+        if (saturates(cfg, hm, b->score[i], l.first, l.second, open, gap)) {
+            b->saturated[i] = 1; b->score[i] = 0; b->end_query[i] = 0; b->end_ref[i] = 0;
+        }
+    }
+}
+
 static void fill_lut(unsigned *lut, const uint8_t *mapper) {
     for (int i = 0; i < 64; ++i)
         lut[i] = (unsigned)mapper[4 * i] | ((unsigned)mapper[4 * i + 1] << 8) | ((unsigned)mapper[4 * i + 2] << 16) |
@@ -338,15 +356,11 @@ static int launch_gotoh32(int K, Variant v, Gotoh32Params &p, int nwork, bool pr
     const int statw = v == V_STATS32 ? 4 : 8;
     const size_t smem = gotoh32_smem_bytes(p.is_pssm ? 0 : p.size, kWarpsPerBlock, stats, statw, prof);
     if (smem > 200 * 1024) { set_error("substitution matrix too large for shared memory"); return PSB_EUNSUPPORTED; }
-    if (smem > 48 * 1024) PSB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
-    PSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kWarpsPerBlock * 32, smem));
-    if (per_sm < 1) per_sm = 1;
-    long long blocks = std::min<long long>((nwork + kWarpsPerBlock - 1) / kWarpsPerBlock, (long long)c.sms * per_sm);
-    if (blocks < 1) blocks = 1;
+    long long blocks = 0;
+    PSB_CUDA(occupancy_per_sm(fn, kWarpsPerBlock, smem, &per_sm));
+    PSB_CUDA(launch_persistent(fn, &p, nwork, kWarpsPerBlock, smem, per_sm, c.sms, c.stream, &blocks));
     if (grid_warps_out) *grid_warps_out = blocks * kWarpsPerBlock;
-    void *args[] = {&p};
-    PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(kWarpsPerBlock * 32), args, smem, c.stream));
     c.launches++;
     return PSB_OK;
 }
@@ -506,6 +520,23 @@ static WaveShape wave_shape(const HostMatrix &m, int open, int gap, bool is_sw, 
     return s;
 }
 
+// What every wavefront launch fills alike in its two parameter blocks: the pair (for several subjects: the query and
+// their bytes, lr = 0), scoring, mode and end gaps (`md`: a Gotoh32Params or a FnConfig), the strip buffers (ctl: the
+// strip counter, then per-strip progress) and the outputs.  The rest is zero: the multi-pair fields (multi_n, r_off,
+// out_map) and the trace records are the caller's to set.
+template <typename Mode>
+static void wave_params(const Mode &md, const uint8_t *q, const uint8_t *r, int lq, int lr, const int *matrix, int size, int open, int gap,
+                        int nstrips, int *bnd, int *ctl, int *cand, int *score, int *end_query, int *end_ref, Wave32Params *p, WaveReduceParams *rp) {
+    std::memset(p, 0, sizeof(*p));
+    p->q = q; p->r = r; p->Lq = lq; p->Lr = lr;
+    p->matrix = matrix; p->size = size; p->open = open; p->gap = gap;
+    p->mode = md.mode; p->s1_beg = md.s1_beg; p->s1_end = md.s1_end; p->s2_beg = md.s2_beg; p->s2_end = md.s2_end;
+    p->bnd = bnd; p->progress = ctl + 1; p->next_strip = ctl; p->cand = cand;
+    std::memset(rp, 0, sizeof(*rp));
+    rp->cand = cand; rp->nstrips = nstrips; rp->mode = md.mode; rp->s1_end = md.s1_end; rp->s2_end = md.s2_end; rp->Lr = lr;
+    rp->score = score; rp->end_query = end_query; rp->end_ref = end_ref;
+}
+
 static int launch_wave32(const Gotoh32Params &g, const HostMatrix &m, long long q_byte_off, int lq, long long r_byte_off, int lr, int out_index,
                          const WaveWalk *ww, PassTimeline &tl) {
     Ctx &c = g_ctx;
@@ -527,26 +558,15 @@ static int launch_wave32(const Gotoh32Params &g, const HostMatrix &m, long long 
     // generation 3 hands rows over through self-validating words: the lines start out all-zero (invalid)
     if (v3) PSB_CUDA(cudaMemsetAsync(d_bnd.p, 0, (size_t)nstrips * 2 * (size_t)lr * sizeof(int), c.stream));
     Wave32Params p;
-    p.q = g.q + q_byte_off; p.r = g.r + r_byte_off; p.Lq = lq; p.Lr = lr;
-    p.matrix = g.matrix; p.size = g.size; p.open = g.open; p.gap = g.gap;
-    p.mode = g.mode; p.s1_beg = g.s1_beg; p.s1_end = g.s1_end; p.s2_beg = g.s2_beg; p.s2_end = g.s2_end;
-    p.bnd = d_bnd.as<int>(); p.progress = d_ctl.as<int>() + 1; p.next_strip = d_ctl.as<int>(); p.cand = d_cand.as<int>();
-    p.multi_n = 0; p.r_off = nullptr;
+    WaveReduceParams r;
+    wave_params(g, g.q + q_byte_off, g.r + r_byte_off, lq, lr, g.matrix, g.size, g.open, g.gap, nstrips, d_bnd.as<int>(), d_ctl.as<int>(),
+                d_cand.as<int>(), g.score + out_index, g.end_query + out_index, g.end_ref + out_index, &p, &r);
     p.trace_h = d_th.as<uint4>(); p.trace_bits = d_tb.as<uint2>();
     const size_t smem = v3 ? wave32v3_smem_bytes(g.size, wpb, K) : (s.gen == 2 ? wave32v2_smem_bytes(g.size, wpb) : wave32_smem_bytes(g.size, wpb));
-    if (smem > 48 * 1024) PSB_CUDA(cudaFuncSetAttribute(s.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    PSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, s.fn, wpb * 32, smem));
-    if (per_sm < 1) per_sm = 1;
     // every launched warp must be resident at once: the strips wait on one another
-    long long blocks = std::min<long long>((nstrips + wpb - 1) / wpb, (long long)c.sms * per_sm);
-    if (blocks < 1) blocks = 1;
-    void *args[] = {&p};
-    PSB_CUDA(cudaLaunchKernel(s.fn, dim3((unsigned)blocks), dim3(wpb * 32), args, smem, c.stream));
-    WaveReduceParams r;
-    r.cand = d_cand.as<int>(); r.nstrips = nstrips; r.mode = g.mode; r.s1_end = g.s1_end; r.s2_end = g.s2_end; r.Lr = lr;
-    r.score = g.score + out_index; r.end_query = g.end_query + out_index; r.end_ref = g.end_ref + out_index;
-    r.multi_n = 0; r.r_off = nullptr; r.out_map = nullptr; r.first_id = 0;
+    int per_sm = 0;
+    PSB_CUDA(occupancy_per_sm(s.fn, wpb, smem, &per_sm));
+    PSB_CUDA(launch_persistent(s.fn, &p, nstrips, wpb, smem, per_sm, c.sms, c.stream));
     wave32_reduce_kernel<<<1, 32, 0, c.stream>>>(r);
     c.launches += 2;
     if (ww) {
@@ -1189,14 +1209,9 @@ static int launch_band(const PairsRequest &req, PassPlan &P, PassBufs &B) {
             while (wpb > 1 && mat + (size_t)wpb * band32_warp_smem(p.rr, cfg.stats) > (size_t)200 * 1024) --wpb;
         const size_t smem = band32_smem_bytes(g.is_pssm ? 0 : g.size, wpb, smem_form, p.rr, cfg.stats);
         if (smem > (size_t)227 * 1024) { set_error("band state and substitution matrix too large for shared memory"); return PSB_EUNSUPPORTED; }
-        if (smem > 48 * 1024) PSB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int per_sm = 0;
-        PSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, wpb * 32, smem));
-        if (per_sm < 1) per_sm = 1;
-        long long blocks = std::min<long long>((p.n + wpb - 1) / wpb, (long long)c.sms * per_sm);
-        if (blocks < 1) blocks = 1;
-        void *args[] = {&p};
-        PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(wpb * 32), args, smem, c.stream));
+        PSB_CUDA(occupancy_per_sm(fn, wpb, smem, &per_sm));
+        PSB_CUDA(launch_persistent(fn, &p, p.n, wpb, smem, per_sm, c.sms, c.stream));
         c.launches++;
     }
     return PSB_OK;
@@ -1250,7 +1265,7 @@ static int launch_walks(const PairsRequest &req, const PassPlan &P, PassBufs &B)
 static int copy_results(const PairsRequest &req, const PassPlan &P, PassBufs &B, psb_batch_t *b, PassOut *po, PassTimeline &tl) {
     Ctx &c = g_ctx;
     const int64_t n = P.n, lo = P.lo;
-    int *outs[6] = {b->score, b->end_query, b->end_ref, b->matches, b->similar, b->length};
+    const std::array<int *, 6> outs = batch_outputs(b);
     const int ncopy = req.cfg.stats ? 6 : 3;
     for (int k = 0; k < ncopy; ++k)
         PSB_CUDA(cudaMemcpyAsync(outs[k] + lo, B.d_out[k].p, (size_t)n * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
@@ -1699,221 +1714,259 @@ static void sw16_rate_update(int K, double cells, double ms) {
 // is -- what limits strong scaling at 8 GPUs.  Those few subjects ("head") are therefore swept by
 // a separate small launch of the same kernel, one warp per SM sub-partition on SMs it owns
 // outright, beside the main launch.
-static int scan_sw16(const FnConfig &cfg, const parasail_profile *prof, DevProfile *dp, const std::vector<Sw16Profile> &strips, int open, int gap, psb_db *db,
-                     int *const d_out[6], int64_t *n_retried, int *retried_host) {
-    Ctx &c = g_ctx;
-    const Sw16Profile &sp = strips[0];
-    const bool multi = strips.size() > 1;
-    const HostMatrix &m = prof->matrix;
-    const int lq = (int)prof->query.size();
+//
+// What one scan launches, decided before the first launch.  The database is sorted by decreasing length: the first
+// nroute subjects go to the wavefront kernel, the next nhead to the head launch, the rest to the main launch.
+struct ScanPlan {
+    double rate = 0, est_ms = 0, long_len = 0;
+    int64_t nroute = 0, nhead = 0;
+    int64_t nshort = 0;     // subjects on the packed kernel (head included)
+    bool multi = false;     // the query has several strips: one sweep of every subject per strip, no head
+    bool general = false;   // more over-long subjects than the route takes: the whole job goes to scan_general
+};
+static ScanPlan plan_scan(const std::vector<Sw16Profile> &strips, int lq, const psb_db *db) {
+    ScanPlan P;
+    const int K = strips[0].K;
+    P.multi = strips.size() > 1;
     // Keep a subject's serial sweep under ~40 % of the time the whole shard needs.  Both figures follow from
     // ONE quantity, the scan rate of this kernel class on this device, which is measured, not assumed: every
     // finished scan job updates it (scan_finish); 4.9 TCUPS is only the value before the first measurement.
     // A group step advances 64*K cells of one of the SM's 16 resident warps: step = 64*K*16*SMs / rate.
-    const double rate = sw16_rate_get(sp.K);
-    const double est_ms = (double)lq * (double)db->residues / rate * 1e3;
-    const double step_ms = 64.0 * sp.K * 16.0 * c.sms / rate * 1e3;
-    const double long_len = std::max(1024.0, 0.4 * est_ms / step_ms);
-    int64_t nroute = 0;
-    while (nroute < (int64_t)db->top_len.size() && db->top_len[nroute] > 65535) ++nroute;
-    int64_t nhead = nroute;
-    while (nhead < (int64_t)db->top_len.size() && db->top_len[nhead] > long_len) ++nhead;
-    nhead = std::min<int64_t>(((nhead - nroute + 3) / 4) * 4, std::max<int64_t>(0, (db->n - nroute) / 8 / 4 * 4));
-    if (multi) nhead = 0;   // strip by strip: every strip sweeps all subjects in one launch
-    if (db->nlong > nroute) {
+    P.rate = sw16_rate_get(K);
+    P.est_ms = (double)lq * (double)db->residues / P.rate * 1e3;
+    const double step_ms = 64.0 * K * 16.0 * g_ctx.sms / P.rate * 1e3;
+    P.long_len = std::max(1024.0, 0.4 * P.est_ms / step_ms);
+    while (P.nroute < (int64_t)db->top_len.size() && db->top_len[P.nroute] > 65535) ++P.nroute;
+    int64_t nhead = P.nroute;
+    while (nhead < (int64_t)db->top_len.size() && db->top_len[nhead] > P.long_len) ++nhead;
+    P.nhead = std::min<int64_t>(((nhead - P.nroute + 3) / 4) * 4, std::max<int64_t>(0, (db->n - P.nroute) / 8 / 4 * 4));
+    if (P.multi) P.nhead = 0;
+    P.nshort = db->n - P.nroute;
+    P.general = db->nlong > P.nroute;
+    if (!P.general && std::getenv("PSB_DEBUG_TIMING"))
+        std::fprintf(stderr, "[psb] sw16: n %lld residues %lld est %.2f ms long_len %.0f nroute %lld nhead %lld top %d\n", (long long)db->n,
+                     (long long)db->residues, P.est_ms, P.long_len, (long long)P.nroute, (long long)P.nhead, db->top_len.empty() ? 0 : db->top_len[0]);
+    return P;
+}
+
+// device buffers the launches of one scan share; freed in stream order when the scan returns
+struct ScanBufs {
+    DevMem retry, cnt;                     // the re-run list; counters: re-runs, main launch, head launch
+    DevMem lbytes, loff, bnd, ctl, cand;   // routed subjects: their bytes, offsets and wavefront state
+    DevMem bndA, bndB;                     // strip by strip: the bottom rows handed to the strip below
+};
+
+// what every packed launch of a scan fills alike: the profile (strip), penalties, database, outputs and re-run list
+static Sw16Params sw16_base_params(const Sw16Profile &sp, int open, int gap, const psb_db *db, int *const d_out[6], ScanBufs &B) {
+    Sw16Params p;
+    std::memset(&p, 0, sizeof(p));
+    p.prof = sp.prof; p.nletters = sp.nletters; p.lq = sp.lq; p.open = open; p.gap = gap; p.max_score = sp.max_score;
+    p.words = db->d_words; p.bits = db->bits;
+    p.score = d_out[0]; p.end_query = d_out[1]; p.end_ref = d_out[2];
+    p.retry = B.retry.as<int>(); p.retry_count = B.cnt.as<int>();
+    p.mul_one = 1u; p.mul_64k = 65536u;
+    return p;
+}
+// the launch's subjects: sorted positions first .. first + n - 1
+static void sw16_subjects(Sw16Params &p, const psb_db *db, int64_t first, int64_t n) {
+    p.word_off = db->d_word_off + first; p.len = db->d_len + first; p.n = n; p.out_map = db->d_perm + first;
+    p.sid_base = (int)first;
+}
+
+// CTA size of a packed launch: two CTAs of 8 warps when their profile copies fit an SM together, else one of 16
+// (long queries with a protein alphabet: one 50 KB profile copy instead of two).  The kernel's shared-memory limit
+// is first raised to the largest of both shapes and `other_smem`, the request of another launch of the kernel.
+struct Sw16Shape { int wpb, per_sm; size_t smem; };
+static int sw16_cta_shape(const void *fn, const Sw16Profile &sp, bool strip, size_t other_smem, Sw16Shape *out) {
+    int wpb = kSw16WarpsPerBlock, per_sm = 0;
+    size_t smem = sw16_smem_bytes(sp.nletters, sp.K, wpb, strip);
+    const size_t smem16 = sw16_smem_bytes(sp.nletters, sp.K, 16, strip);
+    PSB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(std::max(smem, other_smem), smem16)));
+    PSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, wpb * 32, smem));
+    if (per_sm * wpb < 16) {
+        int per_sm16 = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm16, fn, 16 * 32, smem16) == cudaSuccess && per_sm16 * 16 > per_sm * wpb) {
+            wpb = 16; per_sm = per_sm16; smem = smem16;
+        } else cudaGetLastError();
+    }
+    *out = {wpb, std::max(per_sm, 1), smem};
+    return PSB_OK;
+}
+
+// the subjects too long for the packed kernel's 16-bit column indices: unpacked to bytes and swept by the multi-pair
+// wavefront kernel, then reduced into the results
+static int launch_route(const FnConfig &cfg, const parasail_profile *prof, DevProfile *dp, int open, int gap, const psb_db *db,
+                        const ScanPlan &P, int *const d_out[6], ScanBufs &B) {
+    if (P.nroute == 0) return PSB_OK;
+    Ctx &c = g_ctx;
+    const HostMatrix &m = prof->matrix;
+    const int lq = (int)prof->query.size();
+    const int64_t nroute = P.nroute;
+    std::vector<long long> loff(nroute + 1);
+    loff[0] = 0;
+    for (int64_t i = 0; i < nroute; ++i) loff[i + 1] = loff[i] + db->top_len[i];
+    const int K = lq <= 64 ? 1 : 2;
+    const int nstrips = (lq + 32 * K - 1) / (32 * K);
+    PSB_TRY(B.lbytes.alloc((size_t)loff[nroute], c.stream));
+    PSB_TRY(B.loff.alloc((size_t)(nroute + 1) * sizeof(long long), c.stream));
+    PSB_TRY(B.bnd.alloc((size_t)nstrips * 2 * (size_t)loff[nroute] * sizeof(int), c.stream));
+    PSB_TRY(B.ctl.alloc(((size_t)nroute * nstrips + 2) * sizeof(int), c.stream));
+    PSB_TRY(B.cand.alloc((size_t)nroute * nstrips * 8 * sizeof(int), c.stream));
+    PSB_CUDA(cudaMemcpyAsync(B.loff.p, loff.data(), (size_t)(nroute + 1) * sizeof(long long), cudaMemcpyHostToDevice, c.stream));
+    PSB_CUDA(cudaMemsetAsync(B.ctl.p, 0, ((size_t)nroute * nstrips + 2) * sizeof(int), c.stream));
+    PSB_CUDA(cudaStreamSynchronize(c.stream));  // `loff` is a host temporary
+    UnpackParams u;
+    u.words = db->d_words; u.word_off = db->d_word_off; u.ids = nullptr; u.inv_perm = nullptr; u.out_off = B.loff.as<long long>();
+    u.out = B.lbytes.as<uint8_t>(); u.n = nroute; u.bits = db->bits;
+    unpack_db_kernel<<<(unsigned)std::min<int64_t>(nroute, 1024), 256, 0, c.stream>>>(u);
+    Wave32Params w;
+    WaveReduceParams r;
+    wave_params(cfg, dp->d_query, B.lbytes.as<uint8_t>(), lq, 0, dp->d_matrix, m.size, open, gap, nstrips, B.bnd.as<int>(), B.ctl.as<int>(),
+                B.cand.as<int>(), d_out[0], d_out[1], d_out[2], &w, &r);
+    w.multi_n = (int)nroute; w.r_off = B.loff.as<long long>();
+    r.multi_n = (int)nroute; r.r_off = B.loff.as<long long>(); r.out_map = db->d_perm;
+    const bool v2 = wave32_v2_ok(m, open, gap);
+    const void *fn = wave32_fn(K, v2);
+    // Full-size CTAs that also reserve most of an SM's shared memory: the strips of the long
+    // subjects then own a few SMs outright instead of crawling beside sixteen ALU-bound warps
+    // of the main kernel on every SM (each of their steps is a serial dependency).  The main
+    // kernel's blocks that find no room start on those SMs as soon as the strips are done.
+    const int kRouteWarps = v2 ? 8 : 32;   // generation 2 keeps a 12 KB profile per warp
+    const size_t smem = std::max<size_t>(v2 ? wave32v2_smem_bytes(m.size, kRouteWarps) : wave32_smem_bytes(m.size, kRouteWarps), 160 * 1024);
+    PSB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    // all warps of this launch must be resident together (strips wait on one another): one CTA
+    // per SM at most, issued before the main kernel so that its blocks are placed first
+    const long long items = nroute * nstrips;
+    long long blocks = std::min<long long>((items + kRouteWarps - 1) / kRouteWarps, (long long)c.sms);
+    void *args[] = {&w};
+    PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(kRouteWarps * 32), args, smem, c.stream));
+    wave32_reduce_kernel<<<(unsigned)((nroute + 127) / 128), 128, 0, c.stream>>>(r);
+    c.launches += 3;
+    return PSB_OK;
+}
+
+// ---- queries of several strips: one sweep of the database per strip; the bottom row of a strip (T and Fh of both
+// subjects of a word, one uint2 per column) goes through HBM to the strip below: 16 bytes per column and strip
+// boundary against ~K*16*2.5 instructions of fill per column
+static int launch_sw16_strips(const std::vector<Sw16Profile> &strips, int open, int gap, psb_db *db, const ScanPlan &P, int *const d_out[6],
+                              ScanBufs &B) {
+    if (P.nshort == 0 || !P.multi) return PSB_OK;
+    Ctx &c = g_ctx;
+    if (!db->d_res_off) {
+        std::lock_guard<std::mutex> lk(db->mu);
+        if (!db->d_res_off) {
+            long long *ro = nullptr;
+            PSB_CUDA(cudaMallocAsync(&ro, ((size_t)db->n + 1) * sizeof(long long), db->stream));
+            if (db->stream != c.stream) PSB_CUDA(cudaStreamSynchronize(db->stream));
+            size_t tb = 0;
+            DevMem d_tmp;
+            PSB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb, db->d_len, ro, (int)db->n, c.stream));
+            PSB_TRY(d_tmp.alloc(tb, c.stream));
+            PSB_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp.p, tb, db->d_len, ro, (int)db->n, c.stream));
+            PSB_CUDA(cudaStreamSynchronize(c.stream));
+            db->d_res_off = ro;
+        }
+    }
+    PSB_TRY(B.bndA.alloc(((size_t)db->residues + 64) * sizeof(uint2), c.stream));
+    PSB_TRY(B.bndB.alloc(((size_t)db->residues + 64) * sizeof(uint2), c.stream));
+    for (size_t st = 0; st < strips.size(); ++st) {
+        const Sw16Profile &ss = strips[st];
+        Sw16Params p = sw16_base_params(ss, open, gap, db, d_out, B);
+        sw16_subjects(p, db, P.nroute, P.nshort);
+        p.res_off = db->d_res_off + P.nroute;
+        p.bnd_in = st == 0 ? nullptr : ((st & 1) ? B.bndA.as<uint2>() : B.bndB.as<uint2>());
+        p.bnd_out = st + 1 == strips.size() ? nullptr : ((st & 1) ? B.bndB.as<uint2>() : B.bndA.as<uint2>());
+        p.row0 = ss.row0; p.merge = st > 0 ? 1 : 0;
+        DevMem d_cnt_st;   // a work counter per launch
+        PSB_TRY(d_cnt_st.alloc(sizeof(int), c.stream));
+        PSB_CUDA(cudaMemsetAsync(d_cnt_st.p, 0, sizeof(int), c.stream));
+        p.counter = d_cnt_st.as<int>();
+        const void *fn = sw16_fn(ss.K, true);
+        if (!fn) { set_error("sw16: no strip kernel for this query length"); return PSB_EUNSUPPORTED; }
+        Sw16Shape s;
+        PSB_TRY(sw16_cta_shape(fn, ss, true, 0, &s));
+        const long long slots = ((P.nshort + 1) / 2 + 1) / 2;
+        PSB_CUDA(launch_persistent(fn, &p, slots, s.wpb, s.smem, s.per_sm, c.sms, c.stream));
+        c.launches++;
+    }
+    return PSB_OK;
+}
+
+// a single-strip query: the head launch on the compute stream, then the main launch on `main_stream`
+static int launch_sw16(const Sw16Profile &sp, int open, int gap, const psb_db *db, const ScanPlan &P, int *const d_out[6], ScanBufs &B,
+                       cudaStream_t main_stream) {
+    if (P.nshort == 0 || P.multi) return PSB_OK;
+    Ctx &c = g_ctx;
+    Sw16Params p = sw16_base_params(sp, open, gap, db, d_out, B);
+    const void *fn = sw16_fn(sp.K);
+    if (!fn) { set_error("sw16: no kernel for this query length"); return PSB_EUNSUPPORTED; }
+    // the head's CTAs request enough shared memory to be alone on their SMs
+    const size_t smem_excl = std::max<size_t>(sw16_smem_bytes(sp.nletters, sp.K, 4), 150 * 1024);
+    Sw16Shape s;
+    PSB_TRY(sw16_cta_shape(fn, sp, false, smem_excl, &s));
+    if (std::getenv("PSB_DEBUG_TIMING")) std::fprintf(stderr, "[psb] sw16: K %d, %d warps per CTA, %d CTAs per SM, %zu B shared\n", sp.K, s.wpb, s.per_sm, s.smem);
+    if (P.nhead > 0) {
+        // head: the longest subjects, 4 warps per CTA (one per sub-partition), each CTA alone on
+        // its SM (the shared-memory request keeps the main launch's CTAs away)
+        Sw16Params h = p;
+        sw16_subjects(h, db, P.nroute, P.nhead);
+        h.counter = B.cnt.as<int>() + 2;
+        const long long hslots = (P.nhead / 2 + 1) / 2;
+        void *hargs[] = {&h};
+        PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)((hslots + 3) / 4)), dim3(4 * 32), hargs, smem_excl, c.stream));
+        c.launches++;
+    }
+    const int64_t nrest = P.nshort - P.nhead;
+    if (nrest > 0) {
+        sw16_subjects(p, db, P.nroute + P.nhead, nrest);
+        p.counter = B.cnt.as<int>() + 1;
+        const long long slots = ((nrest + 1) / 2 + 1) / 2;  // a warp takes two items (four subjects) at a time
+        PSB_CUDA(launch_persistent(fn, &p, slots, s.wpb, s.smem, s.per_sm, c.sms, main_stream));
+        c.launches++;
+    }
+    return PSB_OK;
+}
+
+// re-run list: launched unconditionally with its length read on the device (usually zero), so the
+// scan needs no host round trip in the middle; the count reaches the host with the results
+static int launch_rerun(const FnConfig &cfg, const parasail_profile *prof, DevProfile *dp, int open, int gap, psb_db *db, const ScanPlan &P,
+                        int *const d_out[6], ScanBufs &B, int64_t *n_retried, int *retried_host) {
+    PSB_TRY(scan_general(cfg, prof, dp, open, gap, db, B.retry.as<int>(), (int)db->n, B.cnt.as<int>(), d_out));
+    PSB_CUDA(cudaMemcpyAsync(retried_host, B.cnt.p, sizeof(int), cudaMemcpyDeviceToHost, g_ctx.stream));
+    *n_retried = P.nroute;   // + *retried_host once the stream has been synchronised
+    return PSB_OK;
+}
+
+static int scan_sw16(const FnConfig &cfg, const parasail_profile *prof, DevProfile *dp, const std::vector<Sw16Profile> &strips, int open, int gap, psb_db *db,
+                     int *const d_out[6], int64_t *n_retried, int *retried_host) {
+    Ctx &c = g_ctx;
+    const ScanPlan P = plan_scan(strips, (int)prof->query.size(), db);
+    if (P.general) {
         // more over-long subjects than the routed head covers: not a workload for the packed kernel
         *n_retried = db->n;
         return scan_general(cfg, prof, dp, open, gap, db, nullptr, 0, nullptr, d_out);
     }
-    if (std::getenv("PSB_DEBUG_TIMING"))
-        std::fprintf(stderr, "[psb] sw16: n %lld residues %lld est %.2f ms long_len %.0f nroute %lld nhead %lld top %d\n", (long long)db->n,
-                     (long long)db->residues, est_ms, long_len, (long long)nroute, (long long)nhead, db->top_len.empty() ? 0 : db->top_len[0]);
-    DevMem d_retry, d_cnt;
-    PSB_TRY(d_retry.alloc(((size_t)db->n * strips.size() + 2) * sizeof(int), c.stream));
-    PSB_TRY(d_cnt.alloc(4 * sizeof(int), c.stream));
-    PSB_CUDA(cudaMemsetAsync(d_cnt.p, 0, 4 * sizeof(int), c.stream));
-
+    ScanBufs B;
+    PSB_TRY(B.retry.alloc(((size_t)db->n * strips.size() + 2) * sizeof(int), c.stream));
+    PSB_TRY(B.cnt.alloc(4 * sizeof(int), c.stream));
+    PSB_CUDA(cudaMemsetAsync(B.cnt.p, 0, 4 * sizeof(int), c.stream));
     // The launches that must own their SMs (wavefront strips, head) go on the compute stream, where
     // they start the moment the preceding work ends; the main launch goes on the side stream behind an
     // event, so it reaches the SMs after them.  The other way round, a busy queue lets the main
     // launch's persistent CTAs take every SM first and the head then runs alone AFTER it.
-    const bool forked = nroute > 0 || nhead > 0;
+    const bool forked = P.nroute > 0 || P.nhead > 0;
     if (forked) {
         PSB_CUDA(cudaEventRecord(c.ev_fork, c.stream));
         PSB_CUDA(cudaStreamWaitEvent(c.side, c.ev_fork, 0));
     }
-    DevMem d_lbytes, d_loff, d_bnd, d_ctl, d_cand;
-    if (nroute > 0) {
-        std::vector<long long> loff(nroute + 1);
-        loff[0] = 0;
-        for (int64_t i = 0; i < nroute; ++i) loff[i + 1] = loff[i] + db->top_len[i];
-        const int K = lq <= 64 ? 1 : 2;
-        const int nstrips = (lq + 32 * K - 1) / (32 * K);
-        PSB_TRY(d_lbytes.alloc((size_t)loff[nroute], c.stream));
-        PSB_TRY(d_loff.alloc((size_t)(nroute + 1) * sizeof(long long), c.stream));
-        PSB_TRY(d_bnd.alloc((size_t)nstrips * 2 * (size_t)loff[nroute] * sizeof(int), c.stream));
-        PSB_TRY(d_ctl.alloc(((size_t)nroute * nstrips + 2) * sizeof(int), c.stream));
-        PSB_TRY(d_cand.alloc((size_t)nroute * nstrips * 8 * sizeof(int), c.stream));
-        PSB_CUDA(cudaMemcpyAsync(d_loff.p, loff.data(), (size_t)(nroute + 1) * sizeof(long long), cudaMemcpyHostToDevice, c.stream));
-        PSB_CUDA(cudaMemsetAsync(d_ctl.p, 0, ((size_t)nroute * nstrips + 2) * sizeof(int), c.stream));
-        PSB_CUDA(cudaStreamSynchronize(c.stream));  // `loff` is a host temporary
-        UnpackParams u;
-        u.words = db->d_words; u.word_off = db->d_word_off; u.ids = nullptr; u.inv_perm = nullptr; u.out_off = d_loff.as<long long>();
-        u.out = d_lbytes.as<uint8_t>(); u.n = nroute; u.bits = db->bits;
-        unpack_db_kernel<<<(unsigned)std::min<int64_t>(nroute, 1024), 256, 0, c.stream>>>(u);
-        Wave32Params w;
-        std::memset(&w, 0, sizeof(w));
-        w.q = dp->d_query; w.r = d_lbytes.as<uint8_t>(); w.Lq = lq; w.Lr = 0;
-        w.matrix = dp->d_matrix; w.size = m.size; w.open = open; w.gap = gap;
-        w.mode = cfg.mode; w.s1_beg = cfg.s1_beg; w.s1_end = cfg.s1_end; w.s2_beg = cfg.s2_beg; w.s2_end = cfg.s2_end;
-        w.bnd = d_bnd.as<int>(); w.next_strip = d_ctl.as<int>(); w.progress = d_ctl.as<int>() + 1; w.cand = d_cand.as<int>();
-        w.multi_n = (int)nroute; w.r_off = d_loff.as<long long>();
-        const bool v2 = wave32_v2_ok(m, open, gap);
-        const void *fn = wave32_fn(K, v2);
-        // Full-size CTAs that also reserve most of an SM's shared memory: the strips of the long
-        // subjects then own a few SMs outright instead of crawling beside sixteen ALU-bound warps
-        // of the main kernel on every SM (each of their steps is a serial dependency).  The main
-        // kernel's blocks that find no room start on those SMs as soon as the strips are done.
-        const int kRouteWarps = v2 ? 8 : 32;   // generation 2 keeps a 12 KB profile per warp
-        const size_t smem = std::max<size_t>(v2 ? wave32v2_smem_bytes(m.size, kRouteWarps) : wave32_smem_bytes(m.size, kRouteWarps), 160 * 1024);
-        PSB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        // all warps of this launch must be resident together (strips wait on one another): one CTA
-        // per SM at most, issued before the main kernel so that its blocks are placed first
-        const long long items = nroute * nstrips;
-        long long blocks = std::min<long long>((items + kRouteWarps - 1) / kRouteWarps, (long long)c.sms);
-        void *args[] = {&w};
-        PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(kRouteWarps * 32), args, smem, c.stream));
-        WaveReduceParams r;
-        std::memset(&r, 0, sizeof(r));
-        r.cand = d_cand.as<int>(); r.nstrips = nstrips; r.mode = cfg.mode; r.s1_end = cfg.s1_end; r.s2_end = cfg.s2_end;
-        r.score = d_out[0]; r.end_query = d_out[1]; r.end_ref = d_out[2];
-        r.multi_n = (int)nroute; r.r_off = d_loff.as<long long>(); r.out_map = db->d_perm; r.first_id = 0;
-        wave32_reduce_kernel<<<(unsigned)((nroute + 127) / 128), 128, 0, c.stream>>>(r);
-        c.launches += 3;
-    }
-    const int64_t nshort = db->n - nroute;
-    DevMem d_bndA, d_bndB, d_scan_tmp16;
-    if (nshort > 0 && multi) {
-        // ---- queries of several strips: one sweep of the database per strip; the bottom row of a strip (T and
-        // Fh of both subjects of a word, one uint2 per column) goes through HBM to the strip below: 16 bytes
-        // per column and strip boundary against ~K*16*2.5 instructions of fill per column ------------------
-        if (!db->d_res_off) {
-            std::lock_guard<std::mutex> lk(db->mu);
-            if (!db->d_res_off) {
-                long long *ro = nullptr;
-                PSB_CUDA(cudaMallocAsync(&ro, ((size_t)db->n + 1) * sizeof(long long), db->stream));
-                if (db->stream != c.stream) PSB_CUDA(cudaStreamSynchronize(db->stream));
-                size_t tb = 0;
-                PSB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb, db->d_len, ro, (int)db->n, c.stream));
-                PSB_TRY(d_scan_tmp16.alloc(tb, c.stream));
-                PSB_CUDA(cub::DeviceScan::ExclusiveSum(d_scan_tmp16.p, tb, db->d_len, ro, (int)db->n, c.stream));
-                PSB_CUDA(cudaStreamSynchronize(c.stream));
-                db->d_res_off = ro;
-            }
-        }
-        PSB_TRY(d_bndA.alloc(((size_t)db->residues + 64) * sizeof(uint2), c.stream));
-        PSB_TRY(d_bndB.alloc(((size_t)db->residues + 64) * sizeof(uint2), c.stream));
-        for (size_t st = 0; st < strips.size(); ++st) {
-            const Sw16Profile &ss = strips[st];
-            Sw16Params p;
-            std::memset(&p, 0, sizeof(p));
-            p.prof = ss.prof; p.nletters = ss.nletters; p.lq = ss.lq; p.open = open; p.gap = gap; p.max_score = ss.max_score;
-            p.words = db->d_words; p.bits = db->bits;
-            p.score = d_out[0]; p.end_query = d_out[1]; p.end_ref = d_out[2];
-            p.retry = d_retry.as<int>(); p.retry_count = d_cnt.as<int>();
-            p.mul_one = 1u; p.mul_64k = 65536u;
-            p.word_off = db->d_word_off + nroute; p.len = db->d_len + nroute; p.n = nshort; p.out_map = db->d_perm + nroute;
-            p.sid_base = (int)nroute;
-            p.res_off = db->d_res_off + nroute;
-            p.bnd_in = st == 0 ? nullptr : ((st & 1) ? d_bndA.as<uint2>() : d_bndB.as<uint2>());
-            p.bnd_out = st + 1 == strips.size() ? nullptr : ((st & 1) ? d_bndB.as<uint2>() : d_bndA.as<uint2>());
-            p.row0 = ss.row0; p.merge = st > 0 ? 1 : 0;
-            DevMem d_cnt_st;   // a work counter per launch
-            PSB_TRY(d_cnt_st.alloc(sizeof(int), c.stream));
-            PSB_CUDA(cudaMemsetAsync(d_cnt_st.p, 0, sizeof(int), c.stream));
-            p.counter = d_cnt_st.as<int>();
-            const void *fn = sw16_fn(ss.K, true);
-            if (!fn) { set_error("sw16: no strip kernel for this query length"); return PSB_EUNSUPPORTED; }
-            int wpb = kSw16WarpsPerBlock, per_sm = 0;
-            size_t smem = sw16_smem_bytes(ss.nletters, ss.K, wpb, true);
-            const size_t smem16 = sw16_smem_bytes(ss.nletters, ss.K, 16, true);
-            PSB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(smem, smem16)));
-            PSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, wpb * 32, smem));
-            if (per_sm * wpb < 16) {
-                int per_sm16 = 0;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm16, fn, 16 * 32, smem16) == cudaSuccess && per_sm16 * 16 > per_sm * wpb) {
-                    wpb = 16; per_sm = per_sm16; smem = smem16;
-                } else cudaGetLastError();
-            }
-            if (per_sm < 1) per_sm = 1;
-            const long long slots = ((nshort + 1) / 2 + 1) / 2;
-            long long blocks = std::min<long long>((slots + wpb - 1) / wpb, (long long)c.sms * per_sm);
-            if (blocks < 1) blocks = 1;
-            void *args[] = {&p};
-            PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(wpb * 32), args, smem, c.stream));
-            c.launches++;
-        }
-    } else if (nshort > 0) {
-        Sw16Params p;
-        std::memset(&p, 0, sizeof(p));
-        p.prof = sp.prof; p.nletters = sp.nletters; p.lq = sp.lq; p.open = open; p.gap = gap; p.max_score = sp.max_score;
-        p.words = db->d_words; p.bits = db->bits;
-        p.score = d_out[0]; p.end_query = d_out[1]; p.end_ref = d_out[2];
-        p.retry = d_retry.as<int>(); p.retry_count = d_cnt.as<int>();
-        p.mul_one = 1u; p.mul_64k = 65536u;
-        const void *fn = sw16_fn(sp.K);
-        if (!fn) { set_error("sw16: no kernel for this query length"); return PSB_EUNSUPPORTED; }
-        // CTA size: two CTAs of 8 warps when their profile copies fit an SM together, else one of 16
-        // (long queries with a protein alphabet: one 50 KB profile copy instead of two)
-        int wpb = kSw16WarpsPerBlock, per_sm = 0;
-        size_t smem = sw16_smem_bytes(sp.nletters, sp.K, wpb);
-        const size_t smem_excl = std::max<size_t>(sw16_smem_bytes(sp.nletters, sp.K, 4), 150 * 1024);
-        const size_t smem16 = sw16_smem_bytes(sp.nletters, sp.K, 16);
-        PSB_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max(std::max(smem, smem_excl), smem16)));
-        PSB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, wpb * 32, smem));
-        if (per_sm * wpb < 16) {
-            int per_sm16 = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm16, fn, 16 * 32, smem16) == cudaSuccess && per_sm16 * 16 > per_sm * wpb) {
-                wpb = 16; per_sm = per_sm16; smem = smem16;
-            } else {
-                cudaGetLastError();
-            }
-        }
-        if (per_sm < 1) per_sm = 1;
-        if (std::getenv("PSB_DEBUG_TIMING")) std::fprintf(stderr, "[psb] sw16: K %d, %d warps per CTA, %d CTAs per SM, %zu B shared\n", sp.K, wpb, per_sm, smem);
-        if (nhead > 0) {
-            // head: the longest subjects, 4 warps per CTA (one per sub-partition), each CTA alone on
-            // its SM (the shared-memory request keeps the main launch's CTAs away)
-            Sw16Params h = p;
-            h.word_off = db->d_word_off + nroute; h.len = db->d_len + nroute; h.n = nhead; h.out_map = db->d_perm + nroute;
-            h.sid_base = (int)nroute; h.counter = d_cnt.as<int>() + 2;
-            const long long hslots = (nhead / 2 + 1) / 2;
-            void *hargs[] = {&h};
-            PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)((hslots + 3) / 4)), dim3(4 * 32), hargs, smem_excl, c.stream));
-            c.launches++;
-        }
-        const int64_t nrest = nshort - nhead;
-        if (nrest > 0) {
-            p.word_off = db->d_word_off + nroute + nhead; p.len = db->d_len + nroute + nhead; p.n = nrest;
-            p.out_map = db->d_perm + nroute + nhead; p.sid_base = (int)(nroute + nhead); p.counter = d_cnt.as<int>() + 1;
-            const long long slots = ((nrest + 1) / 2 + 1) / 2;  // a warp takes two items (four subjects) at a time
-            long long blocks = std::min<long long>((slots + wpb - 1) / wpb, (long long)c.sms * per_sm);
-            if (blocks < 1) blocks = 1;
-            void *args[] = {&p};
-            PSB_CUDA(cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(wpb * 32), args, smem, forked ? c.side : c.stream));
-            c.launches++;
-        }
-    }
+    PSB_TRY(launch_route(cfg, prof, dp, open, gap, db, P, d_out, B));
+    PSB_TRY(launch_sw16_strips(strips, open, gap, db, P, d_out, B));
+    PSB_TRY(launch_sw16(strips[0], open, gap, db, P, d_out, B, forked ? c.side : c.stream));
     if (forked) {
         PSB_CUDA(cudaEventRecord(c.ev_join, c.side));
         PSB_CUDA(cudaStreamWaitEvent(c.stream, c.ev_join, 0));
     }
-    // re-run list: launched unconditionally with its length read on the device (usually zero), so the
-    // scan needs no host round trip in the middle; the count reaches the host with the results
-    PSB_TRY(scan_general(cfg, prof, dp, open, gap, db, d_retry.as<int>(), (int)db->n, d_cnt.as<int>(), d_out));
-    PSB_CUDA(cudaMemcpyAsync(retried_host, d_cnt.p, sizeof(int), cudaMemcpyDeviceToHost, c.stream));
-    *n_retried = nroute;   // + *retried_host once the stream has been synchronised
-    return PSB_OK;
+    return launch_rerun(cfg, prof, dp, open, gap, db, P, d_out, B, n_retried, retried_host);
 }
 
 }  // namespace psb
@@ -1976,16 +2029,9 @@ static int align_pairs(const FnConfig &cfg, const HostMatrix &hm, int open, int 
     req.cfg = cfg; req.matrix = &hm; req.open = open; req.gap = gap;
     req.q_cat = q_cat; req.q_off = q_off; req.r_cat = r_cat; req.r_off = r_off; req.n = n;
     const int rc = run_pairs(req, out);
-    if (rc == PSB_OK && (cfg.width == 8 || cfg.width == 16)) {
-        psb_batch_t *b = *out;
-        const bool pssm = hm.type == PARASAIL_MATRIX_TYPE_PSSM;
-        for (int64_t i = 0; i < n; ++i) {
-            const int lq = pssm ? hm.length : (int)(q_off[i + 1] - q_off[i]), lr = (int)(r_off[i + 1] - r_off[i]);
-            if (saturates(cfg, hm, b->score[i], lq, lr, open, gap)) {
-                b->saturated[i] = 1; b->score[i] = 0; b->end_query[i] = 0; b->end_ref[i] = 0;
-            }
-        }
-    }
+    const bool pssm = hm.type == PARASAIL_MATRIX_TYPE_PSSM;
+    if (rc == PSB_OK)
+        flag_saturated(cfg, hm, open, gap, *out, [&](int64_t i) { return std::make_pair(pssm ? hm.length : span(q_off, i), span(r_off, i)); });
     return rc;
 }
 }  // namespace psb
@@ -2237,30 +2283,48 @@ static psb_db *db_begin(DbBuild &B, const uint8_t *cat, const int64_t *off, int6
     return B.db;
 }
 
-// PSB_DEBUG_TIMING: extra marks on the compute stream (psb_scan_host's device timeline)
-static thread_local std::vector<cudaEvent_t> *g_dbg_marks = nullptr;
-static void dbg_mark_stream(cudaStream_t st) {
-    if (!g_dbg_marks) return;
-    cudaEvent_t e;
-    if (cudaEventCreate(&e) == cudaSuccess) { cudaEventRecord(e, st); g_dbg_marks->push_back(e); }
-}
+// PSB_DEBUG_TIMING on psb_scan_host (inert without it): a device-side timeline, one event per mark on the stream
+// named, reported relative to the first mark
+struct StreamMarks {
+    const bool on = std::getenv("PSB_DEBUG_TIMING") != nullptr;
+    std::vector<cudaEvent_t> ev;
+    StreamMarks() = default;
+    StreamMarks(const StreamMarks &) = delete;
+    StreamMarks &operator=(const StreamMarks &) = delete;
+    ~StreamMarks() { for (cudaEvent_t e : ev) cudaEventDestroy(e); }
+    void mark(cudaStream_t st) {
+        cudaEvent_t e;
+        if (on && cudaEventCreate(&e) == cudaSuccess) { cudaEventRecord(e, st); ev.push_back(e); }
+    }
+    std::string line() const {
+        std::string out;
+        for (size_t i = 1; i < ev.size(); ++i) {
+            float ms = 0.f;
+            cudaEventElapsedTime(&ms, ev[0], ev[i]);
+            char buf[32]; std::snprintf(buf, sizeof buf, " %.3f", ms); out += buf;
+        }
+        return out;
+    }
+};
 
-static int db_finish(DbBuild &B) {
+// `marks`: psb_scan_host's timeline (lengths< >lengths sort> <pack pack>), or nullptr
+static int db_finish(DbBuild &B, StreamMarks *marks = nullptr) {
     Ctx &c = g_ctx;
     psb_db *db = B.db;
     const int64_t n = db->n;
     const size_t n1 = (size_t)n + 1;
     const int rpw = db_residues_per_word(db->bits);
+    auto mark = [&] { if (marks) marks->mark(c.stream); };
     if (B.offs_up) PSB_CUDA(cudaStreamWaitEvent(c.stream, B.offs_up, 0));
-    dbg_mark_stream(c.stream);
+    mark();
     db_lengths_kernel<<<c.sms * 4, 256, 0, c.stream>>>(B.offs(), n, B.d_len0.as<int>(), B.d_idx0.as<int>());
-    dbg_mark_stream(c.stream);
+    mark();
     size_t tb = 0, tb2 = 0;
     PSB_CUDA(cub::DeviceRadixSort::SortPairsDescending(nullptr, tb, B.d_len0.as<int>(), db->d_len, B.d_idx0.as<int>(), db->d_perm, (int)n, 0, 32, c.stream));
     PSB_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, tb2, B.d_wcount.as<long long>(), db->d_word_off, (int)n1, c.stream));
     PSB_TRY(B.d_tmp.alloc(std::max(tb, tb2), c.stream));
     PSB_CUDA(cub::DeviceRadixSort::SortPairsDescending(B.d_tmp.p, tb, B.d_len0.as<int>(), db->d_len, B.d_idx0.as<int>(), db->d_perm, (int)n, 0, 32, c.stream));
-    dbg_mark_stream(c.stream);
+    mark();
     db_wcount_sorted_kernel<<<c.sms * 4, 256, 0, c.stream>>>(db->d_len, n, rpw, B.d_wcount.as<long long>());
     PSB_CUDA(cub::DeviceScan::ExclusiveSum(B.d_tmp.p, tb2, B.d_wcount.as<long long>(), db->d_word_off, (int)n1, c.stream));
     PackParams pp;
@@ -2268,13 +2332,13 @@ static int db_finish(DbBuild &B) {
     pp.word_off = db->d_word_off; pp.words = db->d_words; pp.n = n; pp.bits = db->bits;
     std::memcpy(pp.lut, B.lut, sizeof(pp.lut));
     if (B.uploaded) PSB_CUDA(cudaStreamWaitEvent(c.stream, B.uploaded, 0));
-    dbg_mark_stream(c.stream);
+    mark();
     pack_db_kernel<<<c.sms * 8, 256, 256, c.stream>>>(pp);
     if (B.uploaded) {
         PSB_CUDA(cudaEventCreateWithFlags(&B.packed, cudaEventDisableTiming));
         PSB_CUDA(cudaEventRecord(B.packed, c.stream));
     }
-    dbg_mark_stream(c.stream);
+    mark();
     c.launches += 5;
     PSB_CUDA(cudaGetLastError());
     // no synchronisation: later work on this stream is ordered after the packing kernel, and the
@@ -2356,6 +2420,8 @@ struct ScanJob {
         if (done) cudaEventDestroy(done);
     }
 };
+// the packed 16-bit scan serves this function (if its profile can be packed): local score-only at 8/16 bit or "sat"
+static bool sw16_wanted(const FnConfig &cfg) { return cfg.mode == MODE_SW && !cfg.stats && cfg.width != 32 && cfg.width != 64; }
 static int scan_enqueue(ScanJob &job, const FnConfig &cfg, const parasail_profile *profile, int open, int gap, psb_db *db,
                         int *const hosts[6], int64_t host_base) {
     Ctx &c = g_ctx;
@@ -2371,7 +2437,7 @@ static int scan_enqueue(ScanJob &job, const FnConfig &cfg, const parasail_profil
     PSB_CUDA(cudaEventCreate(&job.ev1));
     PSB_CUDA(cudaEventRecord(job.ev0, c.stream));
     std::vector<Sw16Profile> sp16;
-    const bool fast = cfg.mode == MODE_SW && !cfg.stats && cfg.width != 32 && cfg.width != 64 && sw16_prepare(profile, dp, open, gap, &sp16);
+    const bool fast = sw16_wanted(cfg) && sw16_prepare(profile, dp, open, gap, &sp16);
     int rc;
     if (fast && sp16.size() == 1 && db->nlong == 0) { job.rate_k = sp16[0].K; job.rate_cells = (double)profile->query.size() * (double)db->residues; }
     if (fast) rc = scan_sw16(cfg, profile, dp, sp16, open, gap, db, outp, &job.retried, job.retried_host);
@@ -2398,10 +2464,26 @@ static int scan_finish(ScanJob &job) {
     job.retried += *job.retried_host;
     return PSB_OK;
 }
-static int scan_check(const char *who, const char *fn_name, const parasail_profile_t *profile, FnConfig *cfg) {
+// what every entry point that runs a profile against a database checks first: a profile function name and a profile
+static int profile_fn_check(const char *who, const char *fn_name, const parasail_profile_t *profile, FnConfig *cfg) {
     if (!parse_fn_name(fn_name, cfg) || !cfg->profile) { set_error(std::string(who) + ": not a profile function name: " + (fn_name ? fn_name : "(null)")); return PSB_EINVAL; }
     if (!profile) { set_error(std::string(who) + ": NULL profile"); return PSB_EINVAL; }
+    return PSB_OK;
+}
+// and a scan, which produces no traceback
+static int scan_check(const char *who, const char *fn_name, const parasail_profile_t *profile, FnConfig *cfg) {
+    PSB_TRY(profile_fn_check(who, fn_name, profile, cfg));
     if (cfg->trace || cfg->table || cfg->rowcol) { set_error(std::string(who) + ": trace/table/rowcol outputs are not available for database scans"); return PSB_EUNSUPPORTED; }
+    return PSB_OK;
+}
+// a profile run against a resident database: the calling thread's device holds it, and both use the same alphabet
+static int profile_db_check(const char *who, const parasail_profile_t *profile, const psb_db *db) {
+    PSB_TRY(ensure_ctx());
+    if (db->device != g_ctx.device) { set_error(std::string(who) + ": database lives on another device"); return PSB_EINVAL; }
+    if (profile->matrix.size != db->msize || std::memcmp(profile->matrix.mapper, db->mapper, 256) != 0) {
+        set_error(std::string(who) + ": profile and database were built with different alphabets");
+        return PSB_EINVAL;
+    }
     return PSB_OK;
 }
 // what every call that reads a resident database's subjects by caller id checks: the calling thread's device holds it
@@ -2443,28 +2525,20 @@ int psb_scan(const char *fn_name, const parasail_profile_t *profile, int open, i
     PSB_TRY(scan_check("psb_scan", fn_name, profile, &cfg));
     if (!db_c || !out) { set_error("psb_scan: NULL argument"); return PSB_EINVAL; }
     psb_db *db = const_cast<psb_db *>(db_c);
-    PSB_TRY(ensure_ctx());
+    PSB_TRY(profile_db_check("psb_scan", profile, db));
     Ctx &c = g_ctx;
-    if (db->device != c.device) { set_error("psb_scan: database lives on another device"); return PSB_EINVAL; }
-    if (profile->matrix.size != db->msize || std::memcmp(profile->matrix.mapper, db->mapper, 256) != 0) {
-        set_error("psb_scan: profile and database were built with different alphabets");
-        return PSB_EINVAL;
-    }
     c.last_ms = 0.0; c.launches = 0;
     psb_batch_t *b = new_batch(db->n, cfg);
     if (!b) { set_error("pinned host allocation failed"); return PSB_ENOMEM; }
     b->cells = (double)profile->query.size() * (double)db->residues;
-    int *hosts[6] = {b->score, b->end_query, b->end_ref, b->matches, b->similar, b->length};
     ScanJob job;
-    int rc = scan_enqueue(job, cfg, profile, open, gap, db, hosts, 0);
+    int rc = scan_enqueue(job, cfg, profile, open, gap, db, batch_outputs(b).data(), 0);
     if (rc == PSB_OK) rc = scan_finish(job);
     if (rc != PSB_OK) { cudaStreamSynchronize(c.stream); free_batch(b); return rc; }
     b->n_retried = job.retried;
-    if (cfg.width == 8 || cfg.width == 16)
-        for (int64_t i = 0; i < db->n; ++i)
-            if (saturates(cfg, profile->matrix, b->score[i], (int)profile->query.size(), db->host_len.empty() ? db->maxlen : db->host_len[(size_t)i], open, gap)) {
-                b->saturated[i] = 1; b->score[i] = 0; b->end_query[i] = 0; b->end_ref[i] = 0;
-            }
+    const int lq = (int)profile->query.size();
+    flag_saturated(cfg, profile->matrix, open, gap, b,
+                   [&](int64_t i) { return std::make_pair(lq, db->host_len.empty() ? db->maxlen : db->host_len[(size_t)i]); });
     *out = b;
     return PSB_OK;
 }
@@ -2473,16 +2547,12 @@ int psb_db_align(const char *fn_name, const parasail_profile_t *profile, int ope
                  const int64_t *ids, int64_t n, psb_batch_t **out) {
     if (out) *out = nullptr;
     FnConfig cfg;
-    if (!parse_fn_name(fn_name, &cfg) || !cfg.profile) { set_error(std::string("psb_db_align: not a profile function name: ") + (fn_name ? fn_name : "(null)")); return PSB_EINVAL; }
-    if (!profile) { set_error("psb_db_align: NULL profile"); return PSB_EINVAL; }
+    PSB_TRY(profile_fn_check("psb_db_align", fn_name, profile, &cfg));
     if (cfg.table || cfg.rowcol) { set_error("psb_db_align: _table/_rowcol outputs exist only on the single-pair API"); return PSB_EUNSUPPORTED; }
     if (!db_c || !out) { set_error("psb_db_align: NULL argument"); return PSB_EINVAL; }
     psb_db *db = const_cast<psb_db *>(db_c);
     PSB_TRY(db_check("psb_db_align", db));
-    if (profile->matrix.size != db->msize || std::memcmp(profile->matrix.mapper, db->mapper, 256) != 0) {
-        set_error("psb_db_align: profile and database were built with different alphabets");
-        return PSB_EINVAL;
-    }
+    PSB_TRY(profile_db_check("psb_db_align", profile, db));
     if (n <= 0 || (!ids && n != db->n)) {
         set_error("psb_db_align: " + std::to_string(n) + " ids for a database of " + std::to_string(db->n) + " subjects");
         return PSB_EINVAL;
@@ -2511,13 +2581,7 @@ int psb_db_align(const char *fn_name, const parasail_profile_t *profile, int ope
     req.r_off = r_off.data(); req.n = n; req.r_db = db; req.r_ids = rid.data();
     const int rc = run_pairs(req, out);
     g_ctx.launches += first_use;
-    if (rc == PSB_OK && (cfg.width == 8 || cfg.width == 16)) {
-        psb_batch_t *b = *out;
-        for (int64_t i = 0; i < n; ++i)
-            if (saturates(cfg, profile->matrix, b->score[i], (int)lq, (int)(r_off[(size_t)i + 1] - r_off[(size_t)i]), open, gap)) {
-                b->saturated[i] = 1; b->score[i] = 0; b->end_query[i] = 0; b->end_ref[i] = 0;
-            }
-    }
+    if (rc == PSB_OK) flag_saturated(cfg, profile->matrix, open, gap, *out, [&](int64_t i) { return std::make_pair((int)lq, span(r_off.data(), i)); });
     return rc;
 }
 
@@ -2625,22 +2689,25 @@ struct ScanLeftovers {
         jobs.clear(); builds.clear();
     }
 };
-static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap, const uint8_t *cat,
-                          const int64_t *off, int64_t n, int *const hosts[6], int64_t base, int64_t *n_retried,
-                          ScanLeftovers *leftovers = nullptr) {
-    Ctx &c = g_ctx;
-    const HostMatrix &hm = profile->matrix;
-    // pieces: the upload of piece k+1 (copy stream) runs under the scan of piece k, and nothing on the host waits
-    // for the GPU until the last piece is queued.  The sizes follow from two measured rates (HostScanRates): with
-    // u = upload time and v = scan time per residue, piece k+1 may be r = 0.85 v/u times piece k and still land
-    // before piece k has been scanned; the first piece and the number of pieces minimise
-    // (upload of the first piece) + (pieces - 1) x (cost of a piece boundary).  plan_pieces() below.
+// The pieces of a host scan: the upload of piece k+1 (copy stream) runs under the scan of piece k, and nothing on the
+// host waits for the GPU until the last piece is queued.  The sizes follow from two measured rates (HostScanRates): with
+// u = upload time and v = scan time per residue, piece k+1 may be r = 0.85 v/u times piece k and still land before
+// piece k has been scanned; the first piece and the number of pieces minimise
+// (upload of the first piece) + (pieces - 1) x (cost of a piece boundary).  plan_pieces() above.
+struct PiecePlan {
+    uint64_t rate_key = 0;              // host_scan_key of the scan
+    double u_rate = 0, v_rate = 0;      // upload and scan ms per residue the sizes were planned with
+    std::vector<int64_t> cut;           // piece k is subjects cut[k] .. cut[k + 1] - 1
+};
+static PiecePlan plan_host_pieces(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap, const int64_t *off, int64_t n) {
+    PiecePlan pl;
     const int64_t total = off[n] - off[0];
-    const uint64_t rate_key = host_scan_key(cfg, (int)profile->query.size(), open, gap, hm.size);
-    const double u_rate = g_hs.h2d_ms_per_byte > 0 ? g_hs.h2d_ms_per_byte : 1e3 / 50e9;
-    const bool packed_path = cfg.mode == MODE_SW && !cfg.stats && cfg.width != 32 && cfg.width != 64;
-    const double v_rate = (g_hs.key == rate_key && g_hs.scan_ms_per_byte > 0) ? g_hs.scan_ms_per_byte
-                                                                                : (double)profile->query.size() * 1e3 / (packed_path ? 4.9e12 : 1.5e12);
+    pl.rate_key = host_scan_key(cfg, (int)profile->query.size(), open, gap, profile->matrix.size);
+    const uint64_t rate_key = pl.rate_key;
+    const double u_rate = pl.u_rate = g_hs.h2d_ms_per_byte > 0 ? g_hs.h2d_ms_per_byte : 1e3 / 50e9;
+    const double v_rate = pl.v_rate = (g_hs.key == rate_key && g_hs.scan_ms_per_byte > 0)
+                                          ? g_hs.scan_ms_per_byte
+                                          : (double)profile->query.size() * 1e3 / (sw16_wanted(cfg) ? 4.9e12 : 1.5e12);
     std::vector<int64_t> sizes;
     const char *e_piece = std::getenv("PSB_SCAN_HOST_PIECE_MB"), *e_first = std::getenv("PSB_SCAN_HOST_FIRST_MB"), *e_div = std::getenv("PSB_SCAN_HOST_FIRST_DIV");
     if (e_piece || e_first || e_div) {
@@ -2667,18 +2734,29 @@ static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile
         if (last.total == total && last.key == rate_key && !last.sizes.empty() && exposed(last.sizes) <= 1.05 * exposed(sizes) + 0.05) sizes = last.sizes;
         last.total = total; last.key = rate_key; last.sizes = sizes;
     }
-    std::vector<int64_t> cut(1, 0);
-    {
-        int64_t acc = 0;
-        for (size_t k = 0; k + 1 < sizes.size() && cut.back() < n; ++k) {
-            acc += sizes[k];
-            int64_t at = std::lower_bound(off, off + n + 1, off[0] + acc) - off;
-            if (at <= cut.back()) at = cut.back() + 1;
-            if (at >= n) break;
-            cut.push_back(at);
-        }
-        cut.push_back(n);
+    // cut on subject boundaries
+    std::vector<int64_t> &cut = pl.cut;
+    cut.assign(1, 0);
+    int64_t acc = 0;
+    for (size_t k = 0; k + 1 < sizes.size() && cut.back() < n; ++k) {
+        acc += sizes[k];
+        int64_t at = std::lower_bound(off, off + n + 1, off[0] + acc) - off;
+        if (at <= cut.back()) at = cut.back() + 1;
+        if (at >= n) break;
+        cut.push_back(at);
     }
+    cut.push_back(n);
+    return pl;
+}
+
+static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap, const uint8_t *cat,
+                          const int64_t *off, int64_t n, int *const hosts[6], int64_t base, int64_t *n_retried,
+                          ScanLeftovers *leftovers = nullptr) {
+    Ctx &c = g_ctx;
+    const HostMatrix &hm = profile->matrix;
+    const int64_t total = off[n] - off[0];
+    const PiecePlan pl = plan_host_pieces(cfg, profile, open, gap, off, n);
+    const std::vector<int64_t> &cut = pl.cut;
     const int npieces = (int)cut.size() - 1;
     const double ms_at_entry = c.last_ms;
     int rc = PSB_OK;
@@ -2717,15 +2795,14 @@ static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile
         std::string line;
         for (int k = 0; k < npieces; ++k) line += " " + std::to_string((off[cut[k + 1]] - off[cut[k]]) >> 20);
         std::fprintf(stderr, "[psb] scan_host(dev %d): pieces (MB):%s; upload %.1f GB/s, scan %.1f GB/s of residues\n", c.device, line.c_str(),
-                     1e-6 / u_rate, 1e-6 / v_rate);
+                     1e-6 / pl.u_rate, 1e-6 / pl.v_rate);
     }
     // order of the host's work: the copy engine comes first.  Upload k+1 is queued before any host time goes into
     // piece k (its offsets pass, the sort/pack launches, the scan launches), so the link never waits for the host.
     // PSB_DEBUG_TIMING: a device-side timeline (upload landed / packing begins / scan begins / scan ends / results
     // on the host), relative to an event recorded on the idle compute stream at entry
-    std::vector<cudaEvent_t> tl;
-    if (dbg) g_dbg_marks = &tl;
-    auto mark = [&](cudaStream_t st) { dbg_mark_stream(st); };
+    StreamMarks tl;
+    auto mark = [&](cudaStream_t st) { tl.mark(st); };
     mark(c.stream);
     rc = upload(0);
     mark(c.copy);
@@ -2735,7 +2812,7 @@ static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile
         DevProfile *dp0 = nullptr;
         rc = get_dev_profile(profile, &dp0);
         std::vector<Sw16Profile> sp0;
-        if (rc == PSB_OK && packed_path) sw16_prepare(profile, dp0, open, gap, &sp0);
+        if (rc == PSB_OK && sw16_wanted(cfg)) sw16_prepare(profile, dp0, open, gap, &sp0);
     }
     if (dbg) std::fprintf(stderr, "[psb] scan_host(dev %d): %d pieces, first upload queued at %.3f ms\n", c.device, npieces, since());
     auto next_upload = [&](int k) {
@@ -2752,7 +2829,7 @@ static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile
         rc = db_host_pass(*builds[k], off + cut[k]);
         const double h1 = dbg ? since() : 0.0;
         if (dbg) { cudaStreamWaitEvent(c.stream, builds[k]->offs_up, 0); mark(c.stream); }
-        if (rc == PSB_OK) rc = db_finish(*builds[k]);
+        if (rc == PSB_OK) rc = db_finish(*builds[k], &tl);
         if (dbg) std::fprintf(stderr, "[psb] scan_host(dev %d): piece %d host: offsets pass + allocations %.3f ms, chain launches %.3f ms\n", c.device, k, h1 - h0, since() - h1);
         mark(c.stream);
         // the next piece's upload is queued as soon as its gate (this piece's chain) exists, before host time
@@ -2777,24 +2854,14 @@ static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile
     }
     cudaStreamSynchronize(c.stream);
     if (dbg) std::fprintf(stderr, "[psb] scan_host(dev %d): all done at %.3f ms\n", c.device, since());
-    if (dbg && !tl.empty()) {
-        // order of the marks: entry | upload 0 | per piece k: [upload k+1] upload-k-landed (lengths< >lengths sort> <pack pack>) pack-end results-on-host
-        std::string line;
-        for (size_t i = 1; i < tl.size(); ++i) {
-            float ms = 0.f;
-            cudaEventElapsedTime(&ms, tl[0], tl[i]);
-            char buf[32]; std::snprintf(buf, sizeof buf, " %.3f", ms); line += buf;
-        }
-        std::fprintf(stderr, "[psb] scan_host(dev %d): device timeline (ms after entry):%s\n", c.device, line.c_str());
-        for (cudaEvent_t e : tl) cudaEventDestroy(e);
-    }
-    g_dbg_marks = nullptr;
+    // order of the marks: entry | upload 0 | per piece k: [upload k+1] upload-k-landed (lengths< >lengths sort> <pack pack>) pack-end results-on-host
+    if (dbg && !tl.ev.empty()) std::fprintf(stderr, "[psb] scan_host(dev %d): device timeline (ms after entry):%s\n", c.device, tl.line().c_str());
     // the results are on the host.  What is left is giving the last piece's device memory back: a caller with
     // somewhere better to do that (psb_scan_box's workers, after they have reported completion) takes it over
     if (rc == PSB_OK && total >= ((int64_t)8 << 20) && c.last_ms > ms_at_entry) {
         const double now = (c.last_ms - ms_at_entry) / (double)total;
-        g_hs.scan_ms_per_byte = g_hs.key == rate_key && g_hs.scan_ms_per_byte > 0 ? 0.5 * g_hs.scan_ms_per_byte + 0.5 * now : now;
-        g_hs.key = rate_key;
+        g_hs.scan_ms_per_byte = g_hs.key == pl.rate_key && g_hs.scan_ms_per_byte > 0 ? 0.5 * g_hs.scan_ms_per_byte + 0.5 * now : now;
+        g_hs.key = pl.rate_key;
     }
     if (leftovers && rc == PSB_OK) {
         if (builds[npieces - 1]) note_upload(*builds[npieces - 1]);
@@ -2806,14 +2873,6 @@ static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile
         if (rc == PSB_OK) rc = r;
     }
     return rc;
-}
-
-static void flag_saturated(const FnConfig &cfg, const HostMatrix &hm, int lq, const int64_t *off, int64_t n, int open, int gap, psb_batch_t *b) {
-    if (cfg.width != 8 && cfg.width != 16) return;
-    for (int64_t i = 0; i < n; ++i)
-        if (saturates(cfg, hm, b->score[i], lq, (int)(off[i + 1] - off[i]), open, gap)) {
-            b->saturated[i] = 1; b->score[i] = 0; b->end_query[i] = 0; b->end_ref[i] = 0;
-        }
 }
 
 // ---- one worker thread per device for psb_scan_box: the thread keeps its context (streams, memory pool,
@@ -2854,6 +2913,14 @@ struct BoxWorker {
         cv.wait(lk, [&] { return !has_job; });
     }
 };
+// a new resident worker thread bound to `device`; it lives as long as the process
+static BoxWorker *start_worker(int device) {
+    BoxWorker *w = new BoxWorker();
+    w->device = device;
+    w->th = std::thread([w] { w->loop(); });
+    w->th.detach();
+    return w;
+}
 // ---- lanes for the passes of a large psb_align_pairs batch ------------------------------------------------
 // Each lane is a resident host thread bound to the caller's device, with its own context (streams, events): the
 // passes are handed out in order, so that while one lane's pass is in its kernels the other lane uploads and
@@ -2863,13 +2930,7 @@ static std::map<std::pair<int, int>, BoxWorker *> g_lanes;   // (device, lane) -
 static BoxWorker *pair_lane(int device, int lane) {
     std::lock_guard<std::mutex> lk(g_lane_mu);
     BoxWorker *&w = g_lanes[{device, lane}];
-    if (!w) {
-        w = new BoxWorker();
-        w->device = device;
-        BoxWorker *ww = w;
-        w->th = std::thread([ww] { ww->loop(); });
-        w->th.detach();
-    }
+    if (!w) w = start_worker(device);
     return w;
 }
 static int run_pairs_lanes(const PairsRequest &req, PassCutter &cutter, const PairChunk &first, PassOut *first_out, psb_batch_t *b, int lanes) {
@@ -2918,13 +2979,7 @@ static std::vector<BoxWorker *> g_box;   // index = device; never destroyed (the
 static BoxWorker *box_worker(int device) {
     std::lock_guard<std::mutex> lk(g_box_mu);
     if ((int)g_box.size() <= device) g_box.resize(device + 1, nullptr);
-    if (!g_box[device]) {
-        BoxWorker *w = new BoxWorker();
-        w->device = device;
-        w->th = std::thread([w] { w->loop(); });
-        w->th.detach();
-        g_box[device] = w;
-    }
+    if (!g_box[device]) g_box[device] = start_worker(device);
     return g_box[device];
 }
 }  // namespace psb
@@ -2944,10 +2999,10 @@ int psb_scan_host(const char *fn_name, const parasail_profile_t *profile, int op
     psb_batch_t *b = new_batch(n, cfg);
     if (!b) { set_error("pinned host allocation failed"); return PSB_ENOMEM; }
     b->cells = (double)profile->query.size() * (double)(off[n] - off[0]);
-    int *hosts[6] = {b->score, b->end_query, b->end_ref, b->matches, b->similar, b->length};
-    const int rc = scan_host_into(cfg, profile, open, gap, cat, off, n, hosts, 0, &b->n_retried);
+    const int rc = scan_host_into(cfg, profile, open, gap, cat, off, n, batch_outputs(b).data(), 0, &b->n_retried);
     if (rc != PSB_OK) { free_batch(b); return rc; }
-    flag_saturated(cfg, profile->matrix, (int)profile->query.size(), off, n, open, gap, b);
+    const int lq = (int)profile->query.size();
+    flag_saturated(cfg, profile->matrix, open, gap, b, [&](int64_t i) { return std::make_pair(lq, span(off, i)); });
     *out = b;
     return PSB_OK;
 }
@@ -2983,7 +3038,7 @@ int psb_scan_box(const char *fn_name, const parasail_profile_t *profile, int ope
         cut[d] = std::lower_bound(off, off + n + 1, off[0] + total * d / n_gpus) - off;
         if (cut[d] <= cut[d - 1]) cut[d] = std::min<int64_t>(n, cut[d - 1] + 1);
     }
-    int *hosts[6] = {b->score, b->end_query, b->end_ref, b->matches, b->similar, b->length};
+    const std::array<int *, 6> hosts = batch_outputs(b);
     std::vector<int> rcs(n_gpus, PSB_OK), launches(n_gpus, 0);
     std::vector<int64_t> retried(n_gpus, 0);
     std::vector<double> ms(n_gpus, 0.0);
@@ -2995,7 +3050,7 @@ int psb_scan_box(const char *fn_name, const parasail_profile_t *profile, int ope
             int rc = ensure_ctx();
             if (rc == PSB_OK) {
                 g_ctx.last_ms = 0.0; g_ctx.launches = 0;
-                rc = scan_host_into(cfg, profile, open, gap, cat, off + cut[d], cut[d + 1] - cut[d], hosts, cut[d], &retried[d], &w->left);
+                rc = scan_host_into(cfg, profile, open, gap, cat, off + cut[d], cut[d + 1] - cut[d], hosts.data(), cut[d], &retried[d], &w->left);
                 ms[d] = g_ctx.last_ms; launches[d] = g_ctx.launches;
             }
             rcs[d] = rc;
@@ -3016,7 +3071,8 @@ int psb_scan_box(const char *fn_name, const parasail_profile_t *profile, int ope
         c.launches += launches[d];
     }
     if (rc != PSB_OK) { free_batch(b); return rc; }
-    flag_saturated(cfg, profile->matrix, (int)profile->query.size(), off, n, open, gap, b);
+    const int lq = (int)profile->query.size();
+    flag_saturated(cfg, profile->matrix, open, gap, b, [&](int64_t i) { return std::make_pair(lq, span(off, i)); });
     *out = b;
     return PSB_OK;
 }

@@ -71,20 +71,14 @@ int p16_launch(int cls, bool sw, bool trace, const Pairs16Params &p, int sms, cu
         wpb /= 2;
         smem = pairs16_smem_bytes(c.K, nletters, sw, wpb);
     }
-    cudaError_t e = cudaSuccess;
-    if (smem > 48 * 1024) e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     int per_sm = 0;
-    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, wpb * 32, smem);
+    cudaError_t e = occupancy_per_sm(fn, wpb, smem, &per_sm);
     if (e != cudaSuccess) { *err = std::string("pairs16 launch setup: ") + cudaGetErrorString(e); return PSB_ECUDA; }
-    if (per_sm < 1) per_sm = 1;
     if (warps_per_sm_out) *warps_per_sm_out = per_sm * wpb;
     const int ng = 32 / c.G;
     const long long slots = ((long long)p.nitems + ng - 1) / ng;
-    long long blocks = std::min<long long>((slots + wpb - 1) / wpb, (long long)sms * per_sm);
-    if (blocks < 1) blocks = 1;
     Pairs16Params pp = p;
-    void *args[] = {&pp};
-    e = cudaLaunchKernel(fn, dim3((unsigned)blocks), dim3(wpb * 32), args, smem, stream);
+    e = launch_persistent(fn, &pp, slots, wpb, smem, per_sm, sms, stream);
     if (e != cudaSuccess) { *err = std::string("pairs16 launch: ") + cudaGetErrorString(e); return PSB_ECUDA; }
     return PSB_OK;
 }
