@@ -159,11 +159,14 @@ struct DevMem {
 // calling thread (memcpy of one chunk while the previous one is on the link).  Page-locked sources (and small
 // copies) go straight to cudaMemcpyAsync.
 static constexpr size_t kBounceBytes = (size_t)8 << 20;
+static bool is_pageable(const void *p) {
+    cudaPointerAttributes at;
+    if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return true; }
+    return at.type == cudaMemoryTypeUnregistered;
+}
 static cudaError_t upload_h2d(void *dst, const void *src, size_t bytes, cudaStream_t stream) {
     if (bytes < ((size_t)1 << 20)) return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream);
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, src) != cudaSuccess) { cudaGetLastError(); at.type = cudaMemoryTypeUnregistered; }
-    if (at.type != cudaMemoryTypeUnregistered) return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream);
+    if (!is_pageable(src)) return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream);
     static const bool no_bounce = std::getenv("PSB_NO_BOUNCE") != nullptr;   // A/B knob: leave pageable memory to the driver
     if (no_bounce) return cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream);
     Ctx &c = g_ctx;
@@ -2307,6 +2310,13 @@ struct StreamMarks {
     }
 };
 
+// PSB_DEBUG_TIMING on psb_scan_host / psb_scan_box (`on` is false without it): the host's milliseconds since construction
+struct HostClock {
+    const bool on = std::getenv("PSB_DEBUG_TIMING") != nullptr;
+    const std::chrono::steady_clock::time_point t0 = std::chrono::steady_clock::now();
+    double ms() const { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count(); }
+};
+
 // `marks`: psb_scan_host's timeline (lengths< >lengths sort> <pack pack>), or nullptr
 static int db_finish(DbBuild &B, StreamMarks *marks = nullptr) {
     Ctx &c = g_ctx;
@@ -2346,14 +2356,23 @@ static int db_finish(DbBuild &B, StreamMarks *marks = nullptr) {
     return PSB_OK;
 }
 
+// a database the caller holds in host memory, checked in each entry point's wording; `arg` is the entry point's other
+// required pointer.  The host scans (`scan`) report offsets that do not increase as an empty database, before the
+// subject count; psb_db_create names them, after it.
+static int host_db_check(const char *who, const void *arg, const uint8_t *cat, const int64_t *off, int64_t n, bool scan) {
+    const std::string w(who);
+    if (!arg || !cat || !off || n <= 0 || (scan && off[n] <= off[0])) { set_error(w + ": NULL argument or empty database"); return PSB_EINVAL; }
+    if (n > 0x7ffffffe) { set_error(w + ": more than 2^31-2 subjects"); return PSB_EUNSUPPORTED; }
+    if (off[n] <= off[0]) { set_error(w + ": offsets are not increasing"); return PSB_EINVAL; }
+    return PSB_OK;
+}
+
 }  // namespace psb
 
 extern "C" {
 
 psb_db_t *psb_db_create(const uint8_t *cat, const int64_t *off, int64_t n, const parasail_matrix_t *matrix) {
-    if (!cat || !off || n <= 0 || !matrix) { set_error("psb_db_create: NULL argument or empty database"); return nullptr; }
-    if (n > 0x7ffffffe) { set_error("psb_db_create: more than 2^31-2 subjects"); return nullptr; }
-    if (off[n] <= off[0]) { set_error("psb_db_create: offsets are not increasing"); return nullptr; }
+    if (host_db_check("psb_db_create", matrix, cat, off, n, false) != PSB_OK) return nullptr;
     if (ensure_ctx() != PSB_OK) return nullptr;
     HostMatrix hm(matrix);
     // bits per residue from the residues actually present: a DNA database whose residues are all A/C/G/T
@@ -2493,6 +2512,17 @@ static int db_check(const char *who, const psb_db *db) {
     if (db->host_len.empty()) { set_error(std::string(who) + ": the database has no subject lengths on the host"); return PSB_EUNSUPPORTED; }
     return PSB_OK;
 }
+// the end of a scan entry point: the batch's cells, the flags of explicit _8 / _16 widths, and the batch handed over;
+// `subject_len(i)` is subject i's length
+template <typename SubjectLen>
+static int scan_batch_done(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap, int64_t residues, SubjectLen subject_len,
+                           psb_batch_t *b, psb_batch_t **out) {
+    const int lq = (int)profile->query.size();
+    b->cells = (double)profile->query.size() * (double)residues;
+    flag_saturated(cfg, profile->matrix, open, gap, b, [&](int64_t i) { return std::make_pair(lq, subject_len(i)); });
+    *out = b;
+    return PSB_OK;
+}
 // The database's inverse permutation, built on first use: the scatter runs on db->stream, behind the sort/pack chain
 // psb_db_create queued there (it returns before that chain has finished), and that stream is synchronised before the
 // pointer is published.  So whoever sees the pointer -- any host thread, any stream -- also sees finished packed words.
@@ -2530,17 +2560,12 @@ int psb_scan(const char *fn_name, const parasail_profile_t *profile, int open, i
     c.last_ms = 0.0; c.launches = 0;
     psb_batch_t *b = new_batch(db->n, cfg);
     if (!b) { set_error("pinned host allocation failed"); return PSB_ENOMEM; }
-    b->cells = (double)profile->query.size() * (double)db->residues;
     ScanJob job;
     int rc = scan_enqueue(job, cfg, profile, open, gap, db, batch_outputs(b).data(), 0);
     if (rc == PSB_OK) rc = scan_finish(job);
     if (rc != PSB_OK) { cudaStreamSynchronize(c.stream); free_batch(b); return rc; }
     b->n_retried = job.retried;
-    const int lq = (int)profile->query.size();
-    flag_saturated(cfg, profile->matrix, open, gap, b,
-                   [&](int64_t i) { return std::make_pair(lq, db->host_len.empty() ? db->maxlen : db->host_len[(size_t)i]); });
-    *out = b;
-    return PSB_OK;
+    return scan_batch_done(cfg, profile, open, gap, db->residues, [&](int64_t i) { return db->host_len.empty() ? db->maxlen : db->host_len[(size_t)i]; }, b, out);
 }
 
 int psb_db_align(const char *fn_name, const parasail_profile_t *profile, int open, int gap, const psb_db_t *db_c,
@@ -2620,22 +2645,6 @@ namespace psb {
 // into pieces whose upload (copy stream), device-side sort + packing and scan are pipelined, and the
 // per-subject results land in hosts[k][base ...] (pinned).  Used by psb_scan_host (one device, base 0) and by
 // the per-device workers of psb_scan_box (each with its own range of the caller's arrays).
-// measured rates of the host scan on this thread's device: what the piece plan is computed from
-struct HostScanRates {
-    double h2d_ms_per_byte = 0;     // residue uploads of >= 4 MB, exponentially averaged
-    uint64_t key = 0;               // the scan (function, query length, penalties) the next figure belongs to
-    double scan_ms_per_byte = 0;    // kernel time per database residue of that scan
-};
-static thread_local HostScanRates g_hs;
-// a finished piece's residue upload feeds the measured upload rate (both events have completed by now)
-static void note_upload(DbBuild &B) {
-    if (!B.res_begin || !B.uploaded || !B.db || B.db->residues < ((int64_t)4 << 20)) return;
-    float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, B.res_begin, B.uploaded) != cudaSuccess || ms <= 0.f) { cudaGetLastError(); return; }
-    const double now = (double)ms / (double)B.db->residues;
-    g_hs.h2d_ms_per_byte = g_hs.h2d_ms_per_byte > 0 ? 0.5 * g_hs.h2d_ms_per_byte + 0.5 * now : now;
-    cudaEventDestroy(B.res_begin); B.res_begin = nullptr;   // counted once
-}
 static uint64_t host_scan_key(const FnConfig &cfg, int lq, int open, int gap, int msize) {
     uint64_t h = 1469598103934665603ull;
     for (uint64_t x : {(uint64_t)encode_fn(cfg), (uint64_t)lq, (uint64_t)open, (uint64_t)gap, (uint64_t)msize}) { h ^= x + 1; h *= 1099511628211ull; }
@@ -2681,16 +2690,22 @@ std::vector<int64_t> plan_pieces(int64_t total, double u, double v) {
     return sizes;
 }
 
-struct ScanLeftovers {
-    std::vector<std::unique_ptr<DbBuild>> builds;
-    std::vector<std::unique_ptr<ScanJob>> jobs;
-    void clear() {
-        for (auto &b : builds) if (b && b->db) { psb_db_free(b->db); b->db = nullptr; }
-        jobs.clear(); builds.clear();
+// subject cuts of the database off[0 .. n] at residue targets (counted from off[0], increasing): 0, then for each target
+// the first subject boundary at or past it but at least one subject past the previous cut, then n.  A cut that would
+// leave no subject after it ends the list.
+static std::vector<int64_t> cut_subjects(const int64_t *off, int64_t n, const std::vector<int64_t> &targets) {
+    std::vector<int64_t> cut(1, 0);
+    for (const int64_t t : targets) {
+        const int64_t at = std::max<int64_t>(std::lower_bound(off, off + n + 1, off[0] + t) - off, cut.back() + 1);
+        if (at >= n) break;
+        cut.push_back(at);
     }
-};
+    cut.push_back(n);
+    return cut;
+}
+
 // The pieces of a host scan: the upload of piece k+1 (copy stream) runs under the scan of piece k, and nothing on the
-// host waits for the GPU until the last piece is queued.  The sizes follow from two measured rates (HostScanRates): with
+// host waits for the GPU until the last piece is queued.  The sizes follow from two measured rates (HostScanState): with
 // u = upload time and v = scan time per residue, piece k+1 may be r = 0.85 v/u times piece k and still land before
 // piece k has been scanned; the first piece and the number of pieces minimise
 // (upload of the first piece) + (pieces - 1) x (cost of a piece boundary).  plan_pieces() above.
@@ -2699,179 +2714,168 @@ struct PiecePlan {
     double u_rate = 0, v_rate = 0;      // upload and scan ms per residue the sizes were planned with
     std::vector<int64_t> cut;           // piece k is subjects cut[k] .. cut[k + 1] - 1
 };
-static PiecePlan plan_host_pieces(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap, const int64_t *off, int64_t n) {
-    PiecePlan pl;
-    const int64_t total = off[n] - off[0];
-    pl.rate_key = host_scan_key(cfg, (int)profile->query.size(), open, gap, profile->matrix.size);
-    const uint64_t rate_key = pl.rate_key;
-    const double u_rate = pl.u_rate = g_hs.h2d_ms_per_byte > 0 ? g_hs.h2d_ms_per_byte : 1e3 / 50e9;
-    const double v_rate = pl.v_rate = (g_hs.key == rate_key && g_hs.scan_ms_per_byte > 0)
-                                          ? g_hs.scan_ms_per_byte
-                                          : (double)profile->query.size() * 1e3 / (sw16_wanted(cfg) ? 4.9e12 : 1.5e12);
-    std::vector<int64_t> sizes;
-    const char *e_piece = std::getenv("PSB_SCAN_HOST_PIECE_MB"), *e_first = std::getenv("PSB_SCAN_HOST_FIRST_MB"), *e_div = std::getenv("PSB_SCAN_HOST_FIRST_DIV");
-    if (e_piece || e_first || e_div) {
-        // experiments (tools/shard_e2e_probe.py): a first piece of total/div capped at first_mb, the rest in equal pieces
-        const long long piece_mb = e_piece ? std::max(8ll, std::atoll(e_piece)) : 96, first_mb = e_first ? std::max(1ll, std::atoll(e_first)) : 24;
-        const long long first_div = e_div ? std::max(1ll, std::atoll(e_div)) : 4;
-        const int64_t piece = piece_mb << 20;
-        const int64_t first_cap = std::min<int64_t>(first_mb << 20, std::max<int64_t>((int64_t)4 << 20, total / first_div));
-        const int64_t first = total > first_cap + ((int64_t)4 << 20) ? first_cap : total;
-        const int nrest = first == total ? 0 : (int)std::max<int64_t>(1, std::min<int64_t>(30, (total - first + piece * 3 / 4) / piece));
-        sizes.push_back(first);
-        for (int k = 0; k < nrest; ++k) sizes.push_back((total - first) * (k + 1) / nrest - (total - first) * k / nrest);
-    } else {
-        sizes = plan_pieces(total, u_rate, v_rate);
+// what this thread's host scans are planned from: the measured rates of its device and the previous plan
+struct HostScanState {
+    double h2d_ms_per_byte = 0;     // residue uploads of >= 4 MB
+    uint64_t key = 0;               // the scan (function, query length, penalties) scan_ms_per_byte belongs to
+    double scan_ms_per_byte = 0;    // kernel time per database residue of that scan
+    int64_t last_total = 0;         // the previous plan: residues, scan and piece sizes
+    uint64_t last_key = 0;
+    std::vector<int64_t> last_sizes;
+    // the rates are exponential averages: a new figure counts half
+    static double average(double old, double now) { return old > 0 ? 0.5 * old + 0.5 * now : now; }
+    // a finished piece's residue upload (both events have completed by now), counted once
+    void note_upload(DbBuild &B) {
+        if (!B.res_begin || !B.uploaded || !B.db || B.db->residues < ((int64_t)4 << 20)) return;
+        float ms = 0.f;
+        if (cudaEventElapsedTime(&ms, B.res_begin, B.uploaded) != cudaSuccess || ms <= 0.f) { cudaGetLastError(); return; }
+        h2d_ms_per_byte = average(h2d_ms_per_byte, (double)ms / (double)B.db->residues);
+        cudaEventDestroy(B.res_begin); B.res_begin = nullptr;
+    }
+    // a host scan of `total` residues whose kernels took `ms`
+    void note_scan(uint64_t scan_key, double ms, int64_t total) {
+        scan_ms_per_byte = average(key == scan_key ? scan_ms_per_byte : 0, ms / (double)total);
+        key = scan_key;
+    }
+    // the pieces of a call, from the measured rates (defaults for what has not been measured yet)
+    PiecePlan plan(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap, const int64_t *off, int64_t n) {
+        PiecePlan pl;
+        const int64_t total = off[n] - off[0];
+        pl.rate_key = host_scan_key(cfg, (int)profile->query.size(), open, gap, profile->matrix.size);
+        const double u_rate = pl.u_rate = h2d_ms_per_byte > 0 ? h2d_ms_per_byte : 1e3 / 50e9;
+        const double v_rate = pl.v_rate = (key == pl.rate_key && scan_ms_per_byte > 0)
+                                              ? scan_ms_per_byte
+                                              : (double)profile->query.size() * 1e3 / (sw16_wanted(cfg) ? 4.9e12 : 1.5e12);
+        std::vector<int64_t> sizes = plan_pieces(total, u_rate, v_rate);
         // hysteresis: the rates are measured and move a little from call to call; a plan that is still within 5 % of
         // the best one is kept, so that a service repeating a scan keeps its allocation sizes (a new size can mean a
         // host-blocking growth of the memory pool)
-        static thread_local struct { int64_t total = 0; uint64_t key = 0; std::vector<int64_t> sizes; } last;
         auto exposed = [&](const std::vector<int64_t> &sz) {
             double t = (double)sz[0] * u_rate + 0.35 * (double)(sz.size() - 1);
             for (size_t k = 0; k + 1 < sz.size(); ++k) t += std::max(0.0, (double)sz[k + 1] * u_rate - (double)sz[k] * v_rate);
             return t;
         };
-        if (last.total == total && last.key == rate_key && !last.sizes.empty() && exposed(last.sizes) <= 1.05 * exposed(sizes) + 0.05) sizes = last.sizes;
-        last.total = total; last.key = rate_key; last.sizes = sizes;
+        if (last_total == total && last_key == pl.rate_key && !last_sizes.empty() && exposed(last_sizes) <= 1.05 * exposed(sizes) + 0.05) sizes = last_sizes;
+        last_total = total; last_key = pl.rate_key; last_sizes = sizes;
+        std::vector<int64_t> ends(sizes.size() - 1);   // residues up to the end of every piece but the last
+        std::partial_sum(sizes.begin(), sizes.end() - 1, ends.begin());
+        pl.cut = cut_subjects(off, n, ends);
+        return pl;
     }
-    // cut on subject boundaries
-    std::vector<int64_t> &cut = pl.cut;
-    cut.assign(1, 0);
-    int64_t acc = 0;
-    for (size_t k = 0; k + 1 < sizes.size() && cut.back() < n; ++k) {
-        acc += sizes[k];
-        int64_t at = std::lower_bound(off, off + n + 1, off[0] + acc) - off;
-        if (at <= cut.back()) at = cut.back() + 1;
-        if (at >= n) break;
-        cut.push_back(at);
-    }
-    cut.push_back(n);
-    return pl;
+};
+static thread_local HostScanState g_hs;
+
+// one piece of a host scan: its uploads and packed shard, and its scan.  Destroying it gives the packed shard, the
+// staging blocks and the result arrays back; the owner has synchronised the streams that used them.
+struct HostPiece {
+    DbBuild build;
+    ScanJob job;
+    ~HostPiece() { psb_db_free(build.db); }
+};
+
+// the query side, while the compute stream is idle: a profile's first use on a device uploads it and waits for that
+// upload, which would otherwise happen inside the first piece's scan_enqueue, behind that piece's whole chain
+static int prepare_query(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap) {
+    DevProfile *dp = nullptr;
+    PSB_TRY(get_dev_profile(profile, &dp));
+    std::vector<Sw16Profile> sp;
+    if (sw16_wanted(cfg)) sw16_prepare(profile, dp, open, gap, &sp);
+    return PSB_OK;
 }
 
+// piece k's host pass over its offsets and its sort/pack chain.  PSB_DEBUG_TIMING also makes the chain's first mark
+// wait for the piece's offsets, so that the timeline shows when they landed.
+static int build_piece(HostPiece &p, const int64_t *off, int k, StreamMarks &tl, const HostClock &clk) {
+    Ctx &c = g_ctx;
+    const double h0 = clk.on ? clk.ms() : 0.0;
+    int rc = db_host_pass(p.build, off);
+    const double h1 = clk.on ? clk.ms() : 0.0;
+    if (clk.on) { cudaStreamWaitEvent(c.stream, p.build.offs_up, 0); tl.mark(c.stream); }
+    if (rc == PSB_OK) rc = db_finish(p.build, &tl);
+    if (clk.on) std::fprintf(stderr, "[psb] scan_host(dev %d): piece %d host: offsets pass + allocations %.3f ms, chain launches %.3f ms\n", c.device, k, h1 - h0, clk.ms() - h1);
+    tl.mark(c.stream);
+    return rc;
+}
+
+// waits until the piece's results are on the host; its re-runs and its upload time are counted once
+static int finish_piece(HostPiece &p, int64_t *n_retried) {
+    int rc = PSB_OK;
+    if (p.job.ev0 && !p.job.finished) { rc = scan_finish(p.job); *n_retried += p.job.retried; }
+    g_hs.note_upload(p.build);
+    return rc;
+}
+
+// `keep_last`: takes over the last piece once its results are on the host, for a caller with a better moment to give
+// its device memory back (psb_scan_box's workers, after they have reported completion)
 static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap, const uint8_t *cat,
                           const int64_t *off, int64_t n, int *const hosts[6], int64_t base, int64_t *n_retried,
-                          ScanLeftovers *leftovers = nullptr) {
+                          std::unique_ptr<HostPiece> *keep_last = nullptr) {
     Ctx &c = g_ctx;
-    const HostMatrix &hm = profile->matrix;
-    const int64_t total = off[n] - off[0];
-    const PiecePlan pl = plan_host_pieces(cfg, profile, open, gap, off, n);
+    const HostClock clk{};
+    const PiecePlan pl = g_hs.plan(cfg, profile, open, gap, off, n);
     const std::vector<int64_t> &cut = pl.cut;
     const int npieces = (int)cut.size() - 1;
     const double ms_at_entry = c.last_ms;
-    int rc = PSB_OK;
-    std::vector<std::unique_ptr<DbBuild>> builds(npieces);
-    std::vector<std::unique_ptr<ScanJob>> jobs(npieces);
-    for (int k = 0; k < npieces; ++k) { builds[k].reset(new DbBuild()); jobs[k].reset(new ScanJob()); }
-    bool pageable_src = false;
-    {
-        cudaPointerAttributes at;
-        if (cudaPointerGetAttributes(&at, cat + off[0]) != cudaSuccess) { cudaGetLastError(); pageable_src = true; }
-        else pageable_src = at.type == cudaMemoryTypeUnregistered;
-    }
-    bool eager = false;   // experiment knob: 1 = every upload queued right behind the previous one, no gating
-    if (const char *ev = std::getenv("PSB_SCAN_HOST_EAGER_UPLOAD")) eager = std::atoi(ev) != 0;
-    auto upload = [&](int k) -> int {
-        if (cut[k + 1] <= cut[k]) return PSB_OK;
-        cudaEvent_t gate = (!eager && k > 0 && builds[k - 1]) ? builds[k - 1]->packed : nullptr;
-        return db_upload(*builds[k], cat, off + cut[k], cut[k + 1] - cut[k], hm, true, 0, gate) ? PSB_OK : PSB_ECUDA;
-    };
-    // a finished piece gives its device memory back (staging blocks, packed shard, result arrays), so
-    // at most kDepth pieces are resident however large the host database is
-    const int kDepth = 4;
-    auto retire = [&](int k) -> int {
-        if (k < 0 || !jobs[k]) return PSB_OK;
-        int r = PSB_OK;
-        if (jobs[k]->ev0 && !jobs[k]->finished) { r = scan_finish(*jobs[k]); *n_retried += jobs[k]->retried; }
-        if (builds[k]) note_upload(*builds[k]);
-        if (builds[k] && builds[k]->db) { psb_db_free(builds[k]->db); builds[k]->db = nullptr; }
-        jobs[k].reset(); builds[k].reset();
-        return r;
-    };
-    const bool dbg = std::getenv("PSB_DEBUG_TIMING") != nullptr;
-    const auto t_in = std::chrono::steady_clock::now();
-    auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_in).count(); };
-    if (dbg) {
+    const bool pageable = is_pageable(cat + off[0]);
+    if (clk.on) {
         std::string line;
         for (int k = 0; k < npieces; ++k) line += " " + std::to_string((off[cut[k + 1]] - off[cut[k]]) >> 20);
         std::fprintf(stderr, "[psb] scan_host(dev %d): pieces (MB):%s; upload %.1f GB/s, scan %.1f GB/s of residues\n", c.device, line.c_str(),
                      1e-6 / pl.u_rate, 1e-6 / pl.v_rate);
     }
-    // order of the host's work: the copy engine comes first.  Upload k+1 is queued before any host time goes into
-    // piece k (its offsets pass, the sort/pack launches, the scan launches), so the link never waits for the host.
+    // a finished piece gives its device memory back, so at most kDepth pieces are resident however large the host
+    // database is
+    const int kDepth = 4;
+    std::vector<std::unique_ptr<HostPiece>> pieces(npieces);
+    int rc = PSB_OK;
+    auto finish = [&](int k) {
+        if (!pieces[k]) return;
+        const int r = finish_piece(*pieces[k], n_retried);
+        if (rc == PSB_OK) rc = r;
+        pieces[k].reset();
+    };
     // PSB_DEBUG_TIMING: a device-side timeline (upload landed / packing begins / scan begins / scan ends / results
     // on the host), relative to an event recorded on the idle compute stream at entry
     StreamMarks tl;
-    auto mark = [&](cudaStream_t st) { tl.mark(st); };
-    mark(c.stream);
-    rc = upload(0);
-    mark(c.copy);
-    // the query side now, while the compute stream is idle: a profile's first use on a device uploads it and waits
-    // for that upload, which would otherwise happen inside scan_enqueue(0) behind the first piece's whole chain
-    if (rc == PSB_OK) {
-        DevProfile *dp0 = nullptr;
-        rc = get_dev_profile(profile, &dp0);
-        std::vector<Sw16Profile> sp0;
-        if (rc == PSB_OK && sw16_wanted(cfg)) sw16_prepare(profile, dp0, open, gap, &sp0);
-    }
-    if (dbg) std::fprintf(stderr, "[psb] scan_host(dev %d): %d pieces, first upload queued at %.3f ms\n", c.device, npieces, since());
-    auto next_upload = [&](int k) {
-        if (k + 1 >= npieces || rc != PSB_OK) return;
-        if (k + 1 >= kDepth) rc = retire(k + 1 - kDepth);
-        if (rc == PSB_OK) rc = upload(k + 1);
-        if (rc == PSB_OK) mark(c.copy);
+    // piece k goes up after piece k - kDepth is finished; its residues wait for piece k-1's chain
+    auto upload = [&](int k) {
+        if (k >= npieces || rc != PSB_OK) return;
+        if (k >= kDepth) finish(k - kDepth);
+        if (rc != PSB_OK) return;
+        pieces[k].reset(new HostPiece());
+        cudaEvent_t gate = k > 0 ? pieces[k - 1]->build.packed : nullptr;
+        if (!db_upload(pieces[k]->build, cat, off + cut[k], cut[k + 1] - cut[k], profile->matrix, true, 0, gate)) rc = PSB_ECUDA;
+        else tl.mark(c.copy);
     };
+    auto scan = [&](int k) {
+        if (rc == PSB_OK) rc = scan_enqueue(pieces[k]->job, cfg, profile, open, gap, pieces[k]->build.db, hosts, base + cut[k]);
+        tl.mark(c.stream);
+    };
+    tl.mark(c.stream);
+    upload(0);
+    if (rc == PSB_OK) rc = prepare_query(cfg, profile, open, gap);
+    if (clk.on) std::fprintf(stderr, "[psb] scan_host(dev %d): %d pieces, first upload queued at %.3f ms\n", c.device, npieces, clk.ms());
     for (int k = 0; k < npieces && rc == PSB_OK; ++k) {
-        if (eager) next_upload(k);
-        if (rc != PSB_OK) break;
-        if (!builds[k]->db) { if (!eager) next_upload(k); continue; }
-        const double h0 = dbg ? since() : 0.0;
-        rc = db_host_pass(*builds[k], off + cut[k]);
-        const double h1 = dbg ? since() : 0.0;
-        if (dbg) { cudaStreamWaitEvent(c.stream, builds[k]->offs_up, 0); mark(c.stream); }
-        if (rc == PSB_OK) rc = db_finish(*builds[k], &tl);
-        if (dbg) std::fprintf(stderr, "[psb] scan_host(dev %d): piece %d host: offsets pass + allocations %.3f ms, chain launches %.3f ms\n", c.device, k, h1 - h0, since() - h1);
-        mark(c.stream);
-        // the next piece's upload is queued as soon as its gate (this piece's chain) exists, before host time
-        // goes into this piece's scan launches -- unless the caller's memory is pageable: then the upload is a
-        // memcpy loop on this thread (upload_h2d) and this piece's scan has to be on the device first
-        if (!eager && !pageable_src) next_upload(k);
-        if (rc == PSB_OK) rc = scan_enqueue(*jobs[k], cfg, profile, open, gap, builds[k]->db, hosts, base + cut[k]);
-        mark(c.stream);
-        if (!eager && pageable_src) next_upload(k);
-        if (dbg) std::fprintf(stderr, "[psb] scan_host(dev %d): piece %d queued at %.3f ms\n", c.device, k, since());
+        rc = build_piece(*pieces[k], off + cut[k], k, tl, clk);
+        // the next upload goes in as soon as its gate (this piece's chain) exists -- unless the caller's memory is
+        // pageable: then the upload is a memcpy loop on this thread (upload_h2d) and this piece's scan has to be on the
+        // device first
+        if (pageable) { scan(k); upload(k + 1); } else { upload(k + 1); scan(k); }
+        if (clk.on) std::fprintf(stderr, "[psb] scan_host(dev %d): piece %d queued at %.3f ms\n", c.device, k, clk.ms());
     }
-    // everything is queued: the host retires the earlier pieces while the last ones are still being scanned
-    for (int k = 0; k + 1 < npieces; ++k) {
-        const int r = retire(k);
-        if (rc == PSB_OK) rc = r;
-    }
+    // everything is queued: the host finishes the earlier pieces while the last ones are still being scanned
+    for (int k = 0; k + 1 < npieces; ++k) finish(k);
     cudaStreamSynchronize(c.copy);
-    if (dbg) std::fprintf(stderr, "[psb] scan_host(dev %d): uploads done at %.3f ms\n", c.device, since());
-    if (rc == PSB_OK && jobs[npieces - 1] && jobs[npieces - 1]->ev0) {
-        rc = scan_finish(*jobs[npieces - 1]);
-        *n_retried += jobs[npieces - 1]->retried;
-    }
+    if (clk.on) std::fprintf(stderr, "[psb] scan_host(dev %d): uploads done at %.3f ms\n", c.device, clk.ms());
+    if (rc == PSB_OK) rc = finish_piece(*pieces[npieces - 1], n_retried);
     cudaStreamSynchronize(c.stream);
-    if (dbg) std::fprintf(stderr, "[psb] scan_host(dev %d): all done at %.3f ms\n", c.device, since());
+    if (clk.on) std::fprintf(stderr, "[psb] scan_host(dev %d): all done at %.3f ms\n", c.device, clk.ms());
     // order of the marks: entry | upload 0 | per piece k: [upload k+1] upload-k-landed (lengths< >lengths sort> <pack pack>) pack-end results-on-host
-    if (dbg && !tl.ev.empty()) std::fprintf(stderr, "[psb] scan_host(dev %d): device timeline (ms after entry):%s\n", c.device, tl.line().c_str());
-    // the results are on the host.  What is left is giving the last piece's device memory back: a caller with
-    // somewhere better to do that (psb_scan_box's workers, after they have reported completion) takes it over
-    if (rc == PSB_OK && total >= ((int64_t)8 << 20) && c.last_ms > ms_at_entry) {
-        const double now = (c.last_ms - ms_at_entry) / (double)total;
-        g_hs.scan_ms_per_byte = g_hs.key == pl.rate_key && g_hs.scan_ms_per_byte > 0 ? 0.5 * g_hs.scan_ms_per_byte + 0.5 * now : now;
-        g_hs.key = pl.rate_key;
-    }
-    if (leftovers && rc == PSB_OK) {
-        if (builds[npieces - 1]) note_upload(*builds[npieces - 1]);
-        leftovers->builds.push_back(std::move(builds[npieces - 1]));
-        leftovers->jobs.push_back(std::move(jobs[npieces - 1]));
-    }
-    for (int k = 0; k < npieces; ++k) {
-        const int r = retire(k);
-        if (rc == PSB_OK) rc = r;
-    }
+    if (clk.on && !tl.ev.empty()) std::fprintf(stderr, "[psb] scan_host(dev %d): device timeline (ms after entry):%s\n", c.device, tl.line().c_str());
+    const int64_t total = off[n] - off[0];
+    if (rc == PSB_OK && total >= ((int64_t)8 << 20) && c.last_ms > ms_at_entry) g_hs.note_scan(pl.rate_key, c.last_ms - ms_at_entry, total);
+    if (keep_last && rc == PSB_OK) *keep_last = std::move(pieces[npieces - 1]);
+    for (int k = 0; k < npieces; ++k) finish(k);
     return rc;
 }
 
@@ -2884,7 +2888,7 @@ struct BoxWorker {
     std::condition_variable cv;
     std::function<void()> job;
     bool has_job = false, quit = false;
-    ScanLeftovers left;   // device memory of the last piece of the call just reported: given back after the report
+    std::unique_ptr<HostPiece> left;   // device memory of the last piece of the call just reported: given back after the report
     void loop() {
         psb_set_device(device);
         std::unique_lock<std::mutex> lk(mu);
@@ -2898,7 +2902,7 @@ struct BoxWorker {
             has_job = false;
             cv.notify_all();
             lk.unlock();
-            left.clear();   // off the caller's critical path (about 0.1 ms of frees and event destruction)
+            left.reset();   // off the caller's critical path (about 0.1 ms of frees and event destruction)
             lk.lock();
         }
     }
@@ -2991,20 +2995,15 @@ int psb_scan_host(const char *fn_name, const parasail_profile_t *profile, int op
     if (out) *out = nullptr;
     FnConfig cfg;
     PSB_TRY(scan_check("psb_scan_host", fn_name, profile, &cfg));
-    if (!cat || !off || n <= 0 || !out || off[n] <= off[0]) { set_error("psb_scan_host: NULL argument or empty database"); return PSB_EINVAL; }
-    if (n > 0x7ffffffe) { set_error("psb_scan_host: more than 2^31-2 subjects"); return PSB_EUNSUPPORTED; }
+    PSB_TRY(host_db_check("psb_scan_host", out, cat, off, n, true));
     PSB_TRY(ensure_ctx());
     Ctx &c = g_ctx;
     c.last_ms = 0.0; c.launches = 0;
     psb_batch_t *b = new_batch(n, cfg);
     if (!b) { set_error("pinned host allocation failed"); return PSB_ENOMEM; }
-    b->cells = (double)profile->query.size() * (double)(off[n] - off[0]);
     const int rc = scan_host_into(cfg, profile, open, gap, cat, off, n, batch_outputs(b).data(), 0, &b->n_retried);
     if (rc != PSB_OK) { free_batch(b); return rc; }
-    const int lq = (int)profile->query.size();
-    flag_saturated(cfg, profile->matrix, open, gap, b, [&](int64_t i) { return std::make_pair(lq, span(off, i)); });
-    *out = b;
-    return PSB_OK;
+    return scan_batch_done(cfg, profile, open, gap, off[n] - off[0], [&](int64_t i) { return span(off, i); }, b, out);
 }
 
 // The whole box from one process and one call (SURVEY 8b/8e): the database is cut into n_gpus contiguous
@@ -3017,64 +3016,53 @@ int psb_scan_box(const char *fn_name, const parasail_profile_t *profile, int ope
     if (out) *out = nullptr;
     FnConfig cfg;
     PSB_TRY(scan_check("psb_scan_box", fn_name, profile, &cfg));
-    if (!cat || !off || n <= 0 || !out || off[n] <= off[0]) { set_error("psb_scan_box: NULL argument or empty database"); return PSB_EINVAL; }
-    if (n > 0x7ffffffe) { set_error("psb_scan_box: more than 2^31-2 subjects"); return PSB_EUNSUPPORTED; }
+    PSB_TRY(host_db_check("psb_scan_box", out, cat, off, n, true));
     const int ndev = psb_device_count();
     if (ndev <= 0) { set_error("no CUDA device available: libparasail_b200 has no CPU fallback (needs an sm_100a GPU)"); return PSB_ENODEV; }
     if (n_gpus <= 0 || n_gpus > ndev) n_gpus = ndev;
     if ((int64_t)n_gpus > n) n_gpus = (int)n;
-    const bool dbg = std::getenv("PSB_DEBUG_TIMING") != nullptr;
-    const auto t_in = std::chrono::steady_clock::now();
-    auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_in).count(); };
+    const HostClock clk{};
     PSB_TRY(ensure_ctx());   // the batch's pinned arrays are allocated by the calling thread
     psb_batch_t *b = new_batch(n, cfg);
     if (!b) { set_error("pinned host allocation failed"); return PSB_ENOMEM; }
-    if (dbg) std::fprintf(stderr, "[psb] scan_box: batch ready at %.3f ms\n", since());
+    if (clk.on) std::fprintf(stderr, "[psb] scan_box: batch ready at %.3f ms\n", clk.ms());
     const int64_t total = off[n] - off[0];
-    b->cells = (double)profile->query.size() * (double)total;
-    std::vector<int64_t> cut(n_gpus + 1, n);
-    cut[0] = 0;
-    for (int d = 1; d < n_gpus; ++d) {
-        cut[d] = std::lower_bound(off, off + n + 1, off[0] + total * d / n_gpus) - off;
-        if (cut[d] <= cut[d - 1]) cut[d] = std::min<int64_t>(n, cut[d - 1] + 1);
-    }
+    std::vector<int64_t> targets;
+    for (int d = 1; d < n_gpus; ++d) targets.push_back(total * d / n_gpus);
+    // device d scans range d; the devices past the last range have no work
+    const std::vector<int64_t> cut = cut_subjects(off, n, targets);
+    const int nranges = (int)cut.size() - 1;
     const std::array<int *, 6> hosts = batch_outputs(b);
-    std::vector<int> rcs(n_gpus, PSB_OK), launches(n_gpus, 0);
-    std::vector<int64_t> retried(n_gpus, 0);
-    std::vector<double> ms(n_gpus, 0.0);
-    std::vector<std::string> errs(n_gpus);
-    for (int d = 0; d < n_gpus; ++d) {
-        if (cut[d + 1] <= cut[d]) continue;
+    struct DeviceResult { int rc = PSB_OK, launches = 0; int64_t retried = 0; double ms = 0.0; std::string err; };
+    std::vector<DeviceResult> res(nranges);
+    for (int d = 0; d < nranges; ++d) {
         BoxWorker *w = box_worker(d);
         w->submit([&, d, w] {
-            int rc = ensure_ctx();
-            if (rc == PSB_OK) {
+            DeviceResult &r = res[d];
+            r.rc = ensure_ctx();
+            if (r.rc == PSB_OK) {
                 g_ctx.last_ms = 0.0; g_ctx.launches = 0;
-                rc = scan_host_into(cfg, profile, open, gap, cat, off + cut[d], cut[d + 1] - cut[d], hosts.data(), cut[d], &retried[d], &w->left);
-                ms[d] = g_ctx.last_ms; launches[d] = g_ctx.launches;
+                r.rc = scan_host_into(cfg, profile, open, gap, cat, off + cut[d], cut[d + 1] - cut[d], hosts.data(), cut[d], &r.retried, &w->left);
+                r.ms = g_ctx.last_ms; r.launches = g_ctx.launches;
             }
-            rcs[d] = rc;
-            if (rc != PSB_OK) errs[d] = psb_last_error();
+            if (r.rc != PSB_OK) r.err = psb_last_error();
         });
     }
     int rc = PSB_OK;
     Ctx &c = g_ctx;
     c.last_ms = 0.0; c.launches = 0;
-    if (dbg) std::fprintf(stderr, "[psb] scan_box: %d ranges submitted at %.3f ms\n", n_gpus, since());
-    for (int d = 0; d < n_gpus; ++d) {
-        if (cut[d + 1] <= cut[d]) continue;
+    if (clk.on) std::fprintf(stderr, "[psb] scan_box: %d ranges submitted at %.3f ms\n", n_gpus, clk.ms());
+    for (int d = 0; d < nranges; ++d) {
         box_worker(d)->wait();
-        if (dbg) std::fprintf(stderr, "[psb] scan_box: device %d done at %.3f ms\n", d, since());
-        if (rcs[d] != PSB_OK && rc == PSB_OK) { rc = rcs[d]; set_error("psb_scan_box (device " + std::to_string(d) + "): " + errs[d]); }
-        b->n_retried += retried[d];
-        c.last_ms = std::max(c.last_ms, ms[d]);   // the devices run side by side: the slowest one
-        c.launches += launches[d];
+        if (clk.on) std::fprintf(stderr, "[psb] scan_box: device %d done at %.3f ms\n", d, clk.ms());
+        const DeviceResult &r = res[d];
+        if (r.rc != PSB_OK && rc == PSB_OK) { rc = r.rc; set_error("psb_scan_box (device " + std::to_string(d) + "): " + r.err); }
+        b->n_retried += r.retried;
+        c.last_ms = std::max(c.last_ms, r.ms);   // the devices run side by side: the slowest one
+        c.launches += r.launches;
     }
     if (rc != PSB_OK) { free_batch(b); return rc; }
-    const int lq = (int)profile->query.size();
-    flag_saturated(cfg, profile->matrix, open, gap, b, [&](int64_t i) { return std::make_pair(lq, span(off, i)); });
-    *out = b;
-    return PSB_OK;
+    return scan_batch_done(cfg, profile, open, gap, total, [&](int64_t i) { return span(off, i); }, b, out);
 }
 
 int psb_batch_topk(const psb_batch_t *batch, int k, int64_t *idx_out, int *score_out) {

@@ -2,7 +2,7 @@
 """probe (multi-GPU box): where does a psb_scan_box call spend its time?
  1. plain concurrent host->device copies from ONE pinned buffer to 1, 2, 4, ... devices: the PCIe / host-memory ceiling
  2. psb_scan_box timeline (PSB_DEBUG_TIMING) at the largest device count
- 3. psb_scan_box wall time over the first-piece divisor
+ 3. psb_scan_box wall time at 1, 2, 4, ... devices, with the library's own piece plan
 usage: python tools/box_probe.py [n_gpus]"""
 import os, sys, time, threading
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -47,15 +47,10 @@ def timed(ng, reps=8):
         t0 = time.perf_counter(); a.scan_box(args, ng); ts.append(time.perf_counter() - t0)
     return float(np.median(ts)), min(ts)
 
-# 3. wall time over the knobs
+# 3. wall time per device count
 for ng in [g for g in (1, 2, 4, 8) if g <= ng_max]:
-    for div in (4, 6, 8, 3, 1):
-        os.environ["PSB_SCAN_HOST_FIRST_DIV"] = str(div)
-        if div == 1: os.environ["PSB_SCAN_HOST_FIRST_MB"] = "1000"
-        med, mn = timed(ng)
-        os.environ.pop("PSB_SCAN_HOST_FIRST_MB", None)
-        print(f"scan_box n_gpus {ng} first_div {div}: median {med * 1e3:.3f} ms (min {mn * 1e3:.3f}), {cells / med / 1e9:.0f} GCUPS, slowest device's kernels {ps.kernel_ms():.3f} ms", flush=True)
-os.environ["PSB_SCAN_HOST_FIRST_DIV"] = "4"
+    med, mn = timed(ng)
+    print(f"scan_box n_gpus {ng}: median {med * 1e3:.3f} ms (min {mn * 1e3:.3f}), {cells / med / 1e9:.0f} GCUPS, slowest device's kernels {ps.kernel_ms():.3f} ms", flush=True)
 
 # 2. one timeline
 sys.stdout.flush()

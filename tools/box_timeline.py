@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """probe: one psb_scan_box call with PSB_DEBUG_TIMING (host and device timelines per device) after warm-up.
-usage: python tools/box_timeline.py [n_gpus] [first_div ...]"""
+usage: python tools/box_timeline.py [n_gpus]"""
 import os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -8,28 +8,18 @@ import numpy as np, torch, bench
 import parasail_rs_b200 as ps
 
 ng = min(int(sys.argv[1]) if len(sys.argv) > 1 else 8, torch.cuda.device_count())
-divs = [x for x in sys.argv[2:]] or ["auto"]
 query, cat, off = bench.make_inputs(1000000)
 pc = torch.empty(len(cat), dtype=torch.uint8, pin_memory=True); pc.numpy()[:] = cat
 po = torch.empty(len(off), dtype=torch.int64, pin_memory=True); po.numpy()[:] = off
 a = ps.Aligner.new().local().gap_open(10).gap_extend(1).profile(ps.Profile.new(query, False, ps.Matrix.from_name("blosum62"))).build()
 args = (pc.numpy(), po.numpy())
 cells = 400.0 * float(off[-1])
-for div in divs:
-    # a setting is first_div[:eager]
-    if div == "auto":
-        os.environ.pop("PSB_SCAN_HOST_FIRST_DIV", None)   # the library's own plan (measured rates)
-    else:
-        os.environ["PSB_SCAN_HOST_FIRST_DIV"] = div.split(":")[0]
-    os.environ["PSB_SCAN_HOST_EAGER_UPLOAD"] = div.split(":")[1] if ":" in div else "1"
-    os.environ.pop("PSB_DEBUG_TIMING", None)
-    for _ in range(6): a.scan_box(args, ng)
-    ts = []
-    for _ in range(10):
-        t0 = time.perf_counter(); a.scan_box(args, ng); ts.append(time.perf_counter() - t0)
-    print(f"scan_box n_gpus {ng} first_div {div}: median {np.median(ts) * 1e3:.3f} ms (min {min(ts) * 1e3:.3f}), {cells / np.median(ts) / 1e9:.0f} GCUPS, "
-          f"slowest device's kernels {ps.kernel_ms():.3f} ms", flush=True)
-    os.environ["PSB_DEBUG_TIMING"] = "1"
-    sys.stderr.write(f"---- first_div {div}\n"); sys.stderr.flush()
-    a.scan_box(args, ng)
-    sys.stderr.flush()
+for _ in range(6): a.scan_box(args, ng)
+ts = []
+for _ in range(10):
+    t0 = time.perf_counter(); a.scan_box(args, ng); ts.append(time.perf_counter() - t0)
+print(f"scan_box n_gpus {ng}: median {np.median(ts) * 1e3:.3f} ms (min {min(ts) * 1e3:.3f}), {cells / np.median(ts) / 1e9:.0f} GCUPS, "
+      f"slowest device's kernels {ps.kernel_ms():.3f} ms", flush=True)
+os.environ["PSB_DEBUG_TIMING"] = "1"
+a.scan_box(args, ng)
+sys.stderr.flush()

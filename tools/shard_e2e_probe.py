@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""probe: psb_scan_host on a 1/N shard of the C2 database (what each device of psb_scan_box sees at N GPUs) over the
-piece-size knobs.  usage: python tools/shard_e2e_probe.py [nshards] [first_div:first_mb ...]"""
+"""probe: psb_scan_host on a 1/N shard of the C2 database (what each device of psb_scan_box sees at N GPUs), with the
+library's own piece plan.  usage: python tools/shard_e2e_probe.py [nshards]"""
 import os, sys, time
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -8,7 +8,6 @@ import numpy as np, torch, bench
 import parasail_rs_b200 as ps
 
 nsh = int(sys.argv[1]) if len(sys.argv) > 1 else 8
-settings = [None if a == "auto" else tuple(int(x) for x in a.split(":")) for a in sys.argv[2:]] or [None, (4, 24), (1, 1000)]
 query, cat, off = bench.make_inputs(1000000)
 total = int(off[-1])
 cut = int(np.searchsorted(off, total // nsh))
@@ -22,18 +21,12 @@ fresh = os.environ.get("PROBE_FRESH") == "1"   # a new Profile + Aligner for eve
 def call():
     al = ps.Aligner.new().local().gap_open(10).gap_extend(1).profile(ps.Profile.new(query, False, b62)).build() if fresh else a
     return al.scan_host((pc.numpy(), po.numpy()))
-for st in settings:
-    # None: the library's own plan (measured rates); (div, mb): first piece = total/div capped at mb MB, 96 MB pieces after it
-    div, mb = st if st else ("auto", 0)
-    if st: os.environ["PSB_SCAN_HOST_FIRST_DIV"] = str(div); os.environ["PSB_SCAN_HOST_FIRST_MB"] = str(mb)
-    else: os.environ.pop("PSB_SCAN_HOST_FIRST_DIV", None); os.environ.pop("PSB_SCAN_HOST_FIRST_MB", None)
-    for _ in range(6): call()
-    ts = []
-    for _ in range(10):
-        t0 = time.perf_counter(); call(); ts.append(time.perf_counter() - t0)
-    print(f"shard 1/{nsh} ({so[-1] / 1e6:.1f} MB): first = total/{div} capped at {mb} MB: median {np.median(ts) * 1e3:.3f} ms, min {min(ts) * 1e3:.3f} ms, kernels {ps.kernel_ms():.3f} ms, "
-          f"{cells / np.median(ts) / 1e9:.0f} GCUPS", flush=True)
+for _ in range(6): call()
+ts = []
+for _ in range(10):
+    t0 = time.perf_counter(); call(); ts.append(time.perf_counter() - t0)
+print(f"shard 1/{nsh} ({so[-1] / 1e6:.1f} MB): median {np.median(ts) * 1e3:.3f} ms, min {min(ts) * 1e3:.3f} ms, kernels {ps.kernel_ms():.3f} ms, "
+      f"{cells / np.median(ts) / 1e9:.0f} GCUPS", flush=True)
 # one call with the host and device timelines on stderr
-os.environ.pop("PSB_SCAN_HOST_FIRST_DIV", None); os.environ.pop("PSB_SCAN_HOST_FIRST_MB", None)
 os.environ["PSB_DEBUG_TIMING"] = "1"
 call()
