@@ -410,16 +410,21 @@ PSB_KERNEL void SW16_BOUNDS sw16_scan_kernel(Sw16Params p) {
                 const unsigned long long comp = comps[half];
                 const int sc = (int)(comp >> 26);
                 const int oid = p.out_map ? p.out_map[sid] : (int)sid;
+                // STRIP: a strip that lists an item stores the score -1 for both its subjects; the strips below leave
+                // such an item alone, so it is listed once and the re-run alone writes its results
+                const int osc = STRIP && p.merge ? p.score[oid] : 0;
+                if (osc < 0) continue;
                 if (overflow) {
                     const int slot_r = atomic_add(p.retry_count, 1);
                     p.retry[slot_r] = (int)sid + p.sid_base;
+                    if (STRIP) p.score[oid] = -1;
                 } else {
                     int er = sc == 0 ? 0 : (int)(0xffffu - (unsigned)((comp >> 10) & 0xffffu));
                     int eq = sc == 0 ? 0 : 1023 - (int)(comp & 1023u) + (STRIP ? p.row0 : 0);
                     int best_sc = sc;
                     if (STRIP && p.merge) {
                         // the strips above have stored their best: (score, smaller end_ref, smaller end_query) decides
-                        const int osc = p.score[oid], oer = p.end_ref[oid], oeq = p.end_query[oid];
+                        const int oer = p.end_ref[oid], oeq = p.end_query[oid];
                         if (osc > sc || (osc == sc && (sc == 0 || oer < er || (oer == er && oeq < eq)))) { best_sc = osc; er = oer; eq = oeq; }
                     }
                     p.score[oid] = best_sc; p.end_query[oid] = eq; p.end_ref[oid] = er;

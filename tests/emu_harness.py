@@ -149,8 +149,12 @@ def pack_db(subjects_mapped, bits):
     return np.array(words + [0], dtype=np.uint32), word_off, lens, np.array(perm, dtype=np.int32)
 
 
-def sw16(query, subjects, mat, open, gap, bits=5, nblocks=1):
-    """Run the emulated packed scan kernel: one query vs subjects.  Returns (outs, retry list)."""
+def sw16(query, subjects, mat, open, gap, bits=5, nblocks=1, ranges=None, raw=False):
+    """Run the emulated packed scan kernel: one query vs subjects.  Returns (outs, retry list): the caller ids of
+    the re-run list, sorted, one entry per push (a subject pushed twice is listed twice).
+    ranges: launches over sorted positions [(first, count), ...] as the engine's head and main launches
+    (sw16_subjects: pointers offset by `first`, sid_base = first); default one launch over everything.
+    raw: the re-run list as pushed instead (sorted positions, push order)."""
     assert lib().emu_sizeof_sw16() == C.sizeof(Sw16Params)
     mapper = mat.mapper.astype(np.uint8)
     qm = np.ascontiguousarray(mapper[np.asarray(query, dtype=np.uint8)])
@@ -167,13 +171,16 @@ def sw16(query, subjects, mat, open, gap, bits=5, nblocks=1):
     outs = {k: np.full(n, -777, dtype=np.int32) for k in ("score", "end_query", "end_ref")}
     retry = np.full(n + 2, -1, dtype=np.int32)
     retry_count = np.zeros(1, dtype=np.int32)
-    counter = np.zeros(1, dtype=np.int32)
-    p = Sw16Params(ptr(prof), mat.size + 1, len(qm), open, gap, mx.value, ptr(words), ptr(word_off), ptr(lens), bits, n,
-                   ptr(perm), ptr(outs["score"]), ptr(outs["end_query"]), ptr(outs["end_ref"]), ptr(retry),
-                   ptr(retry_count), 0, ptr(counter), None, None, None, 0, 0, 1, 65536)
-    rc = lib().emu_sw16(K.value, C.byref(p), nblocks)
-    assert rc == 0, (rc, K.value)
-    return outs, sorted(int(perm[i]) for i in retry[: retry_count[0]])
+    at = lambda a, first: C.c_void_p(a.ctypes.data + first * a.itemsize)
+    for first, count in ranges if ranges is not None else [(0, n)]:
+        counter = np.zeros(1, dtype=np.int32)
+        p = Sw16Params(ptr(prof), mat.size + 1, len(qm), open, gap, mx.value, ptr(words), at(word_off, first), at(lens, first), bits,
+                       count, at(perm, first), ptr(outs["score"]), ptr(outs["end_query"]), ptr(outs["end_ref"]), ptr(retry),
+                       ptr(retry_count), first, ptr(counter), None, None, None, 0, 0, 1, 65536)
+        rc = lib().emu_sw16(K.value, C.byref(p), nblocks)
+        assert rc == 0, (rc, K.value)
+    pushed = [int(i) for i in retry[: retry_count[0]]]
+    return outs, pushed if raw else sorted(int(perm[i]) for i in pushed)
 
 
 class Wave32Params(C.Structure):
@@ -295,7 +302,8 @@ def pairs16(qs, rs, mat, G, K, mode, open, gap, flags=(1, 1, 1, 1), what=0, nblo
 
 def sw16_strips(query, subjects, mat, open, gap, rows_per_strip, bits=5, nblocks=1):
     """The strip-wise scan of a long query (STRIP instantiations of csrc/kern_sw16.cuh, host loop as in
-    engine.cu): one sweep of the database per strip of `rows_per_strip` query rows.  Returns (outs, retry)."""
+    engine.cu): one sweep of the database per strip of `rows_per_strip` query rows.  Returns (outs, retry): the
+    caller ids of the re-run list, sorted, one entry per push."""
     mapper = mat.mapper.astype(np.uint8)
     qm = np.ascontiguousarray(mapper[np.asarray(query, dtype=np.uint8)])
     sm = [mapper[np.asarray(s, dtype=np.uint8)] for s in subjects]
@@ -311,4 +319,4 @@ def sw16_strips(query, subjects, mat, open, gap, rows_per_strip, bits=5, nblocks
                                bits, C.c_longlong(n), ptr(perm), ptr(outs["score"]), ptr(outs["end_query"]), ptr(outs["end_ref"]),
                                ptr(retry), ptr(retry_count), nblocks)
     assert rc == 0, rc
-    return outs, sorted(set(int(perm[i]) for i in retry[: retry_count[0]]))
+    return outs, sorted(int(perm[i]) for i in retry[: retry_count[0]])

@@ -96,3 +96,88 @@ def test_strip_wise_scan_ties_across_strips(oracle):
     for i, s in enumerate(subs):
         exp = oracle.align(q, s, mat, mode=2, open=5, gap=2)
         assert (outs["score"][i], outs["end_query"][i], outs["end_ref"][i]) == (exp["score"], exp["end_query"], exp["end_ref"]), i
+
+
+# ---- the re-run list: global sorted positions, the exact threshold, one entry per subject -------------------------
+def sw16_limit(mat, o):
+    """the packed kernel re-runs an item once a half's score reaches 32767 - open - max(S)"""
+    return 32767 - o - int(np.max(mat.table))
+
+
+def test_head_and_main_sub_ranges_push_global_positions(oracle):
+    # the engine's launches over sorted positions: subject 0 routed elsewhere (not launched), a head launch over
+    # positions 1..4 and a main launch over the rest; each launch's pointers start at its first position and its
+    # re-run pushes add sid_base = first.  Overflowing subjects sit in both launches.  Gaps as dear as the matrix
+    # allows (open + max(S) = 127) keep random subjects far below the limit: only the planted copies overflow.
+    mat = oracle.Matrix.create(b"ACGT", 100, -90)
+    o, e = 27, 27
+    q = psb_data.random_seq(41, 0, 400, protein=False)
+    lens = [900, 800, 700, 600, 520, 480, 450, 430, 410, 405, 300, 200, 150]   # distinct: the sort order is fixed
+    subs = [psb_data.random_seq(42, i, L, protein=False) for i, L in enumerate(lens)]
+    subs[2] = np.concatenate([psb_data.random_seq(43, 0, 300, protein=False), q])           # position 2: head
+    subs[7] = np.concatenate([q, psb_data.random_seq(43, 1, 30, protein=False)])            # position 7: main
+    caller = np.random.default_rng(44).permutation(len(subs))                                # caller order != sorted order
+    shuffled = [subs[i] for i in caller]
+    ranges = [(1, 4), (5, len(subs) - 5)]
+    outs, pushed = emu_harness.sw16(q, shuffled, mat, o, e, ranges=ranges, raw=True)
+    exp = [oracle.align(q, s, mat, mode=2, open=o, gap=e) for s in subs]
+    over = [x["score"] >= sw16_limit(mat, o) for x in exp]
+    assert over[2] and over[7] and sum(over) == 2
+    want = set()
+    for first, count in ranges:
+        for a in range(first, first + count, 2):
+            item = [s for s in (a, a + 1) if s < first + count]
+            if any(over[s] for s in item):
+                want.update(item)
+    assert sorted(pushed) == sorted(want) == [1, 2, 7, 8]
+    # sorted position s holds subs[s]; the caller passed it at index where(caller == s)
+    where = {int(c): i for i, c in enumerate(caller)}
+    for s in range(1, len(subs)):
+        if s in want:
+            continue
+        i = where[s]
+        assert (outs["score"][i], outs["end_query"][i], outs["end_ref"][i]) == (exp[s]["score"], exp[s]["end_query"], exp[s]["end_ref"]), s
+    assert outs["score"][where[0]] == -777   # the routed subject is no launch's
+
+
+def threshold_case(psb_data_seed, lq):
+    """DNA +91/-91: a 359-residue core scores 359 * 91 = 32669.  The query is the core, or the core with random
+    flanks (lq > 359); the first subject is the core itself, the others are shorter random subjects."""
+    core = psb_data.random_seq(psb_data_seed, 0, 359, protein=False)
+    pre = (lq - 359) // 3
+    q = np.concatenate([psb_data.random_seq(psb_data_seed, 1, pre, protein=False), core,
+                        psb_data.random_seq(psb_data_seed, 2, lq - 359 - pre, protein=False)])
+    subs = [core.copy()] + [psb_data.random_seq(psb_data_seed, 3 + i, L, protein=False) for i, L in enumerate((300, 200, 100))]
+    return q, subs
+
+
+@pytest.mark.parametrize("lq,rows", [(359, None), (600, 256)])
+def test_rerun_threshold_exactly(oracle, lq, rows):
+    # limit = 32767 - open - 91: open 6 puts the score one below it (exact in 16 bit), open 7 on it, open 8 above
+    mat = oracle.Matrix.create(b"ACGT", 91, -91)
+    q, subs = threshold_case(31, lq)
+    for o, rerun in ((6, False), (7, True), (8, True)):
+        exp = [oracle.align(q, s, mat, mode=2, open=o, gap=1) for s in subs]
+        assert exp[0]["score"] == 32669 and sw16_limit(mat, o) == 32669 + 1 - (o - 6)
+        if rows is None:
+            outs, retry = emu_harness.sw16(q, subs, mat, o, 1)
+        else:
+            outs, retry = emu_harness.sw16_strips(q, subs, mat, o, 1, rows)
+        assert retry == ([0, 1] if rerun else []), o
+        for i, s in enumerate(subs):
+            if i not in retry:
+                assert (outs["score"][i], outs["end_query"][i], outs["end_ref"][i]) == (exp[i]["score"], exp[i]["end_query"], exp[i]["end_ref"]), (o, i)
+
+
+def test_strip_wise_rerun_lists_a_subject_once(oracle):
+    # a 768-residue query in three strips of 256 rows; its copy overflows in strips 2 and 3.  Each subject of the
+    # item goes on the re-run list once, not once per strip in which it is still over the limit.
+    mat = oracle.Matrix.create(b"ACGT", 100, -90)
+    q = psb_data.random_seq(9, 0, 768, protein=False)
+    subs = [q.copy(), psb_data.random_seq(9, 1, 500, protein=False), psb_data.random_seq(9, 2, 60, protein=False),
+            psb_data.random_seq(9, 3, 50, protein=False)]
+    outs, retry = emu_harness.sw16_strips(q, subs, mat, 5, 2, 256)
+    assert retry == [0, 1]
+    for i in (2, 3):
+        exp = oracle.align(q, subs[i], mat, mode=2, open=5, gap=2)
+        assert (outs["score"][i], outs["end_query"][i], outs["end_ref"][i]) == (exp["score"], exp["end_query"], exp["end_ref"]), i
