@@ -1,6 +1,6 @@
 // pairs16_host.h -- launch interface of the packed 16-bit many-pairs kernels (pairs16.cu), kept in its own
-// translation unit so that its ~50 template instantiations compile beside engine.cu, not after it; and the
-// persistent-grid launch both translation units use.
+// translation unit so that its ~50 template instantiations compile beside the other kernel files, not after them; and
+// the persistent-grid launch they all use.
 #pragma once
 #include <cuda_runtime.h>
 

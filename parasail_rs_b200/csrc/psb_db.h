@@ -1,5 +1,5 @@
-// psb_db.h -- the resident database object shared by engine.cu (construction, scans) and db_io.cu
-// (FASTA reader, on-disk packed format).
+// psb_db.h -- the resident database object shared by the engine (db.cu builds it, scan.cu and host_scan.cu scan it)
+// and db_io.cu (FASTA reader, on-disk packed format).
 #pragma once
 #include <cuda_runtime.h>
 
@@ -31,6 +31,6 @@ namespace psb {
 // bits per residue of a packed database for an alphabet of `size` letters (pad / wildcard codes are < size)
 inline int db_bits_for(int size) { return size <= 4 ? 2 : (size <= 8 ? 3 : 5); }
 inline int db_residues_per_word(int bits) { return bits == 2 ? 16 : (bits == 3 ? 10 : 6); }
-// engine.cu: binds the calling thread's context (device, stream); PSB_OK or an error code
+// db.cu: binds the calling thread's context (device, stream); PSB_OK or an error code
 int db_io_ensure_ctx(int *device, cudaStream_t *stream);
 }  // namespace psb

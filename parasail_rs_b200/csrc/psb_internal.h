@@ -116,7 +116,7 @@ struct parasail_profile {
 
 namespace psb {
 
-// ---- engine (engine.cu) --------------------------------------------------------------------
+// ---- engine (pairs.cu, ctx.cu, scan.cu) -------------------------------------------------------
 struct PairsRequest {
     FnConfig cfg;
     const HostMatrix *matrix = nullptr;

@@ -1,6 +1,6 @@
 // result.cpp -- parasail_result_t and its getters, CIGAR and traceback strings, as used by
 // parasail-rs's Alignment [REF src/alignment/mod.rs:54-504].  Single-pair results are n = 1
-// batches of the GPU path (engine.cu); this file only reads what the device produced.
+// batches of the GPU path (pairs.cu); this file only reads what the device produced.
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>

@@ -201,7 +201,7 @@ extern "C" int emu_pairs16(int G, int K, int mode, int s1_beg, int s1_end, int s
     return 0;
 }
 
-// ---- strip-wise scan of a long query (STRIP instantiations of the scan kernel), host loop as in engine.cu ----
+// ---- strip-wise scan of a long query (STRIP instantiations of the scan kernel), host loop as in scan.cu ----
 extern "C" int emu_sw16_strips(const uint8_t *mapped_query, int lq, const int *table, int size, int open, int gap, int rows_per_strip,
                                const unsigned *words, const long long *word_off, const int *len, int bits, long long n,
                                const int *out_map, int *score, int *end_query, int *end_ref, int *retry, int *retry_count, int nblocks) {

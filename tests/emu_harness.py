@@ -302,7 +302,7 @@ def pairs16(qs, rs, mat, G, K, mode, open, gap, flags=(1, 1, 1, 1), what=0, nblo
 
 def sw16_strips(query, subjects, mat, open, gap, rows_per_strip, bits=5, nblocks=1):
     """The strip-wise scan of a long query (STRIP instantiations of csrc/kern_sw16.cuh, host loop as in
-    engine.cu): one sweep of the database per strip of `rows_per_strip` query rows.  Returns (outs, retry): the
+    scan.cu): one sweep of the database per strip of `rows_per_strip` query rows.  Returns (outs, retry): the
     caller ids of the re-run list, sorted, one entry per push."""
     mapper = mat.mapper.astype(np.uint8)
     qm = np.ascontiguousarray(mapper[np.asarray(query, dtype=np.uint8)])
