@@ -328,6 +328,24 @@ int psb_db_align(const char *fn_name, const parasail_profile_t *profile, int ope
 /* subject `id` of a resident database as matrix column indices (what the kernels align): writes min(len, cap)
  * codes to `codes`, returns the subject's length, or a negative PSB_E* code */
 int64_t psb_db_subject(const psb_db_t *db, int64_t id, uint8_t *codes, int64_t cap);
+/* many query profiles against a resident database in one call, each query's best hits chosen on the GPU.  Let
+ * kk = min(k, psb_db_count(db)).  The batch has nq * kk rows: row q*kk + r holds query q's r-th best subject, and
+ * ids_out[q*kk + r] (nq * kk entries, allocated by the caller) is that subject's caller-order id.
+ *   - Which subjects: per query, those of a score-only scan under fn_name without _trace and _stats, ordered by score
+ *     descending, then by smaller id -- psb_batch_topk applied to that query's psb_scan.  Only the kk rows of each
+ *     query leave the device.
+ *   - Fields: with _trace or _stats, the rows are the alignments of those hits under fn_name, equal field for field
+ *     (CIGAR included) to psb_db_align(fn_name, profiles[q], ..., ids of q, kk); the hits of all queries go through
+ *     one pairs pass per group of queries with equal matrices (a PSSM profile has a pass of its own).  With a
+ *     score-only name, score / end_query / end_ref are the scan's own values and no second pass runs.  Explicit
+ *     _8 / _16 widths flag and zero saturated results as psb_scan and psb_db_align do.
+ *   - n_retried: the sum over queries of what psb_scan reports; cells: the nq scans plus the alignment pass.
+ *     psb_last_kernel_ms / psb_last_launches cover the whole call.
+ *   - PSB_EINVAL: not a profile name, nq <= 0, k <= 0, a NULL argument, a NULL profiles[q] or a profile with
+ *     another alphabet than the database (the message names q).  PSB_EUNSUPPORTED: _table / _rowcol, or
+ *     nq * kk > 2^31 - 1.  Every check runs before any device work. */
+int psb_db_search(const char *fn_name, const parasail_profile_t *const *profiles, int64_t nq, int open, int gap,
+                  const psb_db_t *db, int k, int64_t *ids_out, psb_batch_t **out);
 /* the same scan for a database that lives in HOST memory (pinned or pageable): the residues are cut
  * into pieces whose upload, device-side packing and scan are pipelined on two streams, so the
  * host-to-device copy hides under the kernels.  Nothing stays resident afterwards. */

@@ -715,17 +715,31 @@ class Aligner:
 
     def search(self, database, k):
         """scan the whole Database score-only, keep the k best subjects (ties by smaller id) and align those with this
-        aligner's own function: returns (ids, BatchResult) with row i belonging to ids[i]"""
+        aligner's own function: returns (ids, BatchResult) with row i belonging to ids[i].  The one-query case of
+        search_many."""
         if self._profile.is_null():
             raise Panic("search() needs an aligner built with .profile(...)")
-        score_only = self.fn_name.replace("_trace", "").replace("_stats", "")
+        ids, hits = self.search_many(database, [self._profile], k)
+        return ids[0], hits
+
+    def search_many(self, database, profiles, k):
+        """search() for several query Profiles in one call (psb_db_search), with this aligner's function name, gaps
+        and width: each query's scan, and the choice of its k best subjects, run on the GPU; one alignment pass then
+        serves the hits of every query.  Returns (ids, BatchResult): ids has shape (len(profiles), kk) with
+        kk = min(k, database.n), and row q * kk + r of the batch belongs to ids[q, r]."""
+        if self._profile.is_null():
+            raise Panic("search_many() needs an aligner built with .profile(...)")
+        profiles = list(profiles)
+        nq = len(profiles)
+        kk = min(int(k), database.n) if nq and k > 0 else 0
+        ptrs = (C.c_void_p * max(nq, 1))(*[p.inner for p in profiles])
+        ids = np.zeros((nq, kk), dtype=np.int64)
         out = C.POINTER(CBatch)()
-        rc_ = lib().psb_scan(score_only.encode(), self._profile.inner, self.gap_open, self.gap_extend, database.inner,
-                             C.byref(out))
+        rc_ = lib().psb_db_search(self.fn_name.encode(), ptrs, nq, self.gap_open, self.gap_extend, database.inner, int(k),
+                                  ids.ctypes.data_as(C.c_void_p), C.byref(out))
         if rc_ != 0:
-            raise DeviceError(f"psb_scan failed ({rc_}): {last_error()}")
-        ids, _ = BatchResult(out).topk(k)
-        return ids, self.align_subjects(database, ids)
+            raise DeviceError(f"psb_db_search failed ({rc_}): {last_error()}")
+        return ids, BatchResult(out)
 
 
 def _scan_host(self, subjects):

@@ -68,7 +68,7 @@ ALL_SYMBOLS = (
      "parasail_traceback_generic", "parasail_nw_banded", "parasail_ssw", "parasail_ssw_init", "parasail_result_ssw_free",
      "psb_last_error", "psb_device_count", "psb_set_device", "psb_set_stream", "psb_synchronize", "psb_batch_free",
      "psb_align_pairs", "psb_align_pairs_banded", "psb_db_create", "psb_db_count", "psb_db_residues", "psb_db_device_bytes", "psb_db_free",
-     "psb_scan", "psb_db_align", "psb_db_subject", "psb_scan_host", "psb_batch_topk", "psb_shard_plan", "psb_last_kernel_ms", "psb_last_launches", "psb_version"]
+     "psb_scan", "psb_db_align", "psb_db_search", "psb_db_subject", "psb_scan_host", "psb_batch_topk", "psb_shard_plan", "psb_last_kernel_ms", "psb_last_launches", "psb_version"]
     + PROFILE_CREATORS
     + [f"parasail_result_get_{g}" for g in RESULT_INT_GETTERS + RESULT_ARRAY_GETTERS]
     + [f"parasail_result_is_{p}" for p in RESULT_PREDICATES])
@@ -196,6 +196,9 @@ def lib():
     L.psb_db_align.restype = C.c_int
     L.psb_db_align.argtypes = [C.c_char_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64,
                                C.POINTER(C.POINTER(CBatch))]
+    L.psb_db_search.restype = C.c_int
+    L.psb_db_search.argtypes = [C.c_char_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
+                                C.POINTER(C.POINTER(CBatch))]
     L.psb_db_subject.restype = C.c_int64
     L.psb_db_subject.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64]
     L.psb_scan_host.restype = C.c_int

@@ -10,6 +10,7 @@
 //   scan.cu       a resident profile against a resident database: psb_scan (C2), psb_db_align (kern_sw16.cuh), and
 //                 the one-warp-per-pair 32-bit kernels (kern_gotoh32.cuh)
 //   host_scan.cu  the scan of a database in host memory: psb_scan_host, psb_scan_box
+//   search.cu     many profiles against a resident database: psb_db_search, its selection kernels (kern_topk.cuh)
 //   pairs16.cu    the packed 16-bit many-pairs kernels (pairs16_host.h)
 //
 // Each kernel (cub's included) is instantiated in exactly one of them; another file that launches it calls a launcher
@@ -361,10 +362,13 @@ bool sw16_wanted(const FnConfig &cfg);
 // the query side of a scan, queued while the compute stream is idle: the profile's device copy and packed form
 int prepare_query(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap);
 int scan_check(const char *who, const char *fn_name, const parasail_profile_t *profile, FnConfig *cfg);
+// a profile run against a resident database: the calling thread's device holds it, and both use the same alphabet
+int profile_db_check(const char *who, const parasail_profile_t *profile, const psb_db *db);
 
 // one scan of a resident database, in two halves so that psb_scan_host can do host work for the next
 // piece while this one runs: scan_enqueue issues the kernels and the device->host copies of the
-// per-subject results (to hosts[k] + host_base); scan_finish waits for them.
+// per-subject results (to hosts[k] + host_base); scan_finish waits for them.  With hosts == nullptr the
+// results stay in job.d_out only (psb_db_search selects from them on the device).
 struct ScanJob {
     DevMem d_out[6];
     int64_t retried = 0;

@@ -552,7 +552,7 @@ int scan_enqueue(ScanJob &job, const FnConfig &cfg, const parasail_profile *prof
     else rc = scan_general(cfg, profile, dp, open, gap, db, nullptr, 0, nullptr, outp);
     if (rc != PSB_OK) { cudaStreamSynchronize(c.stream); return rc; }
     PSB_CUDA(cudaEventRecord(job.ev1, c.stream));
-    for (int k = 0; k < nout; ++k)
+    for (int k = 0; k < nout && hosts; ++k)
         PSB_CUDA(cudaMemcpyAsync(hosts[k] + host_base, job.d_out[k].p, (size_t)db->n * sizeof(int), cudaMemcpyDeviceToHost, c.stream));
     PSB_CUDA(cudaEventCreateWithFlags(&job.done, cudaEventDisableTiming));
     PSB_CUDA(cudaEventRecord(job.done, c.stream));
@@ -594,7 +594,7 @@ int scan_check(const char *who, const char *fn_name, const parasail_profile_t *p
     return PSB_OK;
 }
 // a profile run against a resident database: the calling thread's device holds it, and both use the same alphabet
-static int profile_db_check(const char *who, const parasail_profile_t *profile, const psb_db *db) {
+int profile_db_check(const char *who, const parasail_profile_t *profile, const psb_db *db) {
     PSB_TRY(ensure_ctx());
     if (db->device != g_ctx.device) { set_error(std::string(who) + ": database lives on another device"); return PSB_EINVAL; }
     if (profile->matrix.size != db->msize || std::memcmp(profile->matrix.mapper, db->mapper, 256) != 0) {
