@@ -357,6 +357,43 @@ int psb_scan_host(const char *fn_name, const parasail_profile_t *profile, int op
  * n_gpus <= 0 means every visible device.  No collective is involved. */
 int psb_scan_box(const char *fn_name, const parasail_profile_t *profile, int open, int gap, const uint8_t *cat,
                  const int64_t *off, int64_t n, int n_gpus, psb_batch_t **out);
+/* a resident database over the devices of the box, driven from one process.  The subjects are cut into contiguous
+ * caller-id ranges of equal residue count (the cut of psb_scan_box); shard s is an ordinary psb_db resident on
+ * devices[s], built, scanned and aligned by that device's worker thread.  devices may repeat (the shards of one device
+ * are built and scanned one after another); devices == NULL: one shard per visible device, n_shards ignored.  There
+ * are fewer shards than asked when there are too few subjects to cut.  NULL + psb_last_error() on failure: the
+ * checks of psb_db_create, n_shards <= 0, a device ordinal out of range, no device, or a shard's build
+ * ("(shard s, device d): ..."). */
+typedef struct psb_box_db psb_box_db_t;
+psb_box_db_t *psb_box_db_create(const uint8_t *cat, const int64_t *off, int64_t n, const parasail_matrix_t *matrix,
+                                const int *devices, int n_shards);
+int64_t psb_box_db_count(const psb_box_db_t *db);
+/* the number of shards; fills first[0..shards] (first caller id of each shard, then n) and device[0..shards-1] if
+ * non-NULL */
+int psb_box_db_shards(const psb_box_db_t *db, int64_t *first, int *device);
+int64_t psb_box_db_subject(const psb_box_db_t *db, int64_t id, uint8_t *codes, int64_t cap);   /* as psb_db_subject */
+void psb_box_db_free(psb_box_db_t *db);
+/* psb_scan, psb_db_align and psb_db_search on a box database: the same ids and rows, field for field, as the
+ * single-device function on a psb_db built from the same arrays.  Each shard's work runs on its device's worker, the
+ * devices side by side.
+ *   - psb_box_scan writes each shard's results at its caller-order range of the batch.
+ *   - psb_box_align aligns each id on the device that holds it and gathers the rows in the order of `ids`.
+ *   - psb_box_search selects each query's min(k, n_s) best subjects on every shard s, merges them per query by the
+ *     same rule (score descending, then smaller caller id) and keeps kk = min(k, n): every global top-kk subject is
+ *     among its own shard's best, so the merge is exact.  With _trace / _stats each kept hit is then aligned on the
+ *     device that holds it, one pairs pass per device and matrix group for all queries.
+ *   - n_retried is the sum over shards.  It can differ from the single-device value: a 16-bit re-run takes the
+ *     subject's word partner along, and the partners depend on the cut.
+ *   - psb_last_kernel_ms is the slowest device's kernel time, psb_last_launches the sum over devices.
+ *   - Errors: the codes and messages of the single-device function under the new name; a failure on a device reads
+ *     "(shard s, device d): ...".  Every check runs before any device work.  Two host threads may call on one box
+ *     database at once. */
+int psb_box_scan(const char *fn_name, const parasail_profile_t *profile, int open, int gap, const psb_box_db_t *db,
+                 psb_batch_t **out);
+int psb_box_align(const char *fn_name, const parasail_profile_t *profile, int open, int gap, const psb_box_db_t *db,
+                  const int64_t *ids, int64_t n, psb_batch_t **out);
+int psb_box_search(const char *fn_name, const parasail_profile_t *const *profiles, int64_t nq, int open, int gap,
+                   const psb_box_db_t *db, int k, int64_t *ids_out, psb_batch_t **out);
 /* indices (caller order) of the k best scores of a scan, ties by smaller index; host-side merge */
 int psb_batch_topk(const psb_batch_t *batch, int k, int64_t *idx_out, int *score_out);
 

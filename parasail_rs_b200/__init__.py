@@ -18,7 +18,7 @@ import numpy as np
 from . import _lib
 from ._lib import CBatch, CMatrix, CResult, FUNCTION_T, PFUNCTION_T, last_error, lib
 
-__all__ = ["Aligner", "AlignerBuilder", "Alignment", "Matrix", "Profile", "ProfileBuilder", "Database", "BatchResult",
+__all__ = ["Aligner", "AlignerBuilder", "Alignment", "Matrix", "Profile", "ProfileBuilder", "Database", "BoxDatabase", "BatchResult",
            "Traceback", "TraceFlags", "Error", "Panic"]
 
 
@@ -488,6 +488,55 @@ class Database:
             pass
 
 
+class BoxDatabase:
+    """a subject database sharded over the GPUs of this box, driven from this process (psb_box_db_create): contiguous
+    caller-id ranges of equal residue count, shard s resident on devices[s] (devices may repeat; None: one shard per
+    visible GPU).  Aligner.scan, align_subjects, search and search_many take it in place of a Database and return
+    the same rows."""
+
+    def __init__(self, subjects, matrix, devices=None):
+        self._keep = matrix
+        self.inner = None
+        cat, off = _concat(subjects)
+        devs = None if devices is None else (C.c_int * max(len(devices), 1))(*devices)
+        self.inner = lib().psb_box_db_create(cat.ctypes.data_as(C.c_void_p), off.ctypes.data_as(C.c_void_p), len(off) - 1,
+                                             matrix.inner, devs, 0 if devices is None else len(devices))
+        if not self.inner:
+            raise DeviceError(last_error())
+        self.n = int(lib().psb_box_db_count(self.inner))
+        self.residues = int(off[-1] - off[0])
+        S = int(lib().psb_box_db_shards(self.inner, None, None))
+        first = np.zeros(S + 1, dtype=np.int64)
+        dev = np.zeros(S, dtype=np.int32)
+        lib().psb_box_db_shards(self.inner, first.ctypes.data_as(C.c_void_p), dev.ctypes.data_as(C.c_void_p))
+        self.shards = [(int(first[s]), int(first[s + 1]), int(dev[s])) for s in range(S)]
+
+    def subject(self, i):
+        """subject `i` (caller order), as Database.subject"""
+        n = int(lib().psb_box_db_subject(self.inner, int(i), None, 0))
+        if n < 0:
+            raise DeviceError(f"psb_box_db_subject failed ({n}): {last_error()}")
+        codes = np.zeros(n, dtype=np.uint8)
+        rc = int(lib().psb_box_db_subject(self.inner, int(i), codes.ctypes.data_as(C.c_void_p), n))
+        if rc < 0:
+            raise DeviceError(f"psb_box_db_subject failed ({rc}): {last_error()}")
+        alphabet = np.frombuffer(self._keep.inner.contents.alphabet, dtype=np.uint8)
+        return alphabet[codes].tobytes()
+
+    def __del__(self):
+        try:
+            if self.inner:
+                lib().psb_box_db_free(self.inner)
+        except Exception:
+            pass
+
+
+def _on(database, single, box):
+    """the C entry point for a Database or a BoxDatabase"""
+    name = box if isinstance(database, BoxDatabase) else single
+    return name, getattr(lib(), name)
+
+
 # ---- Aligner [REF src/aligner/mod.rs:67-535] -----------------------------------------------------
 class AlignerBuilder:
     def __init__(self):
@@ -685,18 +734,19 @@ class Aligner:
         return BatchResult(out)
 
     def scan(self, database):
-        """the aligner's resident profile against a resident Database (psb_scan)"""
+        """the aligner's resident profile against a resident Database or BoxDatabase (psb_scan, psb_box_scan)"""
         if self._profile.is_null():
             raise Panic("scan() needs an aligner built with .profile(...)")
         out = C.POINTER(CBatch)()
-        rc_ = lib().psb_scan(self.fn_name.encode(), self._profile.inner, self.gap_open, self.gap_extend, database.inner,
-                             C.byref(out))
+        name, fn = _on(database, "psb_scan", "psb_box_scan")
+        rc_ = fn(self.fn_name.encode(), self._profile.inner, self.gap_open, self.gap_extend, database.inner, C.byref(out))
         if rc_ != 0:
-            raise DeviceError(f"psb_scan failed ({rc_}): {last_error()}")
+            raise DeviceError(f"{name} failed ({rc_}): {last_error()}")
         return BatchResult(out)
 
     def align_subjects(self, database, ids=None):
-        """the aligner's profile against selected subjects of a resident Database (psb_db_align): row i belongs to
+        """the aligner's profile against selected subjects of a resident Database or BoxDatabase (psb_db_align,
+        psb_box_align): row i belongs to
         ids[i] (caller-order ids, any order, repeats allowed); ids=None aligns every subject.  With use_trace()
         the rows carry CIGARs and begin coordinates, with a stats profile matches/similar/length."""
         if self._profile.is_null():
@@ -707,10 +757,10 @@ class Aligner:
             ids = np.ascontiguousarray(ids, dtype=np.int64)
             ptr, n = ids.ctypes.data_as(C.c_void_p), len(ids)
         out = C.POINTER(CBatch)()
-        rc_ = lib().psb_db_align(self.fn_name.encode(), self._profile.inner, self.gap_open, self.gap_extend, database.inner,
-                                 ptr, n, C.byref(out))
+        name, fn = _on(database, "psb_db_align", "psb_box_align")
+        rc_ = fn(self.fn_name.encode(), self._profile.inner, self.gap_open, self.gap_extend, database.inner, ptr, n, C.byref(out))
         if rc_ != 0:
-            raise DeviceError(f"psb_db_align failed ({rc_}): {last_error()}")
+            raise DeviceError(f"{name} failed ({rc_}): {last_error()}")
         return BatchResult(out)
 
     def search(self, database, k):
@@ -723,7 +773,8 @@ class Aligner:
         return ids[0], hits
 
     def search_many(self, database, profiles, k):
-        """search() for several query Profiles in one call (psb_db_search), with this aligner's function name, gaps
+        """search() for several query Profiles in one call (psb_db_search, or psb_box_search for a BoxDatabase, whose
+        rows are the same), with this aligner's function name, gaps
         and width: each query's scan, and the choice of its k best subjects, run on the GPU; one alignment pass then
         serves the hits of every query.  Returns (ids, BatchResult): ids has shape (len(profiles), kk) with
         kk = min(k, database.n), and row q * kk + r of the batch belongs to ids[q, r]."""
@@ -735,10 +786,11 @@ class Aligner:
         ptrs = (C.c_void_p * max(nq, 1))(*[p.inner for p in profiles])
         ids = np.zeros((nq, kk), dtype=np.int64)
         out = C.POINTER(CBatch)()
-        rc_ = lib().psb_db_search(self.fn_name.encode(), ptrs, nq, self.gap_open, self.gap_extend, database.inner, int(k),
-                                  ids.ctypes.data_as(C.c_void_p), C.byref(out))
+        name, fn = _on(database, "psb_db_search", "psb_box_search")
+        rc_ = fn(self.fn_name.encode(), ptrs, nq, self.gap_open, self.gap_extend, database.inner, int(k), ids.ctypes.data_as(C.c_void_p),
+                 C.byref(out))
         if rc_ != 0:
-            raise DeviceError(f"psb_db_search failed ({rc_}): {last_error()}")
+            raise DeviceError(f"{name} failed ({rc_}): {last_error()}")
         return ids, BatchResult(out)
 
 

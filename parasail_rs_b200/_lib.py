@@ -68,7 +68,8 @@ ALL_SYMBOLS = (
      "parasail_traceback_generic", "parasail_nw_banded", "parasail_ssw", "parasail_ssw_init", "parasail_result_ssw_free",
      "psb_last_error", "psb_device_count", "psb_set_device", "psb_set_stream", "psb_synchronize", "psb_batch_free",
      "psb_align_pairs", "psb_align_pairs_banded", "psb_db_create", "psb_db_count", "psb_db_residues", "psb_db_device_bytes", "psb_db_free",
-     "psb_scan", "psb_db_align", "psb_db_search", "psb_db_subject", "psb_scan_host", "psb_batch_topk", "psb_shard_plan", "psb_last_kernel_ms", "psb_last_launches", "psb_version"]
+     "psb_scan", "psb_db_align", "psb_db_search", "psb_db_subject", "psb_scan_host", "psb_box_db_create", "psb_box_db_count",
+     "psb_box_db_shards", "psb_box_db_subject", "psb_box_db_free", "psb_box_scan", "psb_box_align", "psb_box_search", "psb_batch_topk", "psb_shard_plan", "psb_last_kernel_ms", "psb_last_launches", "psb_version"]
     + PROFILE_CREATORS
     + [f"parasail_result_get_{g}" for g in RESULT_INT_GETTERS + RESULT_ARRAY_GETTERS]
     + [f"parasail_result_is_{p}" for p in RESULT_PREDICATES])
@@ -207,6 +208,24 @@ def lib():
     L.psb_scan_box.restype = C.c_int
     L.psb_scan_box.argtypes = [C.c_char_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
                                C.POINTER(C.POINTER(CBatch))]
+    L.psb_box_db_create.restype = C.c_void_p
+    L.psb_box_db_create.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(CMatrix), C.c_void_p, C.c_int]
+    L.psb_box_db_count.restype = C.c_int64
+    L.psb_box_db_count.argtypes = [C.c_void_p]
+    L.psb_box_db_shards.restype = C.c_int
+    L.psb_box_db_shards.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+    L.psb_box_db_subject.restype = C.c_int64
+    L.psb_box_db_subject.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64]
+    L.psb_box_db_free.restype = None
+    L.psb_box_db_free.argtypes = [C.c_void_p]
+    L.psb_box_scan.restype = C.c_int
+    L.psb_box_scan.argtypes = [C.c_char_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.POINTER(CBatch))]
+    L.psb_box_align.restype = C.c_int
+    L.psb_box_align.argtypes = [C.c_char_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int64,
+                                C.POINTER(C.POINTER(CBatch))]
+    L.psb_box_search.restype = C.c_int
+    L.psb_box_search.argtypes = [C.c_char_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
+                                 C.POINTER(C.POINTER(CBatch))]
     L.psb_batch_topk.restype = C.c_int
     L.psb_batch_topk.argtypes = [C.POINTER(CBatch), C.c_int, C.c_void_p, C.c_void_p]
     L.psb_shard_plan.restype = C.c_int

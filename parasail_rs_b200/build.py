@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libparasail_b200.so")
-SOURCES = ["scan.cu", "pairs.cu", "pairs16.cu", "wave32.cu", "db.cu", "host_scan.cu", "search.cu", "ctx.cu", "db_io.cu", "matrix.cpp", "fn_name.cpp",
+SOURCES = ["scan.cu", "pairs.cu", "pairs16.cu", "wave32.cu", "db.cu", "host_scan.cu", "search.cu", "box.cu", "ctx.cu", "db_io.cu", "matrix.cpp", "fn_name.cpp",
            "result.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC"]
 

@@ -139,6 +139,17 @@ void pinned_free(void *p, size_t bytes) {
     else cudaFreeHost(p);
 }
 
+std::vector<int64_t> cut_subjects(const int64_t *off, int64_t n, const std::vector<int64_t> &targets) {
+    std::vector<int64_t> cut(1, 0);
+    for (const int64_t t : targets) {
+        const int64_t at = std::max<int64_t>(std::lower_bound(off, off + n + 1, off[0] + t) - off, cut.back() + 1);
+        if (at >= n) break;
+        cut.push_back(at);
+    }
+    cut.push_back(n);
+    return cut;
+}
+
 // a batch's per-pair result arrays in the order the kernels' outputs use (score, end_query, end_ref, then the statistics)
 std::array<int *, 6> batch_outputs(psb_batch_t *b) { return {b->score, b->end_query, b->end_ref, b->matches, b->similar, b->length}; }
 // the length of sequence i of a concatenation
@@ -255,6 +266,16 @@ BoxWorker *start_worker(int device) {
     w->th = std::thread([w] { w->loop(); });
     w->th.detach();
     return w;
+}
+
+// the per-device workers of psb_scan_box and of the box database (box.cu)
+static std::mutex g_box_mu;
+static std::vector<BoxWorker *> g_box;   // index = device; never destroyed (the threads live as long as the process)
+BoxWorker *box_worker(int device) {
+    std::lock_guard<std::mutex> lk(g_box_mu);
+    if ((int)g_box.size() <= device) g_box.resize(device + 1, nullptr);
+    if (!g_box[device]) g_box[device] = start_worker(device);
+    return g_box[device];
 }
 
 // the lanes of the pairs pass (run_pairs_lanes, pairs.cu)

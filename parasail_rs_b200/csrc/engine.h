@@ -11,6 +11,8 @@
 //                 the one-warp-per-pair 32-bit kernels (kern_gotoh32.cuh)
 //   host_scan.cu  the scan of a database in host memory: psb_scan_host, psb_scan_box
 //   search.cu     many profiles against a resident database: psb_db_search, its selection kernels (kern_topk.cuh)
+//   box.cu        a resident database sharded over the devices of the box: psb_box_db_* and psb_box_scan / _align /
+//                 _search, each shard's work on its device's worker
 //   pairs16.cu    the packed 16-bit many-pairs kernels (pairs16_host.h)
 //
 // Each kernel (cub's included) is instantiated in exactly one of them; another file that launches it calls a launcher
@@ -151,6 +153,10 @@ size_t device_mem_available();
 psb_batch_t *new_batch(int64_t n, const FnConfig &cfg);
 std::array<int *, 6> batch_outputs(psb_batch_t *b);
 int span(const int64_t *off, int64_t i);
+// subject cuts of the database off[0 .. n] at residue targets (counted from off[0], increasing): 0, then for each target
+// the first subject boundary at or past it but at least one subject past the previous cut, then n.  A cut that would
+// leave no subject after it ends the list.  (psb_scan_box's ranges, its pieces, and the box database's shards)
+std::vector<int64_t> cut_subjects(const int64_t *off, int64_t n, const std::vector<int64_t> &targets);
 void fill_lut(unsigned *lut, const uint8_t *mapper);
 
 struct BatchImpl {
@@ -361,9 +367,13 @@ struct StreamMarks {
 bool sw16_wanted(const FnConfig &cfg);
 // the query side of a scan, queued while the compute stream is idle: the profile's device copy and packed form
 int prepare_query(const FnConfig &cfg, const parasail_profile_t *profile, int open, int gap);
+// a profile function name and a profile; scan_check adds: no traceback, table or row/column outputs
+int profile_fn_check(const char *who, const char *fn_name, const parasail_profile_t *profile, FnConfig *cfg);
 int scan_check(const char *who, const char *fn_name, const parasail_profile_t *profile, FnConfig *cfg);
 // a profile run against a resident database: the calling thread's device holds it, and both use the same alphabet
 int profile_db_check(const char *who, const parasail_profile_t *profile, const psb_db *db);
+// the alphabet half of profile_db_check, which needs no device
+int profile_alphabet_check(const char *who, const parasail_profile_t *profile, const psb_db *db);
 
 // one scan of a resident database, in two halves so that psb_scan_host can do host work for the next
 // piece while this one runs: scan_enqueue issues the kernels and the device->host copies of the
@@ -404,6 +414,23 @@ int scan_batch_done(const FnConfig &cfg, const parasail_profile_t *profile, int 
     return PSB_OK;
 }
 
+// ---- search.cu: the two halves of psb_db_search, which the box database runs per shard -------------------------
+// (a) per query q, the kk best subjects of `db` under the score-only form of `cfg`, in the order of psb_batch_topk:
+// row q * kk + r of each plane.  Sets the thread's counters to the scans' and selections' device time and launches.
+struct SearchHits {
+    std::vector<int> id, score, end_query, end_ref, saturated;
+    int64_t retried = 0;   // the scans' re-runs at 32 bit
+};
+int search_select(const FnConfig &cfg, const parasail_profile_t *const *profiles, int64_t nq, int open, int gap, psb_db *db, int64_t kk,
+                  SearchHits *hits);
+// (b) the alignments of n rows, row i being query row_q[i] against subject row_id[i] of `db` (caller order): one pairs
+// pass per group of queries with equal matrices, gathered in row order.  The rows of one query are psb_db_align's
+// request exactly.  Adds the passes' device time and launches to the thread's counters.
+int align_rows(const FnConfig &cfg, const parasail_profile_t *const *profiles, int64_t nq, const int64_t *row_q, const int64_t *row_id,
+               int64_t n, int open, int gap, psb_db *db, psb_batch_t **out);
+// the rows of the batches `gb` (`src[row]` = (batch, row in it)) gathered into one batch in row order; cells summed
+int gather_rows(const FnConfig &cfg, const std::vector<psb_batch_t *> &gb, const std::vector<std::pair<int, int64_t>> &src, psb_batch_t **out);
+
 // one piece of a host scan (host_scan.cu): its uploads and packed shard, and its scan.  Destroying it gives the packed
 // shard, the staging blocks and the result arrays back; the owner has synchronised the streams that used them.
 struct HostPiece {
@@ -412,7 +439,7 @@ struct HostPiece {
     ~HostPiece() { psb_db_free(build.db); }
 };
 
-// ---- resident worker threads: one per device for psb_scan_box, and the lanes of the pairs pass.  The thread keeps
+// ---- resident worker threads: one per device for psb_scan_box and the box database, and the lanes of the pairs pass.  The thread keeps
 // its context (streams, memory pool, staging blocks) warm across calls --------------------------------------------
 struct BoxWorker {
     int device = 0;
@@ -454,5 +481,7 @@ struct BoxWorker {
 BoxWorker *start_worker(int device);
 // the worker of lane `lane` of the pairs pass on `device`, started on first use
 BoxWorker *pair_lane(int device, int lane);
+// the worker of `device` that psb_scan_box and the box database run on, started on first use
+BoxWorker *box_worker(int device);
 
 }  // namespace psb

@@ -7,7 +7,6 @@
 #include <cmath>
 #include <cstdio>
 #include <memory>
-#include <mutex>
 #include <numeric>
 #include <string>
 #include <vector>
@@ -63,20 +62,6 @@ std::vector<int64_t> plan_pieces(int64_t total, double u, double v) {
         if (floor_hit) break;
     }
     return sizes;
-}
-
-// subject cuts of the database off[0 .. n] at residue targets (counted from off[0], increasing): 0, then for each target
-// the first subject boundary at or past it but at least one subject past the previous cut, then n.  A cut that would
-// leave no subject after it ends the list.
-static std::vector<int64_t> cut_subjects(const int64_t *off, int64_t n, const std::vector<int64_t> &targets) {
-    std::vector<int64_t> cut(1, 0);
-    for (const int64_t t : targets) {
-        const int64_t at = std::max<int64_t>(std::lower_bound(off, off + n + 1, off[0] + t) - off, cut.back() + 1);
-        if (at >= n) break;
-        cut.push_back(at);
-    }
-    cut.push_back(n);
-    return cut;
 }
 
 // The pieces of a host scan: the upload of piece k+1 (copy stream) runs under the scan of piece k, and nothing on the
@@ -242,16 +227,6 @@ static int scan_host_into(const FnConfig &cfg, const parasail_profile_t *profile
     if (keep_last && rc == PSB_OK) *keep_last = std::move(pieces[npieces - 1]);
     for (int k = 0; k < npieces; ++k) finish(k);
     return rc;
-}
-
-// the workers of psb_scan_box
-static std::mutex g_box_mu;
-static std::vector<BoxWorker *> g_box;   // index = device; never destroyed (the threads live as long as the process)
-static BoxWorker *box_worker(int device) {
-    std::lock_guard<std::mutex> lk(g_box_mu);
-    if ((int)g_box.size() <= device) g_box.resize(device + 1, nullptr);
-    if (!g_box[device]) g_box[device] = start_worker(device);
-    return g_box[device];
 }
 
 }  // namespace psb

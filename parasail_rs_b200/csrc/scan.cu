@@ -582,7 +582,7 @@ int scan_finish(ScanJob &job) {
     return PSB_OK;
 }
 // what every entry point that runs a profile against a database checks first: a profile function name and a profile
-static int profile_fn_check(const char *who, const char *fn_name, const parasail_profile_t *profile, FnConfig *cfg) {
+int profile_fn_check(const char *who, const char *fn_name, const parasail_profile_t *profile, FnConfig *cfg) {
     if (!parse_fn_name(fn_name, cfg) || !cfg->profile) { set_error(std::string(who) + ": not a profile function name: " + (fn_name ? fn_name : "(null)")); return PSB_EINVAL; }
     if (!profile) { set_error(std::string(who) + ": NULL profile"); return PSB_EINVAL; }
     return PSB_OK;
@@ -597,6 +597,9 @@ int scan_check(const char *who, const char *fn_name, const parasail_profile_t *p
 int profile_db_check(const char *who, const parasail_profile_t *profile, const psb_db *db) {
     PSB_TRY(ensure_ctx());
     if (db->device != g_ctx.device) { set_error(std::string(who) + ": database lives on another device"); return PSB_EINVAL; }
+    return profile_alphabet_check(who, profile, db);
+}
+int profile_alphabet_check(const char *who, const parasail_profile_t *profile, const psb_db *db) {
     if (profile->matrix.size != db->msize || std::memcmp(profile->matrix.mapper, db->mapper, 256) != 0) {
         set_error(std::string(who) + ": profile and database were built with different alphabets");
         return PSB_EINVAL;

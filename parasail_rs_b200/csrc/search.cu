@@ -97,36 +97,35 @@ static bool same_matrix(const HostMatrix &a, const HostMatrix &b) {
     return a.type == b.type && a.size == b.size && a.length == b.length && a.table == b.table && std::memcmp(a.mapper, b.mapper, 256) == 0;
 }
 
-// the alignments of the hits of the queries `qs` (rows q * kk ...), ids in `ids` (sorted rows, caller order): one
-// pairs pass.  One query is psb_db_align's request exactly; several carry each hit's query bytes in row order.
-static int align_group(const FnConfig &cfg, const parasail_profile_t *const *profiles, const std::vector<int64_t> &qs, int open, int gap, psb_db *db,
-                       int64_t kk, const int64_t *ids, psb_batch_t **out) {
-    const int64_t n = (int64_t)qs.size() * kk;
+// the alignments of the rows `rows` (one group: equal matrices), in that order: one pairs pass.  Rows of one query are
+// psb_db_align's request exactly; rows of several carry each row's query bytes.
+static int align_group(const FnConfig &cfg, const parasail_profile_t *const *profiles, const std::vector<int64_t> &rows, const int64_t *row_q,
+                       const int64_t *row_id, int open, int gap, psb_db *db, psb_batch_t **out) {
+    const int64_t n = (int64_t)rows.size();
     std::vector<int> rid((size_t)n);
     std::vector<int64_t> r_off((size_t)n + 1), q_off;
     std::vector<uint8_t> q_cat;
     r_off[0] = 0;
-    for (size_t g = 0; g < qs.size(); ++g)
-        for (int64_t r = 0; r < kk; ++r) {
-            const int64_t i = (int64_t)g * kk + r, id = ids[qs[g] * kk + r];
-            rid[(size_t)i] = (int)id;
-            r_off[(size_t)i + 1] = r_off[(size_t)i] + db->host_len[(size_t)id];
-        }
-    const parasail_profile_t *p0 = profiles[qs[0]];
+    bool one_query = true;
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t id = row_id[rows[(size_t)i]];
+        rid[(size_t)i] = (int)id;
+        r_off[(size_t)i + 1] = r_off[(size_t)i] + db->host_len[(size_t)id];
+        one_query = one_query && row_q[rows[(size_t)i]] == row_q[rows[0]];
+    }
+    const parasail_profile_t *p0 = profiles[row_q[rows[0]]];
     PairsRequest req;
     req.cfg = cfg;
     req.matrix = &p0->matrix; req.open = open; req.gap = gap;
-    if (qs.size() == 1) {
+    if (one_query) {
         q_off = {0, (int64_t)p0->query.size()};
         req.q_cat = p0->query.data(); req.shared_query = true;
     } else {
         q_off.assign((size_t)n + 1, 0);
-        for (size_t g = 0; g < qs.size(); ++g) {
-            const std::vector<uint8_t> &q = profiles[qs[g]]->query;
-            for (int64_t r = 0; r < kk; ++r) {
-                q_cat.insert(q_cat.end(), q.begin(), q.end());
-                q_off[(size_t)g * kk + r + 1] = (int64_t)q_cat.size();
-            }
+        for (int64_t i = 0; i < n; ++i) {
+            const std::vector<uint8_t> &q = profiles[row_q[rows[(size_t)i]]]->query;
+            q_cat.insert(q_cat.end(), q.begin(), q.end());
+            q_off[(size_t)i + 1] = (int64_t)q_cat.size();
         }
         req.q_cat = q_cat.data(); req.shared_query = false;
     }
@@ -134,13 +133,12 @@ static int align_group(const FnConfig &cfg, const parasail_profile_t *const *pro
     req.r_off = r_off.data(); req.n = n; req.r_db = db; req.r_ids = rid.data();
     PSB_TRY(run_pairs(req, out));
     flag_saturated(cfg, p0->matrix, open, gap, *out, [&](int64_t i) {
-        return std::make_pair((int)profiles[qs[(size_t)(i / kk)]]->query.size(), span(r_off.data(), i));
+        return std::make_pair((int)profiles[row_q[rows[(size_t)i]]]->query.size(), span(r_off.data(), i));
     });
     return PSB_OK;
 }
 
-// the rows of the group batches (`src[row]` = (group, row in it)) gathered into one batch in row order
-static int gather_rows(const FnConfig &cfg, const std::vector<psb_batch_t *> &gb, const std::vector<std::pair<int, int64_t>> &src, psb_batch_t **out) {
+int gather_rows(const FnConfig &cfg, const std::vector<psb_batch_t *> &gb, const std::vector<std::pair<int, int64_t>> &src, psb_batch_t **out) {
     const int64_t n = (int64_t)src.size();
     psb_batch_t *b = new_batch(n, cfg);
     if (!b) { set_error("pinned host allocation failed"); return PSB_ENOMEM; }
@@ -170,18 +168,23 @@ static int gather_rows(const FnConfig &cfg, const std::vector<psb_batch_t *> &gb
     return PSB_OK;
 }
 
-// the alignment pass over every query's hits: one pairs pass per group of queries with equal matrices
-static int align_hits(const FnConfig &cfg, const parasail_profile_t *const *profiles, int64_t nq, int open, int gap, psb_db *db, int64_t kk,
-                      const int64_t *ids, psb_batch_t **out) {
+int align_rows(const FnConfig &cfg, const parasail_profile_t *const *profiles, int64_t nq, const int64_t *row_q, const int64_t *row_id,
+               int64_t n, int open, int gap, psb_db *db, psb_batch_t **out) {
+    // the groups in order of their first row; a PSSM profile gets a group of its own
+    std::vector<int> group_of((size_t)nq, -1);
     std::vector<std::vector<int64_t>> groups;
-    for (int64_t q = 0; q < nq; ++q) {
-        const HostMatrix &m = profiles[q]->matrix;
-        auto it = std::find_if(groups.begin(), groups.end(), [&](const std::vector<int64_t> &g) {
-            const HostMatrix &g0 = profiles[g[0]]->matrix;
-            return m.type != PARASAIL_MATRIX_TYPE_PSSM && g0.type != PARASAIL_MATRIX_TYPE_PSSM && same_matrix(m, g0);
-        });
-        if (it == groups.end()) groups.push_back({q});
-        else it->push_back(q);
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t q = row_q[i];
+        if (group_of[(size_t)q] < 0) {
+            const HostMatrix &m = profiles[q]->matrix;
+            auto it = std::find_if(groups.begin(), groups.end(), [&](const std::vector<int64_t> &g) {
+                const HostMatrix &g0 = profiles[row_q[g[0]]]->matrix;
+                return m.type != PARASAIL_MATRIX_TYPE_PSSM && g0.type != PARASAIL_MATRIX_TYPE_PSSM && same_matrix(m, g0);
+            });
+            group_of[(size_t)q] = (int)(it - groups.begin());
+            if (it == groups.end()) groups.emplace_back();
+        }
+        groups[(size_t)group_of[(size_t)q]].push_back(i);
     }
     int first_use = 0;
     PSB_TRY(db_inv_perm(db, &first_use));
@@ -189,53 +192,25 @@ static int align_hits(const FnConfig &cfg, const parasail_profile_t *const *prof
     double ms = c.last_ms;
     int launches = c.launches + first_use;
     std::vector<psb_batch_t *> gb;
-    std::vector<std::pair<int, int64_t>> src((size_t)(nq * kk));
+    std::vector<std::pair<int, int64_t>> src((size_t)n);
     int rc = PSB_OK;
     for (size_t g = 0; g < groups.size() && rc == PSB_OK; ++g) {
         psb_batch_t *b = nullptr;
-        rc = align_group(cfg, profiles, groups[g], open, gap, db, kk, ids, &b);   // (run_pairs restarts the counters)
+        rc = align_group(cfg, profiles, groups[g], row_q, row_id, open, gap, db, &b);   // (run_pairs restarts the counters)
         ms += c.last_ms; launches += c.launches;
         if (rc != PSB_OK) break;
         gb.push_back(b);
-        for (size_t t = 0; t < groups[g].size(); ++t)
-            for (int64_t r = 0; r < kk; ++r) src[(size_t)(groups[g][t] * kk + r)] = {(int)g, (int64_t)t * kk + r};
+        for (size_t t = 0; t < groups[g].size(); ++t) src[(size_t)groups[g][t]] = {(int)g, (int64_t)t};
     }
     c.last_ms = ms; c.launches = launches;
-    if (rc == PSB_OK && gb.size() == 1) { *out = gb[0]; return PSB_OK; }   // one group holds every query in row order
+    if (rc == PSB_OK && gb.size() == 1) { *out = gb[0]; return PSB_OK; }   // one group holds every row in row order
     if (rc == PSB_OK) rc = gather_rows(cfg, gb, src, out);
     for (psb_batch_t *b : gb) free_batch(b);
     return rc;
 }
 
-}  // namespace psb
-
-using namespace psb;
-
-extern "C" {
-
-int psb_db_search(const char *fn_name, const parasail_profile_t *const *profiles, int64_t nq, int open, int gap, const psb_db_t *db_c, int k,
-                  int64_t *ids_out, psb_batch_t **out) {
-    if (out) *out = nullptr;
-    FnConfig cfg;
-    if (!parse_fn_name(fn_name, &cfg) || !cfg.profile) {
-        set_error(std::string("psb_db_search: not a profile function name: ") + (fn_name ? fn_name : "(null)"));
-        return PSB_EINVAL;
-    }
-    if (cfg.table || cfg.rowcol) { set_error("psb_db_search: _table/_rowcol outputs exist only on the single-pair API"); return PSB_EUNSUPPORTED; }
-    if (!profiles || !db_c || !ids_out || !out) { set_error("psb_db_search: NULL argument"); return PSB_EINVAL; }
-    if (nq <= 0 || k <= 0) { set_error("psb_db_search: " + std::to_string(nq) + " queries, k = " + std::to_string(k)); return PSB_EINVAL; }
-    psb_db *db = const_cast<psb_db *>(db_c);
-    PSB_TRY(db_check("psb_db_search", db));
-    const int64_t kk = std::min<int64_t>(k, db->n);
-    if (nq > INT_MAX / kk) {
-        set_error("psb_db_search: " + std::to_string(nq) + " queries x " + std::to_string(kk) + " hits is more than 2^31-1 rows");
-        return PSB_EUNSUPPORTED;
-    }
-    for (int64_t q = 0; q < nq; ++q) {
-        const std::string who = "psb_db_search: profiles[" + std::to_string(q) + "]";
-        if (!profiles[q]) { set_error(who + " is NULL"); return PSB_EINVAL; }
-        PSB_TRY(profile_db_check(who.c_str(), profiles[q], db));
-    }
+int search_select(const FnConfig &cfg, const parasail_profile_t *const *profiles, int64_t nq, int open, int gap, psb_db *db, int64_t kk,
+                  SearchHits *hits) {
     const int64_t R = nq * kk;
     Ctx &c = g_ctx;
     c.last_ms = 0.0; c.launches = 0;
@@ -275,10 +250,9 @@ int psb_db_search(const char *fn_name, const parasail_profile_t *const *profiles
     if (rc == PSB_OK && cudaStreamSynchronize(c.stream) != cudaSuccess) {
         set_error(std::string("psb_db_search: ") + cudaGetErrorString(cudaGetLastError())); rc = PSB_ECUDA;
     }
-    int64_t retried = 0;
     for (auto &j : jobs) {
         if (rc == PSB_OK) rc = scan_finish(*j);
-        retried += j->retried;
+        hits->retried += j->retried;
     }
     if (rc != PSB_OK) {
         cudaStreamSynchronize(c.stream);
@@ -290,31 +264,73 @@ int psb_db_search(const char *fn_name, const parasail_profile_t *const *profiles
     if (cudaEventElapsedTime(&sel_ms, jobs[0]->ev0, c.ev1) == cudaSuccess) c.last_ms = sel_ms;
     jobs.clear();
     // each query's rows in the order of psb_batch_topk
-    const int *r_id = rows, *r_score = rows + R, *r_eq = rows + 2 * R, *r_er = rows + 3 * R, *r_sat = rows + 4 * R;
+    const int *r_id = rows, *r_score = rows + R;
     std::vector<int64_t> order((size_t)R);
     for (int64_t q = 0; q < nq; ++q) {
         int64_t *o = order.data() + q * kk;
         std::iota(o, o + kk, q * kk);
         std::sort(o, o + kk, [&](int64_t a, int64_t b) { return r_score[a] != r_score[b] ? r_score[a] > r_score[b] : r_id[a] < r_id[b]; });
-        for (int64_t r = 0; r < kk; ++r) ids_out[q * kk + r] = r_id[o[r]];
     }
+    std::vector<int> *planes[5] = {&hits->id, &hits->score, &hits->end_query, &hits->end_ref, &hits->saturated};
+    for (int k = 0; k < 5; ++k) {
+        planes[k]->resize((size_t)R);
+        const int *src = rows + (size_t)k * R;
+        for (int64_t i = 0; i < R; ++i) (*planes[k])[(size_t)i] = src[order[(size_t)i]];
+    }
+    pinned_free(rows, (size_t)R * 5 * sizeof(int));
+    return PSB_OK;
+}
+
+}  // namespace psb
+
+using namespace psb;
+
+extern "C" {
+
+int psb_db_search(const char *fn_name, const parasail_profile_t *const *profiles, int64_t nq, int open, int gap, const psb_db_t *db_c, int k,
+                  int64_t *ids_out, psb_batch_t **out) {
+    if (out) *out = nullptr;
+    FnConfig cfg;
+    if (!parse_fn_name(fn_name, &cfg) || !cfg.profile) {
+        set_error(std::string("psb_db_search: not a profile function name: ") + (fn_name ? fn_name : "(null)"));
+        return PSB_EINVAL;
+    }
+    if (cfg.table || cfg.rowcol) { set_error("psb_db_search: _table/_rowcol outputs exist only on the single-pair API"); return PSB_EUNSUPPORTED; }
+    if (!profiles || !db_c || !ids_out || !out) { set_error("psb_db_search: NULL argument"); return PSB_EINVAL; }
+    if (nq <= 0 || k <= 0) { set_error("psb_db_search: " + std::to_string(nq) + " queries, k = " + std::to_string(k)); return PSB_EINVAL; }
+    psb_db *db = const_cast<psb_db *>(db_c);
+    PSB_TRY(db_check("psb_db_search", db));
+    const int64_t kk = std::min<int64_t>(k, db->n);
+    if (nq > INT_MAX / kk) {
+        set_error("psb_db_search: " + std::to_string(nq) + " queries x " + std::to_string(kk) + " hits is more than 2^31-1 rows");
+        return PSB_EUNSUPPORTED;
+    }
+    for (int64_t q = 0; q < nq; ++q) {
+        const std::string who = "psb_db_search: profiles[" + std::to_string(q) + "]";
+        if (!profiles[q]) { set_error(who + " is NULL"); return PSB_EINVAL; }
+        PSB_TRY(profile_db_check(who.c_str(), profiles[q], db));
+    }
+    const int64_t R = nq * kk;
+    SearchHits h;
+    PSB_TRY(search_select(cfg, profiles, nq, open, gap, db, kk, &h));
+    for (int64_t i = 0; i < R; ++i) ids_out[i] = h.id[(size_t)i];
     double scan_cells = 0;
     for (int64_t q = 0; q < nq; ++q) scan_cells += (double)profiles[q]->query.size() * (double)db->residues;
     psb_batch_t *b = nullptr;
     if (cfg.trace || cfg.stats) {
-        rc = align_hits(cfg, profiles, nq, open, gap, db, kk, ids_out, &b);
+        std::vector<int64_t> row_q((size_t)R);
+        for (int64_t i = 0; i < R; ++i) row_q[(size_t)i] = i / kk;
+        PSB_TRY(align_rows(cfg, profiles, nq, row_q.data(), ids_out, R, open, gap, db, &b));
     } else {
         b = new_batch(R, cfg);
-        if (!b) { set_error("pinned host allocation failed"); rc = PSB_ENOMEM; }
-        for (int64_t i = 0; b && i < R; ++i) {
-            const int64_t j = order[(size_t)i];
-            b->score[i] = r_score[j]; b->end_query[i] = r_eq[j]; b->end_ref[i] = r_er[j]; b->saturated[i] = (uint8_t)r_sat[j];
+        if (!b) { set_error("pinned host allocation failed"); return PSB_ENOMEM; }
+        for (int64_t i = 0; i < R; ++i) {
+            b->score[i] = h.score[(size_t)i]; b->end_query[i] = h.end_query[(size_t)i]; b->end_ref[i] = h.end_ref[(size_t)i];
+            b->saturated[i] = (uint8_t)h.saturated[(size_t)i];
         }
     }
-    pinned_free(rows, (size_t)R * 5 * sizeof(int));
-    if (rc != PSB_OK) return rc;
     b->cells += scan_cells;
-    b->n_retried = retried;
+    b->n_retried = h.retried;
     *out = b;
     return PSB_OK;
 }
